@@ -52,6 +52,7 @@ UNIQUE_STREAMS = 128  # distinct pink-noise streams generated on the host, tiled
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 FP32_FMA_TFLOPS_MEASURED = 70.88  # tools/microbench/fp32_pipes.cu on this pool's B200 (profiles/r01_fp32_pipes_microbench.jsonl)
 SUSTAINED_SECONDS = float(os.environ.get("OHS_BENCH_SUSTAINED_S", "3.0"))
+DUMP_STREAMS = min(128, 64_000_000 // (2 * FRAMES_PER_STEP * 4))  # --dump-outputs: 50 MB at the default step, never above 64 MB
 
 
 def algorithmic_bytes_per_stream(k_blocks: int, block: int = BLOCK, parts: int = 1) -> int:
@@ -155,13 +156,13 @@ def workload_config(n_gpus: int) -> dict:
 # library is never loaded here: signals is pure numpy, the EQ design is the oracle's own).
 # --------------------------------------------------------------------------------------------------------------
 def native_oracle():
-    """The oracle built -march=native on the box it is timed on (oracle/_native/, git-ignored); falls back to the
-    portable build that travels with the repo."""
+    """The oracle built -march=native on the box it is timed on, in a temporary directory that is gone once the library
+    is mapped (the benchmark writes nothing into the tree); falls back to the portable build of oracle/."""
     from oracle import oracle as O
 
     try:
-        path = O.build_native()
-        O.use_library(path)
+        with tempfile.TemporaryDirectory(prefix="ohs_oracle_") as d:
+            O.use_library(O.build_native(d))  # loaded before the directory goes: the mapping outlives the file
         return O, "gcc -O3 -march=native -ffp-contract=off (built on this box)"
     except Exception as e:  # no compiler on the box: the portable library
         return O, "portable x86-64-v3 build (native build failed: %s)" % (str(e)[:80],)
@@ -217,7 +218,7 @@ def run_reference(args, signals):
     if rank != 0:
         return
     # each step is the stated config: 1024 streams x 1.024 s of audio (about 0.4 s of CPU work per step on 16 cores)
-    steps = max(1, min(args.steps, 40))
+    steps = args.steps
     value, cores, sample, ms = cpu_reference_run(signals, steps, min(args.warmup, 1), N_STREAMS, FRAMES_PER_STEP / FS)
     cpu = {"value": value, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample}
     bound = pocketfft_conv_bound(signals, cores, 256, 48)
@@ -543,6 +544,16 @@ def run_object_config(ctx: Ctx, reps: int):
     return out
 
 
+def dump_outputs(out_dir: str, torch, d_out):
+    """What the headline step hands its caller: y[stream, channel, frame] of the last timed step, float32.  The whole step
+    is 400 MB, so a fixed sample of DUMP_STREAMS streams (seed 0, sorted, spread over the batch) is written.  The inputs,
+    the warm-up and the step count fix the engine's state, so equal arguments give equal outputs on one build."""
+    idx = np.sort(np.random.default_rng(0).choice(N_STREAMS, DUMP_STREAMS, replace=False))
+    y = d_out[torch.from_numpy(idx).to(d_out.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "y.npy"), y)
+
+
 def run_gpu(args, pkg):
     ctx = Ctx(args, pkg)
     torch, dist = ctx.torch, ctx.dist
@@ -580,6 +591,8 @@ def run_gpu(args, pkg):
     ms_per_step = ctx.timed(stream, step, args.steps)
     launches = eng.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, d_out)
     stream_seconds_per_step = N_STREAMS * world * FRAMES_PER_STEP / FS
     value = stream_seconds_per_step / (ms_per_step * 1e-3)
 
@@ -710,13 +723,22 @@ def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, help="timed steps (default 50; 40 with --impl reference, whose steps take seconds on the CPU)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the configs 3/4/5 legs")
     ap.add_argument("--device-only", action="store_true", help="only the device-resident arm (used under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's output for %d streams (a fixed sample; rank 0's streams "
+                         "when several GPUs run) to DIR/y.npy" % DUMP_STREAMS)
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 40 if args.impl == "reference" else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         # signals only (pure numpy): the product library is never mapped by this arm

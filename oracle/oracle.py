@@ -35,18 +35,14 @@ def build(force: bool = False) -> str:
     return _LIB_PATH
 
 
-def build_native() -> str:
-    """The same source built -march=native into oracle/_native/ (git-ignored) on the machine that will TIME it — the
-    CPU-baseline legs of bench.py only; the parity tests keep the portable build that travels with the repo."""
-    out_dir = os.path.join(_HERE, "_native")
-    os.makedirs(out_dir, exist_ok=True)
+def build_native(out_dir: str) -> str:
+    """The same source built -march=native into out_dir on the machine that will TIME it — the CPU-baseline legs of
+    bench.py only; the parity tests keep the portable build in oracle/.  out_dir is the caller's: the source tree may
+    be read-only where the benchmark runs."""
     out = os.path.join(out_dir, "libohs_oracle_native.so")
     src = os.path.join(_HERE, "ohs_oracle.c")
-    if not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
-        tmp = out + ".tmp.%d" % os.getpid()
-        subprocess.check_call(["gcc", "-O3", "-march=native", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-std=gnu11", "-shared",
-                               "-o", tmp, src, "-lm", "-lpthread"], cwd=_HERE)
-        os.replace(tmp, out)
+    subprocess.check_call(["gcc", "-O3", "-march=native", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-std=gnu11", "-shared",
+                           "-o", out, src, "-lm", "-lpthread"], cwd=out_dir)
     return out
 
 
@@ -55,10 +51,17 @@ _lib_path = _LIB_PATH
 
 
 def use_library(path: str) -> None:
-    """Bind this module to another build of the oracle (build_native()); call before the first use."""
+    """Bind this module to another build of the oracle (build_native()), loaded now: if it does not load, the module
+    stays bound to the library it had."""
     global _lib, _lib_path
     if path != _lib_path:
+        old = _lib, _lib_path
         _lib, _lib_path = None, path
+        try:
+            lib()
+        except Exception:
+            _lib, _lib_path = old
+            raise
 
 
 def lib():

@@ -1,6 +1,4 @@
 """Host-side rows next to the hot path (SURVEY.md §8f): HRIR selection/wiring and AutoEQ CSV ingestion.  CPU only."""
-import os
-
 import numpy as np
 import pytest
 
@@ -36,11 +34,22 @@ def test_wire_speakers_calls_set_ir_for_the_four_paths(cipic):
     assert np.array_equal(calls[0][1], cipic["ir"][308, 0]) and np.array_equal(calls[3][1], cipic["ir"][908, 1])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/hrtf/subject_003.sofa"), reason="reference tree only exists in the dev container")
-def test_load_sofa_reads_the_bundled_file_without_hdf5(cipic):
-    h = sofa.load_sofa("/root/reference/data/hrtf/subject_003.sofa")
+@pytest.fixture(scope="module")
+def cipic_sofa(cipic, tmp_path_factory):
+    """The reference's bundled CIPIC subject 003 file, rebuilt from tests/golden/cipic003_hrir.npz (what its two datasets
+    decode to, see tests/golden/make_sofa_fixture.py): full size, M = 1250 x R = 2 x N = 200, as byte-shuffled f64 zlib
+    streams among unrelated bytes."""
+    path = tmp_path_factory.mktemp("sofa") / "subject_003.sofa"
+    write_sofa_datasets(path, cipic["pos"], cipic["ir"], np.random.default_rng(3))
+    return str(path)
+
+
+def test_load_sofa_reads_the_bundled_file_without_hdf5(cipic, cipic_sofa):
+    """The bundled CIPIC data at full size, read back exactly.  The file is cipic_sofa's rebuild: the real file's HDF5
+    byte layout around the two datasets is not exercised."""
+    h = sofa.load_sofa(cipic_sofa)
     assert h.ir.shape == (1250, 2, 200)
-    assert np.array_equal(h.ir, cipic["ir"]) and np.allclose(h.position, cipic["pos"])
+    assert np.array_equal(h.ir, cipic["ir"]) and np.array_equal(h.position, cipic["pos"])
 
 
 def test_parse_autoeq_csv():
@@ -72,20 +81,26 @@ import open_headstage_b200 as ohs  # noqa: E402
 
 
 def write_sofa_like(path, m=24, n=32, seed=3):
-    """A file with the two datasets the readers look for, stored the way HDF5 stores them in a SimpleFreeFieldHRIR file
-    (f64, byte-shuffled, zlib) between unrelated bytes — including stray 0x78 bytes and a decoy zlib stream."""
+    """A small seeded HRIR set written by write_sofa_datasets."""
     rng = np.random.default_rng(seed)
     az = np.array([0, 15, 30, 45, 60, 90, 120, 150, 180, 210, 240, 270, 300, 315, 330, 345] + [30, 330, 0, 90, 270, 180, 45, 315], np.float64)[:m]
     el = np.array([0.0] * 16 + [30.0] * 8)[:m]
     pos = np.stack([az, el, np.ones(m)], axis=1)
     ir = (rng.standard_normal((m, 2, n)) * np.exp(-np.arange(n) / 6.0)).astype(np.float32).astype(np.float64)  # f32-representable
+    write_sofa_datasets(path, pos, ir, rng)
+    return pos.astype(np.float32), ir.astype(np.float32)
+
+
+def write_sofa_datasets(path, pos, ir, rng):
+    """A file with the two datasets the readers look for, stored the way HDF5 stores them in a SimpleFreeFieldHRIR file
+    (f64, byte-shuffled, zlib) between unrelated bytes — including stray 0x78 bytes and a decoy zlib stream."""
+    pos, ir = np.asarray(pos, np.float64), np.asarray(ir, np.float64)
     shuffle = lambda a: np.ascontiguousarray(a).view(np.uint8).reshape(-1, 8).T.copy().tobytes()  # noqa: E731
     junk = rng.integers(0, 256, 5000, dtype=np.uint8).tobytes()
     decoy = zlib.compress(b"not a dataset" * 40)
     with open(path, "wb") as f:
         f.write(b"\x89HDF\r\n\x1a\n" + junk[:700] + b"\x78\x9c" + junk[700:1500] + decoy + zlib.compress(shuffle(pos), 6) + junk[1500:2600] + b"\x78"
                 + zlib.compress(shuffle(ir), 9) + junk[2600:])
-    return pos.astype(np.float32), ir.astype(np.float32)
 
 
 def run_tool(*args):
@@ -118,9 +133,10 @@ def test_cpp_sofa_reader_matches_python_reader(tmp_path):
     assert run_tool("sofa", str(tmp_path / "missing.sofa"), 24, 32, 0, 0, 0, 0).returncode == 1
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/hrtf/subject_003.sofa"), reason="reference tree only exists in the dev container")
-def test_cpp_sofa_reader_reads_the_bundled_file(cipic):
-    r = run_tool("sofa", "/root/reference/data/hrtf/subject_003.sofa", 1250, 200, 30, 0, 330, 0)
+def test_cpp_sofa_reader_reads_the_bundled_file(cipic, cipic_sofa):
+    """As test_load_sofa_reads_the_bundled_file_without_hdf5, through the C++ reader: the real file's HDF5 byte layout
+    is not exercised."""
+    r = run_tool("sofa", cipic_sofa, 1250, 200, 30, 0, 330, 0)
     assert r.returncode == 0, r.stderr
     d = json.loads(r.stdout)
     assert (d["M"], d["N"], d["left_index"], d["right_index"]) == (1250, 200, 308, 908)     # SURVEY.md 8c indices
