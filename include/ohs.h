@@ -101,6 +101,26 @@ int ohs_set_ir(ohs_engine* h, int hrir_set, int path, const float* ir, size_t le
 int ohs_num_partitions(ohs_engine* h, int hrir_set, int path, int* out);
 /* Which HRIR set a stream (or OHS_ALL) convolves with; clears that stream's convolution history. */
 int ohs_bind_stream_hrir(ohs_engine* h, int stream, int hrir_set);
+/* ---- moving sources (an extension: the reference reads its speaker angles and never applies them) -------------
+ * A stream changes HRIR sets WITHOUT losing its history, crossfaded over one engine block.  Every stream has a set
+ * set(t) for every block t it convolves; block t is a transition when set(t) != set(t-1) (for a call's first block,
+ * set(t-1) is the binding before the call).  With y_X[t] the output block t of a stream bound to set X since its
+ * history began (gain included, exactly what the engine renders without moves):
+ *   non-transition block:  out[t] = y_set(t)[t]
+ *   transition block:      a = y_set(t-1)[t], b = y_set(t)[t], w[n] = (2n+1)/(2B), n = 0..B-1,
+ *                          out[t][n] = a[n] + w[n]*(b[n] - a[n]), each operation rounded on its own in f32
+ * A switch never touches history (EQ state, overlap-save block, delay line): after its transition block a moved
+ * stream is bit-identical to one bound to the target set from the start.  Sets with different partition counts mix
+ * freely.  Pending moves and schedules are configuration, like bindings: they are not part of the state blob.
+ *
+ * Per-buffer form (head tracking, host automation): records a pending target for `stream` (or OHS_ALL).  The next
+ * engine block that stream convolves crossfades from its binding to the target (ohs_process_device, the first chunk
+ * of ohs_process, the first whole engine block ohs_process_fifo renders, possibly in a later call); the binding is
+ * the target from then on.  Moving to the binding, or back to it before any call, is a no-op; ohs_bind_stream_hrir
+ * cancels the move (and clears the history, as always).  Bypassed calls and calls with the convolution disabled
+ * leave the move pending.  The commit of set_ir work at the start of a call clears the streams BOUND to re-committed
+ * sets before moves apply: write the new direction into a spare set, then move to it, and nothing is cleared. */
+int ohs_move_stream_hrir(ohs_engine* h, int stream, int hrir_set);
 /* Device-resident filter spectra of all sets, for a caller-side NCCL broadcast (SURVEY.md §8e): pointer and byte
  * size of the table the render kernel reads.  ohs_commit_filters uploads pending set_ir work first; after an
  * external overwrite (broadcast receive) call ohs_mark_filters_external so pending host IRs do not overwrite it. */
@@ -155,6 +175,16 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io);
  * same state afterwards; the call is still ordered on the engine's stream alone; ohs_set_time_batch(h, 0) disables
  * it. */
 int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride);
+/* ohs_process_device with a per-block set schedule (offline rendering of moving sources, definition above the
+ * ohs_move_stream_hrir declaration): `sets` is HOST memory [n_streams][sets_stride], block t < n_frames/B of stream s
+ * convolves with set sets[s*sets_stride + t].  Validated before anything is enqueued: a null pointer, sets_stride <
+ * n_frames/B, a set out of range or the convolution disabled return OHS_ERR_INVALID with the engine untouched.  Pending
+ * moves are superseded (block 0 compares with the binding); afterwards every stream is bound to its last column.  A
+ * call with a transition runs the block-by-block kernel (long responses included: the time-batched route convolves
+ * one set per stream and call); a schedule without one renders exactly like ohs_process_device.  Bypass behaves as
+ * there and leaves the bindings unchanged. */
+int ohs_process_device_scheduled(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride,
+                                 const int32_t* sets, size_t sets_stride);
 /* Host flavour: pointers are host memory (pinned memory from ohs_host_alloc gives full PCIe speed); the call
  * stages time chunks through HBM with copies overlapped against the kernels and returns when `out` is complete. */
 int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride);

@@ -124,16 +124,25 @@ struct ohs_engine {
     // FIFO adaptor (src/dsp/convolution.rs:141-182)
     std::vector<float> fifo_in, fifo_out;  // [row][cap]
     size_t fifo_cap = 0, fifo_in_len = 0, fifo_out_len = 0;
+
+    // moving sources (DESIGN §10): ohs_move_stream_hrir targets (-1: none) applied by the next convolving block, the
+    // bindings they replace (the kernel's from_set) and ohs_process_device_scheduled's per-block sets
+    std::vector<int> h_move_to, h_from_set;
+    bool any_move = false;
+    int* d_from_set = nullptr;
+    int* d_sched = nullptr;
+    size_t sched_cap = 0;   // ints
 };
 
 namespace {
 
 using namespace ohs;
 
-int launch_render(ohs_engine* h, const RenderParams& p, int first_stream = 0) {
+// moving: render_kernel_moving (p.from_set set, p.block_set optional)
+int launch_render(ohs_engine* h, const RenderParams& p, int first_stream = 0, bool moving = false) {
     // few blocks per launch: nothing overlaps inside the launch, so the variant built for latency runs it
     const bool latency = p.n_blocks <= h->latency_blocks;
-    RenderLaunch L{h->G, h->cfg.device, h->stream, first_stream, latency ? 1 : 0, 0, h->dependent_launch};
+    RenderLaunch L{h->G, h->cfg.device, h->stream, first_stream, latency ? 1 : 0, 0, h->dependent_launch, moving};
     RenderParams q = p;
     q.trace = h->d_trace;
     cudaError_t e = cudaErrorInvalidValue;
@@ -741,6 +750,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     const size_t per_path = (size_t)h->pmax * B;
 
     h->h_stream_hrir.assign(S, 0);
+    h->h_move_to.assign(S, -1);
     h->h_stream_eq.assign(S, 0);
     h->h_gain.assign(S, 1.0f);
     h->h_set_parts.assign(cfg->n_hrir_sets, 1);
@@ -781,6 +791,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     }
     h->filt_bytes = sizeof(float4) * (size_t)cfg->n_hrir_sets * h->pmax * h->N;
     OHS_TRY(cudaMalloc(&h->d_stream_hrir, sizeof(int) * S));
+    OHS_TRY(cudaMalloc(&h->d_from_set, sizeof(int) * S));
     OHS_TRY(cudaMalloc(&h->d_stream_eq, sizeof(int) * S));
     OHS_TRY(cudaMalloc(&h->d_stream_gain, sizeof(float) * S));
     OHS_TRY(cudaMalloc(&h->d_filt, h->filt_bytes));
@@ -825,7 +836,7 @@ int ohs_destroy(ohs_engine* h) {
     for (cudaEvent_t e : {h->ev_fwd[0], h->ev_fwd[1], h->ev_call}) if (e) cudaEventDestroy(e);
     void* ptrs[] = {h->d_stream_hrir, h->d_stream_eq, h->d_stream_gain, h->d_filt, h->d_set_parts, h->d_set_list, h->d_set_flags,
                     h->d_fdl, h->d_prev, h->d_eqc, h->d_eqs, h->d_tw, h->d_ir, h->d_stage[0], h->d_stage[1], h->d_stage[2],
-                    h->d_zlin, h->d_wlin, h->d_xf};
+                    h->d_zlin, h->d_wlin, h->d_xf, h->d_from_set, h->d_sched};
     for (void* p : ptrs) if (p) cudaFree(p);
     for (int i = 0; i < kPipe; ++i) {
         if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
@@ -872,6 +883,8 @@ int ohs_bind_stream_hrir(ohs_engine* h, int stream, int hrir_set) {
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     if (stream == OHS_ALL) std::fill(h->h_stream_hrir.begin(), h->h_stream_hrir.end(), hrir_set);
     else h->h_stream_hrir[stream] = hrir_set;
+    if (stream == OHS_ALL) std::fill(h->h_move_to.begin(), h->h_move_to.end(), -1);   // a hard bind cancels a pending move
+    else h->h_move_to[stream] = -1;
     h->bind_dirty = true;
     // a re-bound stream starts from empty history, like a ConvolutionEngine that was just given its IRs
     if (stream == OHS_ALL) {
@@ -883,6 +896,16 @@ int ohs_bind_stream_hrir(ohs_engine* h, int stream, int hrir_set) {
     h->zlin_valid = false;
     OHS_CUDA(cudaMemsetAsync(h->d_fdl + (size_t)stream * h->pmax * h->N, 0, sizeof(float2) * (size_t)h->pmax * h->N, h->stream));
     OHS_CUDA(cudaMemsetAsync(h->d_prev + (size_t)stream * h->B, 0, sizeof(float2) * (size_t)h->B, h->stream));
+    return OHS_OK;
+}
+
+int ohs_move_stream_hrir(ohs_engine* h, int stream, int hrir_set) {
+    OHS_CHECK_HANDLE(h);
+    if (hrir_set < 0 || hrir_set >= h->cfg.n_hrir_sets) return fail(OHS_ERR_INVALID, "hrir_set %d out of range", hrir_set);
+    if (stream != OHS_ALL && (stream < 0 || stream >= h->cfg.n_streams)) return fail(OHS_ERR_INVALID, "stream %d out of range", stream);
+    const int lo = stream == OHS_ALL ? 0 : stream, hi = stream == OHS_ALL ? h->cfg.n_streams : stream + 1;
+    for (int s = lo; s < hi; ++s) h->h_move_to[s] = hrir_set == h->h_stream_hrir[s] ? -1 : hrir_set;   // back to the binding: no move
+    h->any_move = std::any_of(h->h_move_to.begin(), h->h_move_to.end(), [](int v) { return v >= 0; });
     return OHS_OK;
 }
 
@@ -1037,11 +1060,22 @@ int ohs_debug_trace(ohs_engine* h, unsigned long long* d_stamps) {
 }
 
 // ---- processing ---------------------------------------------------------------------------------------------
-int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride) {
-    OHS_CHECK_HANDLE(h);
-    int rc = check_audio_args(h, d_in, d_out, n_frames, row_stride, true);
-    if (rc) return rc;
-    OHS_CUDA(cudaSetDevice(h->cfg.device));
+}  // extern "C"
+
+namespace {
+
+// A multi-set engine with a delay line where some stream is bound to a one-partition set: render_kernel does not put
+// that stream's spectra into the delay line (it never reads them), but a later move to a longer set needs them, so
+// such calls run render_kernel_moving, which writes every block's.  Same outputs, more delay-line traffic.
+bool needs_full_ring(const ohs_engine* h) {
+    if (h->pmax == 1 || h->cfg.n_hrir_sets == 1) return false;
+    for (int set : h->h_stream_hrir) if (h->h_set_parts[set] == 1) return true;
+    return false;
+}
+
+// ohs_process_device, and ohs_process_device_scheduled with `sets` (validated by the caller)
+int process_device_impl(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride, const int32_t* sets,
+                        size_t sets_stride) {
     if (n_frames == 0) return OHS_OK;
     if (h->bypass) {  // master_bypass: buffer untouched, no state advances (src/lib.rs:1169)
         if (d_in != d_out)
@@ -1049,7 +1083,7 @@ int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_
                                        (size_t)h->cfg.n_streams * 2, cudaMemcpyDeviceToDevice, h->stream));
         return OHS_OK;
     }
-    rc = commit_filters(h);
+    int rc = commit_filters(h);
     if (rc) return rc;
     RenderParams p{};
     p.in = d_in; p.out = d_out; p.row_stride = p.out_row_stride = (long long)row_stride;
@@ -1066,10 +1100,55 @@ int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_
     p.filt_in_smem = 0;
     if (h->cfg.n_hrir_sets == 1 && h->N <= 512 && (size_t)h->h_set_parts[0] * h->N * sizeof(float4) <= 16 * 1024)
         p.filt_in_smem = h->h_set_parts[0];
+    // moving sources: does this call carry a transition (set of a block != set of the block before)?  Pending moves
+    // apply only to convolving calls, after the commit above has cleared the streams bound to re-committed sets.
+    const size_t S = (size_t)h->cfg.n_streams, K = (size_t)p.n_blocks;
+    bool transition = false;
+    if (sets) {
+        for (size_t s = 0; s < S && !transition; ++s) {
+            int prev = h->h_stream_hrir[s];
+            for (size_t t = 0; t < K; ++t) {
+                const int cur = sets[s * sets_stride + t];
+                if (cur != prev) { transition = true; break; }
+                prev = cur;
+            }
+        }
+        if (transition) {
+            if (S * K > h->sched_cap) {
+                OHS_CUDA(cudaStreamSynchronize(h->stream));   // an earlier launch may still read the old buffer
+                if (h->d_sched) OHS_CUDA(cudaFree(h->d_sched));
+                h->d_sched = nullptr; h->sched_cap = 0;
+                OHS_CUDA(cudaMalloc(&h->d_sched, sizeof(int) * S * K));
+                h->sched_cap = S * K;
+            }
+            OHS_CUDA(cudaMemcpy2DAsync(h->d_sched, sizeof(int) * K, sets, sizeof(int) * sets_stride, sizeof(int) * K, S,
+                                       cudaMemcpyHostToDevice, h->stream));
+            p.block_set = h->d_sched; p.block_set_stride = (long long)K;
+        }
+        p.from_set = h->d_stream_hrir;   // block 0 compares with the binding
+        std::fill(h->h_move_to.begin(), h->h_move_to.end(), -1);   // the schedule supersedes pending moves
+        h->any_move = false;
+        for (size_t s = 0; s < S; ++s) {
+            const int last = sets[s * sets_stride + K - 1];
+            if (last != h->h_stream_hrir[s]) { h->h_stream_hrir[s] = last; h->bind_dirty = true; }   // uploaded by the next call
+        }
+    } else if (h->any_move && h->conv_enable) {
+        h->h_from_set = h->h_stream_hrir;
+        for (size_t s = 0; s < S; ++s)
+            if (h->h_move_to[s] >= 0) { h->h_stream_hrir[s] = h->h_move_to[s]; h->h_move_to[s] = -1; }
+        h->any_move = false;
+        h->bind_dirty = true;
+        transition = true;
+        rc = upload_bindings(h);
+        if (rc) return rc;
+        OHS_CUDA(cudaMemcpyAsync(h->d_from_set, h->h_from_set.data(), sizeof(int) * S, cudaMemcpyHostToDevice, h->stream));
+        p.from_set = h->d_from_set;
+    }
     // (off by default: an event between two launches keeps the second from starting while the first drains)
     if (h->timing) OHS_CUDA(cudaEventRecord(h->ev_k0, h->stream));
     // long responses over many blocks: convolve along time per bin instead of re-reading the delay line every block
-    bool batched = time_batch_eligible(h, p.n_blocks);
+    // (one set per stream and call: a call with a transition runs the block-by-block kernel)
+    bool batched = !transition && time_batch_eligible(h, p.n_blocks);
     if (batched) {
         rc = process_time_batched(h, p, d_in, d_out, row_stride);
         if (rc < 0) return rc;
@@ -1077,7 +1156,9 @@ int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_
     }
     if (!batched) {
         if (h->conv_enable) { rc = ensure_ring(h); if (rc) return rc; }   // the kernel reads and extends the delay-line ring
-        rc = launch_render(h, p);
+        const bool moving = transition || (h->conv_enable && needs_full_ring(h));
+        if (moving && !p.from_set) p.from_set = h->d_stream_hrir;
+        rc = launch_render(h, p, 0, moving);
         if (rc) return rc;
         if (h->conv_enable) {
             h->head = (int)(((size_t)h->head + p.n_blocks) % (size_t)h->pmax);
@@ -1086,6 +1167,36 @@ int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_
     }
     if (h->timing) { OHS_CUDA(cudaEventRecord(h->ev_k1, h->stream)); h->timed = true; }
     return OHS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride) {
+    OHS_CHECK_HANDLE(h);
+    int rc = check_audio_args(h, d_in, d_out, n_frames, row_stride, true);
+    if (rc) return rc;
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    return process_device_impl(h, d_in, d_out, n_frames, row_stride, nullptr, 0);
+}
+
+int ohs_process_device_scheduled(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride,
+                                 const int32_t* sets, size_t sets_stride) {
+    OHS_CHECK_HANDLE(h);
+    int rc = check_audio_args(h, d_in, d_out, n_frames, row_stride, true);
+    if (rc) return rc;
+    if (!sets) return fail(OHS_ERR_INVALID, "null schedule");
+    if (!h->conv_enable) return fail(OHS_ERR_INVALID, "a schedule needs the convolution enabled");
+    const size_t K = n_frames / (size_t)h->B;
+    if (sets_stride < K) return fail(OHS_ERR_INVALID, "sets_stride %zu < %zu blocks", sets_stride, K);
+    for (size_t s = 0; s < (size_t)h->cfg.n_streams; ++s)
+        for (size_t t = 0; t < K; ++t) {
+            const int v = sets[s * sets_stride + t];
+            if (v < 0 || v >= h->cfg.n_hrir_sets) return fail(OHS_ERR_INVALID, "schedule: stream %zu block %zu names hrir_set %d out of range", s, t, v);
+        }
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    return process_device_impl(h, d_in, d_out, n_frames, row_stride, sets, sets_stride);
 }
 
 int ohs_sync(ohs_engine* h) {

@@ -88,6 +88,11 @@ struct RenderParams {
     int first_stream;           // CTA 0 renders streams first_stream .. first_stream+G-1 (set by the launcher)
     int io_first_stream;        // the stream whose rows sit at in/out row 0 (host staging by stream range), else 0
     unsigned long long* trace;  // OHS_TRACE builds: [CTA][16] clock64 stamps of the launch's milestones, else unused
+    // moving sources (render_kernel_moving only; DESIGN §10): the set of block t is block_set[s*block_set_stride + t],
+    // or stream_hrir[s] for every block when block_set is null; from_set[s] is the set of the block before block 0
+    const int* from_set;
+    const int* block_set;
+    long long block_set_stride;
 };
 
 #ifdef OHS_TRACE
@@ -917,7 +922,40 @@ struct OutputStore {
     }
 };
 
-template <int N, int G, int V>
+// OutputStore of the moving-sources kernel.  With `blend` (second pass of a transition block) the rows already hold the
+// old set's output a, written by this same thread (the last passes of the two inverse transforms map elements to
+// threads identically), this pass's output is b, and out[n] = a + w[n]*(b - a) with w[n] = (2n+1)/(2B), exact in f32,
+// each operation rounded on its own
+struct MixStore {
+    float* ol; float* orr; float gain; int B; bool blend;
+    __device__ __forceinline__ float mix(float a, float b, int n) const {
+        const float w = __fmul_rn((float)(2 * n + 1), __frcp_rn((float)(2 * B)));
+        return __fadd_rn(a, __fmul_rn(w, __fsub_rn(b, a)));
+    }
+    __device__ __forceinline__ void st(int i, float2 v) const {
+        if (i >= B) {
+            float l = __fmul_rn(v.y, gain), r = __fmul_rn(v.x, gain);
+            if (blend) { l = mix(ol[i], l, i - B); r = mix(orr[i], r, i - B); }
+            ol[i] = l; orr[i] = r;
+        }
+    }
+    __device__ __forceinline__ void st2(int i, float2 a, float2 b) const {  // i even
+        if (i >= B) {
+            float2 l = make_float2(__fmul_rn(a.y, gain), __fmul_rn(b.y, gain)), r = make_float2(__fmul_rn(a.x, gain), __fmul_rn(b.x, gain));
+            if (blend) {
+                const float2 la = *reinterpret_cast<const float2*>(ol + i), ra = *reinterpret_cast<const float2*>(orr + i);
+                l = make_float2(mix(la.x, l.x, i - B), mix(la.y, l.y, i + 1 - B));
+                r = make_float2(mix(ra.x, r.x, i - B), mix(ra.y, r.y, i + 1 - B));
+            }
+            *reinterpret_cast<float2*>(ol + i) = l;
+            *reinterpret_cast<float2*>(orr + i) = r;
+        }
+    }
+};
+
+// M: the moving-sources instantiation (render_kernel_moving).  Every block may name its own set; a block whose set
+// differs from the previous block's renders both sets' outputs from the one history and crossfades them (MixStore).
+template <int N, int G, int V, bool M = false>
 __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned char* smem, int stream0, int conv_index) {
     using SM = RenderSmem<N, G, V>;
     const bool conv_on = !SM::kEqOnly && p.conv_enable != 0;   // compile-time false in the EQ-only variant: its transforms are dead code
@@ -955,6 +993,8 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
     auto stream_sync = [&]() { if (T > 32) bar_sync(kBarStream0 + g, T); else __syncwarp(); };
     // the delay line, the history rows and possibly the input rows are what the previous launch wrote
     grid_dependency_wait();
+    int set_prev = 0;   // moving: the set of the block before block t
+    if constexpr (M) { if (valid) set_prev = p.from_set[s]; }
     bar_sync(kBarInitConv, 32 + G * T);   // the staging warp has initialised the mbarriers
     // this stream's block-0 input rows and overlap-save history rows (ring slot 2): two copies each, issued here so
     // that the CTA's streams fetch theirs side by side (stager_warp_main)
@@ -1013,6 +1053,20 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
     for (int t = 0; t < p.n_blocks; ++t) {
         int slot = p.head + t;
         slot -= (slot / p.pmax) * p.pmax;
+        // moving: this block's set; a transition block (set differs from the previous block's) renders the old set's
+        // output as well, so its history product waits until after the forward transform
+        bool trans = false;
+        int set_old = set_prev;
+        if constexpr (M) {
+            if (valid) {
+                const int set = p.block_set ? p.block_set[(size_t)s * p.block_set_stride + t] : p.stream_hrir[s];
+                trans = set != set_prev;
+                set_prev = set;
+                nparts = p.set_parts[set];
+                filt_g = p.filt + (size_t)set * p.pmax * N;
+                filt = p.filt_in_smem ? reinterpret_cast<const float4*>(smem + SM::kFiltOff) : filt_g;
+            }
+        }
         // ---- delay-line history first.  The partitions 1..P-1 of this block's product only need spectra of EARLIER
         // blocks, so their multiply-accumulate (the HBM-heavy part of a long impulse response: P-1 tiles of 8*N bytes per
         // stream) runs BEFORE the wait for this block's EQ output and overlaps the EQ warps' sequential work.  A thread
@@ -1088,7 +1142,7 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
                 }
             }
         } }
-        if (!tma_filters && valid && conv_on && nparts > 1) {
+        if (!tma_filters && valid && conv_on && nparts > 1 && !trans) {
 #pragma unroll 1
             for (int m = 0; m < kPairs; ++m) {
                 const int k = 2 * (tid + m * T);
@@ -1139,7 +1193,8 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
             continue;
         }
         if constexpr (SM::kFusedMac) {
-            if (nparts == 1) {
+            // (moving: not where the delay line must carry every block's spectrum, and not in a transition block)
+            if (nparts == 1 && (!M || (p.pmax == 1 && !trans))) {
                 // ---- single partition: forward passes 1 and 2 through shared memory; then the last forward pass, the
                 // spectral product and the first inverse pass in registers.  The last pass's butterfly i produces the
                 // bins i + q*NB (q < R), exactly the inputs of the inverse transform's first-pass butterfly i, and the
@@ -1197,8 +1252,10 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
         fft_run<N, T>(tid, tw, b0, b1, RingWindow{xp, xc, B, SM::kRingRowR}, zbuf, stream_sync,
                       [&]() { if (release) bar_arrive(kBarEmpty0 + (t & 1), kCount); });
         stream_sync();
-        // ---- this block's spectrum: into the delay line, and its product with partition 0 on top of the history
-        if (nparts > 1) {
+        // ---- this block's spectrum: into the delay line, and its product with partition 0 on top of the history.
+        // (Moving: always.  A later block may move to a set with more partitions than this one's, and a transition
+        // block re-reads it after its first inverse transform.)
+        if (M || nparts > 1) {
             float4* dstz = reinterpret_cast<float4*>(fdl_s + (size_t)slot * N);
 #pragma unroll
             for (int e = 0; e < N / 2 / T; ++e) {
@@ -1228,6 +1285,70 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
                 wbuf.st(m1, make_float2(acc[m][3].y, acc[m][3].x));
             }
         };
+        if constexpr (M) {
+            // Partition 0 reads this block's spectrum back from its delay-line slot (the first inverse transform of a
+            // transition block overwrites both FFT buffers).  A transition block runs two passes: the old set's output
+            // a into the output rows, then the new set's b blended onto it (MixStore); both in the static path's
+            // order, history partitions first (mac_history, the same loop as above), then partition 0.
+            auto mac_history = [&](const float4* fq, int np) {
+#pragma unroll 1
+                for (int m = 0; m < kPairs; ++m) {
+                    const int k = 2 * (tid + m * T);
+                    const int m0 = k ? N - k : N / 2, m1 = N - k - 1;
+                    float2 a4[4] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
+                    int q = 1;
+#pragma unroll 1
+                    for (; q + 3 < np; q += 4) {
+                        Operands o[4];
+#pragma unroll
+                        for (int jq = 0; jq < 4; ++jq) {
+                            int sl = slot - (q + jq); if (sl < 0) sl += p.pmax;
+                            o[jq] = load_ops(fdl_s + (size_t)sl * N, fq + (size_t)(q + jq) * N, k, m0, m1);
+                        }
+#pragma unroll
+                        for (int jq = 0; jq < 4; ++jq) mac_ops(a4, o[jq], k);
+                    }
+#pragma unroll 1
+                    for (; q < np; ++q) {
+                        int sl = slot - q; if (sl < 0) sl += p.pmax;
+                        const Operands o = load_ops(fdl_s + (size_t)sl * N, fq + (size_t)q * N, k, m0, m1);
+                        mac_ops(a4, o, k);
+                    }
+#pragma unroll
+                    for (int mm = 0; mm < kPairs; ++mm)
+                        if (mm == m) { acc[mm][0] = a4[0]; acc[mm][1] = a4[1]; acc[mm][2] = a4[2]; acc[mm][3] = a4[3]; }
+                }
+            };
+            stream_sync();
+            const float2* zs = fdl_s + (size_t)slot * N;
+#pragma unroll 1
+            for (int pass = trans ? 0 : 1; pass < 2; ++pass) {
+                const float4* fq = filt_g;
+                if (trans) {
+                    int np = nparts;
+                    if (pass == 0) { fq = p.filt + (size_t)set_old * p.pmax * N; np = p.set_parts[set_old]; }
+#pragma unroll
+                    for (int m = 0; m < kPairs; ++m)
+#pragma unroll
+                        for (int e = 0; e < 4; ++e) acc[m][e] = make_float2(0.f, 0.f);
+                    if (np > 1) mac_history(fq, np);
+                }
+#pragma unroll
+                for (int m = 0; m < kPairs; ++m) {
+                    const int k = 2 * (tid + m * T);
+                    const int m0 = k ? N - k : N / 2, m1 = N - k - 1;
+                    mac_ops(acc[m], load_ops(zs, fq, k, m0, m1), k);
+                    wbuf.st2(k, make_float2(acc[m][0].y, acc[m][0].x), make_float2(acc[m][1].y, acc[m][1].x));
+                    wbuf.st(m0, make_float2(acc[m][2].y, acc[m][2].x));
+                    wbuf.st(m1, make_float2(acc[m][3].y, acc[m][3].x));
+                }
+                stream_sync();
+                fft_run<N, T>(tid, tw, zbuf.p, wbuf.p, wbuf, MixStore{out_l + (size_t)t * B - B, out_r + (size_t)t * B - B, gain, B, trans && pass == 1},
+                              stream_sync, [&]() {});
+                if (pass == 0) stream_sync();   // both FFT buffers are free again
+            }
+            continue;
+        }
         if (SM::kFiltSmemBytes > 0 && p.filt_in_smem) mac_partition0(reinterpret_cast<const float4*>(smem + SM::kFiltOff));
         else mac_partition0(filt_g);
         stream_sync();
@@ -1272,6 +1393,21 @@ __global__ void __maxnreg__((RenderSmem<N, G, V>::kMaxRegs)) render_kernel(const
     if (warp == SM::kStagerWarpId) { stager_warp_main<N, G, V>(p, smem, stream0); return; }
     const int conv_index = find_conv_index<N, G, V>(warp, std::make_integer_sequence<int, SM::kConvWarps>{});
     if (conv_index >= 0) conv_warps_main<N, G, V>(p, smem, stream0, conv_index);  // other warp slots are placement padding
+}
+
+// Moving sources: the same kernel with per-block HRIR sets and one-block crossfades (conv_warps_main<..., true>).  A
+// kernel of its own, launched only for calls that need it, so that render_kernel's instantiations stay as they are.
+template <int N, int G, int V = 0>
+__global__ void __maxnreg__((RenderSmem<N, G, V>::kMaxRegs)) render_kernel_moving(const RenderParams p) {
+    using SM = RenderSmem<N, G, V>;
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int stream0 = p.first_stream + blockIdx.x * G;
+    launch_dependents();
+    const int warp = threadIdx.x >> 5;
+    if (warp < SM::kEqWarps) { eq_warp_main<N, G, V>(p, smem, stream0, warp); return; }
+    if (warp == SM::kStagerWarpId) { stager_warp_main<N, G, V>(p, smem, stream0); return; }
+    const int conv_index = find_conv_index<N, G, V>(warp, std::make_integer_sequence<int, SM::kConvWarps>{});
+    if (conv_index >= 0) conv_warps_main<N, G, V, true>(p, smem, stream0, conv_index);
 }
 
 }  // namespace ohs

@@ -13,18 +13,20 @@ namespace {
 
 constexpr int N = OHS_RENDER_N;
 
-template <int G, int V> cudaError_t launch_gv(const RenderLaunch& L, const RenderParams& p) {
+// Moving: render_kernel_moving (per-block HRIR sets, crossfaded transitions) instead of render_kernel
+template <int G, int V, bool Moving = false> cudaError_t launch_gv(const RenderLaunch& L, const RenderParams& p) {
     using SM = RenderSmem<N, G, V>;
     if constexpr (!SM::kFits) {
         return cudaErrorInvalidConfiguration;
     } else {
+        constexpr auto kernel = [] { if constexpr (Moving) return render_kernel_moving<N, G, V>; else return render_kernel<N, G, V>; }();
         // function attributes are per device; distinct handles may race here, so the flags are atomic (setting an
         // attribute twice is harmless)
         static std::atomic<unsigned char> attr_set[64];
         if (L.device >= 0 && L.device < 64 && !attr_set[L.device].load(std::memory_order_acquire)) {
-            cudaError_t e = cudaFuncSetAttribute(render_kernel<N, G, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kEqOnly ? 227 * 1024 : (int)SM::kBytes);
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kEqOnly ? 227 * 1024 : (int)SM::kBytes);
             if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(render_kernel<N, G, V>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+            e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             if (e != cudaSuccess) return e;
             attr_set[L.device].store(1, std::memory_order_release);
         }
@@ -42,13 +44,22 @@ template <int G, int V> cudaError_t launch_gv(const RenderLaunch& L, const Rende
         attr[0].val.programmaticStreamSerializationAllowed = L.dependent ? 1 : 0;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        return cudaLaunchKernelEx(&cfg, render_kernel<N, G, V>, q);
+        return cudaLaunchKernelEx(&cfg, kernel, q);
     }
 }
 
 // the latency variant (RenderSmem, V = 1) where it exists and fits, else the throughput variant; the EQ-only variant
-// (V = 2) on request
+// (V = 2) on request.  The moving-sources kernel exists in the throughput and latency variants.
 template <int G> cudaError_t launch_g(const RenderLaunch& L, const RenderParams& p) {
+    if (L.moving) {
+        if (L.variant == 2) return cudaErrorInvalidConfiguration;
+        if constexpr (N == 512) {
+            if constexpr (RenderSmem<N, G, 1>::kFits) {
+                if (L.variant == 1) return launch_gv<G, 1, true>(L, p);
+            }
+        }
+        return launch_gv<G, 0, true>(L, p);
+    }
     if constexpr (N == 512) {
         if (L.variant == 2) {
             if constexpr (RenderSmem<N, G, 2>::kFits) return launch_gv<G, 2>(L, p);

@@ -44,6 +44,7 @@ SYMBOLS = [
     ("ohs_set_ir", C.c_int, [_VP, C.c_int, C.c_int, _f32p, C.c_size_t]),
     ("ohs_num_partitions", C.c_int, [_VP, C.c_int, C.c_int, C.POINTER(C.c_int)]),
     ("ohs_bind_stream_hrir", C.c_int, [_VP, C.c_int, C.c_int]),
+    ("ohs_move_stream_hrir", C.c_int, [_VP, C.c_int, C.c_int]),
     ("ohs_commit_filters", C.c_int, [_VP]),
     ("ohs_filter_table", C.c_int, [_VP, C.POINTER(_VP), C.POINTER(C.c_size_t)]),
     ("ohs_mark_filters_external", C.c_int, [_VP, C.c_int, C.c_int]),
@@ -63,6 +64,7 @@ SYMBOLS = [
     ("ohs_prepare", C.c_int, [_VP, C.c_size_t, C.c_int]),
     ("ohs_debug_trace", C.c_int, [_VP, _VP]),
     ("ohs_process_device", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
+    ("ohs_process_device_scheduled", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t, _VP, C.c_size_t]),
     ("ohs_process", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
     ("ohs_process_fifo", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
     ("ohs_sync", C.c_int, [_VP]),
@@ -229,6 +231,10 @@ class Engine:
     def bind_stream_hrir(self, stream: int, hrir_set: int):
         _check(self._L.ohs_bind_stream_hrir(self._h, stream, hrir_set))
 
+    def move_stream_hrir(self, stream: int, hrir_set: int):
+        """Moving source: the stream's next convolved block crossfades to `hrir_set`, history kept (ohs.h)."""
+        _check(self._L.ohs_move_stream_hrir(self._h, stream, hrir_set))
+
     def commit_filters(self):
         _check(self._L.ohs_commit_filters(self._h))
 
@@ -325,9 +331,18 @@ class Engine:
         _check(self._L.ohs_process_fifo(self._h, x.ctypes.data, y.ctypes.data, x.shape[2], x.shape[2]))
         return y
 
-    def process_device(self, d_in: int, d_out: int, n_frames: int, row_stride: int | None = None):
-        """Device flavour: raw device pointers (e.g. torch.Tensor.data_ptr()); enqueues on the engine's stream."""
-        _check(self._L.ohs_process_device(self._h, d_in, d_out, n_frames, n_frames if row_stride is None else row_stride))
+    def process_device(self, d_in: int, d_out: int, n_frames: int, row_stride: int | None = None, hrir_schedule=None):
+        """Device flavour: raw device pointers (e.g. torch.Tensor.data_ptr()); enqueues on the engine's stream.
+        hrir_schedule: optional int32 array [n_streams, n_blocks >= n_frames / block], the HRIR set of every block of
+        every stream (moving sources, ohs_process_device_scheduled); afterwards each stream is bound to its last column."""
+        rs = n_frames if row_stride is None else row_stride
+        if hrir_schedule is None:
+            _check(self._L.ohs_process_device(self._h, d_in, d_out, n_frames, rs))
+            return
+        sched = np.ascontiguousarray(hrir_schedule, dtype=np.int32)
+        if sched.ndim != 2 or sched.shape[0] != self.n_streams:
+            raise ValueError("hrir_schedule must be [n_streams, n_blocks], got %s" % (sched.shape,))
+        _check(self._L.ohs_process_device_scheduled(self._h, d_in, d_out, n_frames, rs, sched.ctypes.data, sched.shape[1]))
 
     def mix_device(self, d_in: int, d_bus: int, n_frames: int, row_stride: int | None = None, bus_stride: int | None = None):
         """Sum this engine's rendered streams into a stereo bus [2][bus_stride] (config 4 object mixdown)."""
