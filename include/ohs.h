@@ -157,8 +157,8 @@ int ohs_set_time_batch(ohs_engine* h, int enable);
 /* Streams each CTA of the render kernel carries for this handle (which instantiation render_kernel<2*block, G> runs). */
 int ohs_streams_per_cta(ohs_engine* h, int* out);
 /* Set-up that would otherwise happen lazily inside the first process call of that size: uploads pending set_ir /
- * EQ / binding work and allocates the scratch (time-batched route) and, for host_io != 0, the staging buffers that
- * calls of n_frames frames need.  Optional; lets a caller keep allocation out of a timed or real-time region, the
+ * EQ / binding work and allocates the scratch (time-batched route, f32 rows of ohs_process_device_pcm) and, for
+ * host_io != 0, the staging buffers that calls of n_frames frames need (of ohs_process and ohs_process_pcm alike).  Optional; lets a caller keep allocation out of a timed or real-time region, the
  * way Plugin::initialize (src/lib.rs:1124-1150) allocates before process() runs. */
 int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io);
 
@@ -191,6 +191,40 @@ int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, siz
 /* Arbitrary host-block length for ONE-call-per-host-buffer use: the reference's input/output FIFO adaptation
  * (src/dsp/convolution.rs:141-182) including the zero-filled output while fewer than n frames are ready. */
 int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride);
+
+/* ---- integer PCM in and out (an extension: the reference processes f32 only) ------------------------------------
+ * 16- and 24-bit audio converted on the GPU, so the host flavour moves 2 or 3 bytes per sample over PCIe instead of 4.
+ * Layout as above: rows are (stream*2 + channel), row_stride counts FRAMES for both buffers, and row r of a buffer starts
+ * at byte r * row_stride * bytes_per_sample(its format).
+ *   decode   S16: q -> q * 2^-15        S24: q -> q * 2^-23        (both exact in f32)
+ *   render   exactly what ohs_process / ohs_process_device do with the decoded rows (EQ, convolution, gain, the
+ *            time-batched route, pending moves, state); the engine state afterwards is the state after the f32 call on
+ *            the decoded input
+ *   encode   b = 16 / 24:  v = y * 2^(b-1) in f32 (exact for finite y), rounded to nearest with ties to even, clamped to
+ *            [-2^(b-1), 2^(b-1) - 1]; NaN -> 0, +-inf -> the clamp bounds; no dither
+ * so out == encode(render(decode(in))) bit for bit.  OHS_FMT_F32 on a side means no conversion on that side; F32 -> F32
+ * is ohs_process / ohs_process_device.  Bypass: out = encode(decode(in)) (equal formats: the bytes unchanged), state
+ * untouched.  Checked before anything is enqueued (OHS_ERR_INVALID, engine untouched): an unknown format, n_frames not
+ * a multiple of B while the convolution is on, row_stride < n_frames, and in == out or overlapping byte ranges when the
+ * formats differ (in place needs equal formats).  Device flavour: OHS_ERR_ALIGNMENT unless both pointers are 16-byte
+ * aligned and row_stride is a multiple of 4 / 8 / 16 frames for every format involved (F32 / S16 / S24).
+ * The host flavour cuts calls into chunks of about OHS_STAGE_MB per copy of the wider side's rows, so S16 chunks hold
+ * twice the frames of ohs_process's; the block-by-block kernel renders alike however a call is cut, the time-batched
+ * route within round-off.  The device flavour decodes through f32 scratch rows of the engine (up to 256 MiB, allocated
+ * on first use or by ohs_prepare; longer calls go through them in time chunks of whole blocks), except that a call with
+ * f32 output decodes into the output rows and renders them in place.
+ * Not provided: a PCM form of ohs_process_fifo or of ohs_process_device_scheduled, dither, a clip counter, S32 and F64. */
+typedef enum ohs_sample_format {
+    OHS_FMT_F32 = 0,   /* float, as everywhere else in this API */
+    OHS_FMT_S16 = 1,   /* int16_t, little-endian */
+    OHS_FMT_S24 = 2    /* packed 3-byte little-endian two's complement (WAV/FLAC 24-bit), 3 bytes per sample */
+} ohs_sample_format;
+/* host memory; the same contract as ohs_process */
+int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride);
+/* device memory; the same contract as ohs_process_device */
+int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void* d_out, int out_format, size_t n_frames,
+                           size_t row_stride);
+
 int ohs_sync(ohs_engine* h);
 /* The engine's cudaStream_t (as void*) so callers can order their own work / NCCL calls against it. */
 int ohs_cuda_stream(ohs_engine* h, void** stream);

@@ -97,6 +97,12 @@ struct ohs_engine {
     float* d_stage[kPipe] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_in[kPipe] = {}, ev_comp[kPipe] = {}, ev_out[kPipe] = {};
     size_t stage_frames = 0;
+    // ... and its integer-PCM form (ohs_process_pcm): the PCM rows of a chunk, both directions, beside d_stage
+    unsigned char* d_pcm_stage[kPipe] = {nullptr, nullptr, nullptr};
+    size_t pcm_stage_bytes = 0;
+    // f32 rows of ohs_process_device_pcm's time chunks (decoded input, rendered in place)
+    float* d_pcm_scratch = nullptr;
+    size_t pcm_scratch_frames = 0;
 
     // time-batched long-response path: spectra in time order and frequency-domain products of one sub-launch
     float2* d_zlin = nullptr;
@@ -374,6 +380,102 @@ int ensure_stage_buffers(ohs_engine* h, size_t chunk) {
         OHS_CUDA(cudaMalloc(&h->d_stage[i], rows * chunk * sizeof(float)));
     }
     h->stage_frames = chunk;
+    return OHS_OK;
+}
+
+// ---- integer PCM (ohs_process_pcm, ohs_process_device_pcm) --------------------------------------------------------
+size_t pcm_sample_bytes(int fmt) { return fmt == OHS_FMT_S16 ? 2 : fmt == OHS_FMT_S24 ? 3 : 4; }
+// frames in one 16-byte-aligned unit of the format: device rows start 16-byte aligned when the pitch is a multiple
+size_t pcm_align_frames(int fmt) { return fmt == OHS_FMT_S16 ? 8 : fmt == OHS_FMT_S24 ? 16 : 4; }
+size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
+
+int check_pcm_args(ohs_engine* h, const void* in, int in_format, const void* out, int out_format, size_t n_frames, size_t row_stride,
+                   bool device) {
+    for (int f : {in_format, out_format})
+        if (f != OHS_FMT_F32 && f != OHS_FMT_S16 && f != OHS_FMT_S24) return fail(OHS_ERR_INVALID, "unknown sample format %d", f);
+    int rc = check_audio_args(h, in, out, n_frames, row_stride, false);
+    if (rc) return rc;
+    if (in_format != out_format) {
+        // the decode of a later chunk must not read what the encode of an earlier one has written
+        const size_t rows = (size_t)h->cfg.n_streams * 2;
+        const uintptr_t a = (uintptr_t)in, b = (uintptr_t)out;
+        const size_t na = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(in_format);
+        const size_t nb = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(out_format);
+        if (a == b || (a < b + nb && b < a + na))
+            return fail(OHS_ERR_INVALID, "input and output overlap; in place needs equal sample formats");
+    }
+    if (device) {
+        const size_t align = std::max(pcm_align_frames(in_format), pcm_align_frames(out_format));
+        if ((((uintptr_t)in | (uintptr_t)out) & 15u) || row_stride % align)
+            return fail(OHS_ERR_ALIGNMENT, "device PCM pointers must be 16-byte aligned and row_stride a multiple of %zu frames", align);
+    }
+    return OHS_OK;
+}
+
+// PCM rows <-> f32 rows on the engine's stream; pcm_pitch in bytes, f32_pitch in floats
+int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t pcm_pitch, float* f32, size_t f32_pitch, size_t n_frames) {
+    const size_t rows = (size_t)h->cfg.n_streams * 2;
+    const size_t groups = (n_frames + pcm_align_frames(fmt) - 1) / pcm_align_frames(fmt), total = rows * groups;
+    const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
+    if (decode && fmt == OHS_FMT_S16)
+        pcm_decode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
+    else if (decode)
+        pcm_decode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
+    else if (fmt == OHS_FMT_S16)
+        pcm_encode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total);
+    else
+        pcm_encode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total);
+    OHS_CUDA(cudaGetLastError());
+    h->launches++;
+    return OHS_OK;
+}
+
+// frames per chunk of ohs_process_pcm: about stage_bytes per copy of the wider side's rows (the default is a copy-size
+// optimum, tools/e2e_probe.py), whole blocks, at least one block
+size_t pcm_chunk_frames(const ohs_engine* h, size_t n_frames, size_t wide_bytes) {
+    const size_t rows = (size_t)h->cfg.n_streams * 2;
+    size_t chunk = h->stage_bytes / (rows * wide_bytes);
+    chunk = std::max<size_t>(h->B, (chunk / h->B) * h->B);
+    return std::min(chunk, round_up(n_frames, 16));
+}
+
+int ensure_pcm_stage(ohs_engine* h, size_t bytes) {
+    if (bytes <= h->pcm_stage_bytes) return OHS_OK;
+    OHS_CUDA(cudaStreamSynchronize(h->stream));
+    OHS_CUDA(cudaStreamSynchronize(h->d2h));
+    for (int i = 0; i < kPipe; ++i) {
+        if (h->d_pcm_stage[i]) OHS_CUDA(cudaFree(h->d_pcm_stage[i]));
+        h->d_pcm_stage[i] = nullptr;
+        OHS_CUDA(cudaMalloc(&h->d_pcm_stage[i], bytes));
+    }
+    h->pcm_stage_bytes = bytes;
+    return OHS_OK;
+}
+
+// the staging ohs_process_pcm needs for calls of n_frames in any format pair (ohs_prepare): S16 gives the most frames
+// per chunk, the PCM rows of either integer format come to about stage_bytes
+int ensure_pcm_host_staging(ohs_engine* h, size_t n_frames) {
+    const size_t rows = (size_t)h->cfg.n_streams * 2;
+    int rc = ensure_stage_buffers(h, pcm_chunk_frames(h, n_frames, 2));
+    if (rc) return rc;
+    return ensure_pcm_stage(h, rows * std::max(pcm_chunk_frames(h, n_frames, 2) * 2, pcm_chunk_frames(h, n_frames, 3) * 3));
+}
+
+// f32 scratch rows of ohs_process_device_pcm: whole blocks, at most 256 MiB (longer calls go through it in time chunks)
+size_t pcm_scratch_chunk(const ohs_engine* h, size_t n_frames) {
+    const size_t rows = (size_t)h->cfg.n_streams * 2;
+    size_t chunk = ((size_t)256 << 20) / (rows * sizeof(float));
+    chunk = std::max<size_t>(h->B, (chunk / h->B) * h->B);
+    return std::min(chunk, round_up(n_frames, 4));
+}
+
+int ensure_pcm_scratch(ohs_engine* h, size_t frames) {
+    if (frames <= h->pcm_scratch_frames) return OHS_OK;
+    OHS_CUDA(cudaStreamSynchronize(h->stream));
+    if (h->d_pcm_scratch) OHS_CUDA(cudaFree(h->d_pcm_scratch));
+    h->d_pcm_scratch = nullptr; h->pcm_scratch_frames = 0;
+    OHS_CUDA(cudaMalloc(&h->d_pcm_scratch, (size_t)h->cfg.n_streams * 2 * frames * sizeof(float)));
+    h->pcm_scratch_frames = frames;
     return OHS_OK;
 }
 
@@ -836,7 +938,8 @@ int ohs_destroy(ohs_engine* h) {
     for (cudaEvent_t e : {h->ev_fwd[0], h->ev_fwd[1], h->ev_call}) if (e) cudaEventDestroy(e);
     void* ptrs[] = {h->d_stream_hrir, h->d_stream_eq, h->d_stream_gain, h->d_filt, h->d_set_parts, h->d_set_list, h->d_set_flags,
                     h->d_fdl, h->d_prev, h->d_eqc, h->d_eqs, h->d_tw, h->d_ir, h->d_stage[0], h->d_stage[1], h->d_stage[2],
-                    h->d_zlin, h->d_wlin, h->d_xf, h->d_from_set, h->d_sched};
+                    h->d_zlin, h->d_wlin, h->d_xf, h->d_from_set, h->d_sched, h->d_pcm_stage[0], h->d_pcm_stage[1],
+                    h->d_pcm_stage[2], h->d_pcm_scratch};
     for (void* p : ptrs) if (p) cudaFree(p);
     for (int i = 0; i < kPipe; ++i) {
         if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
@@ -1038,6 +1141,12 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io) {
         per_launch = stage_chunk_frames(h, n_frames);
         rc = ensure_stage_buffers(h, per_launch);
         if (rc) return rc;
+        rc = ensure_pcm_host_staging(h, n_frames);   // ohs_process_pcm
+        if (rc) return rc;
+        per_launch = std::max(per_launch, pcm_chunk_frames(h, n_frames, 2));
+    } else if (n_frames) {
+        rc = ensure_pcm_scratch(h, pcm_scratch_chunk(h, n_frames));   // ohs_process_device_pcm
+        if (rc) return rc;
     }
     const int n_blocks = (int)((per_launch + h->B - 1) / h->B);
     if (time_batch_eligible(h, n_blocks)) {
@@ -1169,6 +1278,40 @@ int process_device_impl(ohs_engine* h, const float* d_in, float* d_out, size_t n
     return OHS_OK;
 }
 
+// ohs_process_device_pcm past validation, at least one side an integer format
+int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_format, unsigned char* out, int out_format, size_t n_frames,
+                            size_t row_stride) {
+    if (n_frames == 0) return OHS_OK;
+    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
+    unsigned char* src = const_cast<unsigned char*>(in);   // the decode only reads it
+    if (h->bypass && in_format == out_format) {
+        if (in != out)
+            OHS_CUDA(cudaMemcpy2DAsync(out, row_stride * bo, in, row_stride * bi, n_frames * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
+        return OHS_OK;
+    }
+    if (out_format == OHS_FMT_F32) {   // decode straight into the output rows, render them in place
+        float* y = reinterpret_cast<float*>(out);
+        int rc = launch_pcm(h, true, in_format, src, row_stride * bi, y, row_stride, n_frames);
+        if (rc || h->bypass) return rc;
+        return process_device_impl(h, y, y, n_frames, row_stride, nullptr, 0);
+    }
+    if (in_format == OHS_FMT_F32 && h->bypass)
+        return launch_pcm(h, false, out_format, out, row_stride * bo, reinterpret_cast<float*>(src), row_stride, n_frames);
+    const size_t chunk = pcm_scratch_chunk(h, n_frames);
+    int rc = ensure_pcm_scratch(h, chunk);
+    if (rc) return rc;
+    float* x = h->d_pcm_scratch;
+    for (size_t f0 = 0; f0 < n_frames; f0 += chunk) {
+        const size_t n = std::min(chunk, n_frames - f0), pitch = round_up(n, 4);
+        if (in_format == OHS_FMT_F32)
+            OHS_CUDA(cudaMemcpy2DAsync(x, pitch * sizeof(float), src + f0 * bi, row_stride * bi, n * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
+        else if ((rc = launch_pcm(h, true, in_format, src + f0 * bi, row_stride * bi, x, pitch, n))) return rc;
+        if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
+        if ((rc = launch_pcm(h, false, out_format, out + f0 * bo, row_stride * bo, x, pitch, n))) return rc;
+    }
+    return OHS_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1197,6 +1340,17 @@ int ohs_process_device_scheduled(ohs_engine* h, const float* d_in, float* d_out,
         }
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     return process_device_impl(h, d_in, d_out, n_frames, row_stride, sets, sets_stride);
+}
+
+int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void* d_out, int out_format, size_t n_frames, size_t row_stride) {
+    OHS_CHECK_HANDLE(h);
+    int rc = check_pcm_args(h, d_in, in_format, d_out, out_format, n_frames, row_stride, true);
+    if (rc) return rc;
+    if (in_format == OHS_FMT_F32 && out_format == OHS_FMT_F32)
+        return ohs_process_device(h, static_cast<const float*>(d_in), static_cast<float*>(d_out), n_frames, row_stride);
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    return process_device_pcm_impl(h, static_cast<const unsigned char*>(d_in), in_format, static_cast<unsigned char*>(d_out), out_format,
+                                   n_frames, row_stride);
 }
 
 int ohs_sync(ohs_engine* h) {
@@ -1438,6 +1592,70 @@ int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, siz
         OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
         OHS_CUDA(cudaMemcpy2DAsync(out + done, row_stride * sizeof(float), h->d_stage[b], pitch * sizeof(float), n * sizeof(float), rows,
                                    cudaMemcpyDeviceToHost, h->d2h));
+        OHS_CUDA(cudaEventRecord(h->ev_out[b], h->d2h));
+        used[b] = true;
+        done += n;
+        ++idx;
+    }
+    OHS_CUDA(cudaStreamSynchronize(h->d2h));
+    OHS_CUDA(cudaStreamSynchronize(h->stream));
+    return OHS_OK;
+}
+
+// ohs_process with integer PCM on either side: the same three-slot pipeline, the PCM rows crossing the link and converted
+// in HBM.  Per chunk: copy-in (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into
+// the f32 buffer, render there in place, encode back into the PCM buffer, copy-out.
+int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride) {
+    OHS_CHECK_HANDLE(h);
+    int rc = check_pcm_args(h, in, in_format, out, out_format, n_frames, row_stride, false);
+    if (rc) return rc;
+    if (in_format == OHS_FMT_F32 && out_format == OHS_FMT_F32)
+        return ohs_process(h, static_cast<const float*>(in), static_cast<float*>(out), n_frames, row_stride);
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    if (n_frames == 0) return OHS_OK;
+    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
+    const unsigned char* src = static_cast<const unsigned char*>(in);
+    unsigned char* dst = static_cast<unsigned char*>(out);
+    if (h->bypass && in_format == out_format) {
+        if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(dst + r * row_stride * bo, src + r * row_stride * bi, n_frames * bi);
+        return OHS_OK;
+    }
+    const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32;
+    const size_t chunk = pcm_chunk_frames(h, n_frames, std::max(bi, bo));
+    rc = ensure_stage_buffers(h, chunk);
+    if (rc) return rc;
+    rc = ensure_pcm_stage(h, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0));
+    if (rc) return rc;
+    if (!h->bypass) {
+        rc = commit_filters(h);
+        if (rc) return rc;
+    }
+    OHS_CUDA(cudaStreamSynchronize(h->stream));
+    size_t done = 0;
+    int idx = 0;
+    bool used[kPipe] = {false, false, false};
+    while (done < n_frames) {
+        const size_t n = std::min(chunk, n_frames - done);
+        const size_t pitch = round_up(n, 4), pcm_pitch = round_up(n, 16);   // 16-byte aligned rows in every format
+        const int b = idx % kPipe;
+        float* x = h->d_stage[b];
+        unsigned char* q = h->d_pcm_stage[b];
+        if (used[b]) OHS_CUDA(cudaStreamWaitEvent(h->h2d, h->ev_out[b], 0));  // buffers free once their copy-out finished
+        if (pcm_in)
+            OHS_CUDA(cudaMemcpy2DAsync(q, pcm_pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
+        else
+            OHS_CUDA(cudaMemcpy2DAsync(x, pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
+        OHS_CUDA(cudaEventRecord(h->ev_in[b], h->h2d));
+        OHS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
+        if (pcm_in && (rc = launch_pcm(h, true, in_format, q, pcm_pitch * bi, x, pitch, n))) return rc;
+        if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
+        if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n))) return rc;
+        OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
+        OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
+        if (pcm_out)
+            OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, q, pcm_pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
+        else
+            OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, x, pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
         OHS_CUDA(cudaEventRecord(h->ev_out[b], h->d2h));
         used[b] = true;
         done += n;

@@ -350,4 +350,130 @@ __global__ void mix_streams_kernel(const float* __restrict__ in, float* __restri
     *reinterpret_cast<float4*>(bus + (size_t)c * bus_stride + q * 4) = acc;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Integer PCM in and out (ohs_process_pcm, include/ohs.h): decode q -> q * 2^-(b-1) and encode
+// clamp(rint(y * 2^(b-1))) with NaN -> 0, between PCM rows and f32 rows.  One thread converts one group of frames of one
+// row with 16-byte accesses: 8 frames (one uint4) of S16, 16 frames (48 bytes, three uint4) of S24.  Row starts are
+// 16-byte aligned on both sides (PCM rows: pitch a multiple of the group; f32 rows: of 4 frames); a row's last group
+// may be partial and is converted sample by sample, touching nothing past n_frames.  Launched without the
+// programmatic-serialization attribute: a render launch after a decode starts once the decode has finished, and an
+// encode after a render waits for the whole render.
+// ---------------------------------------------------------------------------------------------------------------
+enum PcmFormat { kPcmF32 = 0, kPcmS16 = 1, kPcmS24 = 2 };   // OHS_FMT_*
+
+template <int Fmt> struct PcmTraits;
+template <> struct PcmTraits<kPcmS16> {
+    static constexpr int kBytes = 2, kGroup = 8;
+    static constexpr float kDecode = 0x1p-15f, kEncode = 0x1p15f, kLo = -32768.0f, kHi = 32767.0f;
+};
+template <> struct PcmTraits<kPcmS24> {
+    static constexpr int kBytes = 3, kGroup = 16;
+    static constexpr float kDecode = 0x1p-23f, kEncode = 0x1p23f, kLo = -8388608.0f, kHi = 8388607.0f;
+};
+
+// y * 2^(b-1) (exact), round to nearest even, clamp (clamping first is the same: the bounds are integers); NaN -> 0
+template <int Fmt> __device__ __forceinline__ int pcm_quantise(float y) {
+    using P = PcmTraits<Fmt>;
+    const float v = y * P::kEncode;
+    if (v != v) return 0;
+    return __float2int_rn(fminf(fmaxf(v, P::kLo), P::kHi));
+}
+
+template <int Fmt> __device__ __forceinline__ int pcm_load_one(const unsigned char* p) {
+    if (Fmt == kPcmS16) return (int)*reinterpret_cast<const short*>(p);
+    return (int)(((unsigned)p[0] | ((unsigned)p[1] << 8) | ((unsigned)p[2] << 16)) << 8) >> 8;
+}
+
+template <int Fmt> __device__ __forceinline__ void pcm_store_one(unsigned char* p, int q) {
+    if (Fmt == kPcmS16) { *reinterpret_cast<short*>(p) = (short)q; return; }
+    p[0] = (unsigned char)q; p[1] = (unsigned char)(q >> 8); p[2] = (unsigned char)(q >> 16);
+}
+
+// the kGroup samples of a whole group from its kGroup * kBytes / 4 little-endian words, and back
+template <int Fmt> __device__ __forceinline__ void pcm_unpack(const unsigned (&w)[PcmTraits<Fmt>::kGroup * PcmTraits<Fmt>::kBytes / 4],
+                                                              int (&q)[PcmTraits<Fmt>::kGroup]) {
+    constexpr int G = PcmTraits<Fmt>::kGroup, NB = PcmTraits<Fmt>::kBytes;
+#pragma unroll
+    for (int k = 0; k < G; ++k) {
+        const int o = k * NB, i = o >> 2, s = o & 3;
+        if (Fmt == kPcmS16) {
+            q[k] = s ? (int)w[i] >> 16 : (int)(short)(w[i] & 0xffffu);
+        } else {
+            const unsigned u = (s <= 1) ? (w[i] >> (8 * s)) : __funnelshift_r(w[i], w[i + 1 < G * NB / 4 ? i + 1 : i], 8 * s);
+            q[k] = (int)(u << 8) >> 8;
+        }
+    }
+}
+
+template <int Fmt> __device__ __forceinline__ void pcm_pack(const int (&q)[PcmTraits<Fmt>::kGroup],
+                                                            unsigned (&w)[PcmTraits<Fmt>::kGroup * PcmTraits<Fmt>::kBytes / 4]) {
+    constexpr int G = PcmTraits<Fmt>::kGroup, NB = PcmTraits<Fmt>::kBytes, W = G * NB / 4;
+#pragma unroll
+    for (int j = 0; j < W; ++j) w[j] = 0u;
+#pragma unroll
+    for (int k = 0; k < G; ++k) {
+        const int o = k * NB, i = o >> 2, s = o & 3;
+        const unsigned u = (unsigned)q[k] & (NB == 2 ? 0xffffu : 0xffffffu);
+        w[i] |= u << (8 * s);
+        if (8 * s + 8 * NB > 32) w[i + 1 < W ? i + 1 : i] |= u >> (32 - 8 * s);
+    }
+}
+
+// in: PCM rows (pitch in bytes), out: f32 rows (pitch in floats); `groups` = groups per row
+template <int Fmt>
+__global__ void __launch_bounds__(256) pcm_decode_kernel(const unsigned char* __restrict__ in, size_t in_pitch, float* __restrict__ out,
+                                                         size_t out_pitch, size_t n_frames, size_t groups, size_t total) {
+    using P = PcmTraits<Fmt>;
+    constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const size_t row = t / groups, f0 = (t - row * groups) * G;
+        const unsigned char* src = in + row * in_pitch + f0 * NB;
+        float* dst = out + row * out_pitch + f0;
+        if (f0 + G <= n_frames) {
+            unsigned w[W];
+#pragma unroll
+            for (int v = 0; v < W / 4; ++v) {
+                const uint4 x = reinterpret_cast<const uint4*>(src)[v];
+                w[4 * v] = x.x; w[4 * v + 1] = x.y; w[4 * v + 2] = x.z; w[4 * v + 3] = x.w;
+            }
+            int q[G];
+            pcm_unpack<Fmt>(w, q);
+#pragma unroll
+            for (int v = 0; v < G / 4; ++v)
+                reinterpret_cast<float4*>(dst)[v] = make_float4((float)q[4 * v] * P::kDecode, (float)q[4 * v + 1] * P::kDecode,
+                                                                (float)q[4 * v + 2] * P::kDecode, (float)q[4 * v + 3] * P::kDecode);
+        } else {
+            for (size_t k = 0; f0 + k < n_frames; ++k) dst[k] = (float)pcm_load_one<Fmt>(src + k * NB) * P::kDecode;
+        }
+    }
+}
+
+// in: f32 rows (pitch in floats), out: PCM rows (pitch in bytes)
+template <int Fmt>
+__global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict__ in, size_t in_pitch, unsigned char* __restrict__ out,
+                                                         size_t out_pitch, size_t n_frames, size_t groups, size_t total) {
+    using P = PcmTraits<Fmt>;
+    constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const size_t row = t / groups, f0 = (t - row * groups) * G;
+        const float* src = in + row * in_pitch + f0;
+        unsigned char* dst = out + row * out_pitch + f0 * NB;
+        if (f0 + G <= n_frames) {
+            int q[G];
+#pragma unroll
+            for (int v = 0; v < G / 4; ++v) {
+                const float4 y = reinterpret_cast<const float4*>(src)[v];
+                q[4 * v] = pcm_quantise<Fmt>(y.x); q[4 * v + 1] = pcm_quantise<Fmt>(y.y);
+                q[4 * v + 2] = pcm_quantise<Fmt>(y.z); q[4 * v + 3] = pcm_quantise<Fmt>(y.w);
+            }
+            unsigned w[W];
+            pcm_pack<Fmt>(q, w);
+#pragma unroll
+            for (int v = 0; v < W / 4; ++v) reinterpret_cast<uint4*>(dst)[v] = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
+        } else {
+            for (size_t k = 0; f0 + k < n_frames; ++k) pcm_store_one<Fmt>(dst + k * NB, pcm_quantise<Fmt>(src[k]));
+        }
+    }
+}
+
 }  // namespace ohs

@@ -19,6 +19,7 @@ OHS_ALL = -1
 ABI_VERSION = 2   # OHS_ABI_VERSION of include/ohs.h this binding was written against
 LSL, LSR, RSL, RSR = 0, 1, 2, 3
 PEAK, LOWSHELF, HIGHSHELF, LOWPASS, HIGHPASS, BANDPASS, NOTCH, ALLPASS = range(8)
+FMT_F32, FMT_S16, FMT_S24 = 0, 1, 2   # ohs_sample_format
 
 _f32p = C.POINTER(C.c_float)
 
@@ -67,6 +68,8 @@ SYMBOLS = [
     ("ohs_process_device_scheduled", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t, _VP, C.c_size_t]),
     ("ohs_process", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
     ("ohs_process_fifo", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
+    ("ohs_process_pcm", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_int, C.c_size_t, C.c_size_t]),
+    ("ohs_process_device_pcm", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_int, C.c_size_t, C.c_size_t]),
     ("ohs_sync", C.c_int, [_VP]),
     ("ohs_cuda_stream", C.c_int, [_VP, C.POINTER(_VP)]),
     ("ohs_launch_count", C.c_int, [_VP, C.POINTER(C.c_uint64)]),
@@ -168,14 +171,16 @@ class Comm:
 
 
 class PinnedBuffer:
-    """cudaHostAlloc'd float32 array (ohs_host_alloc) viewed as numpy."""
+    """cudaHostAlloc'd array (ohs_host_alloc) viewed as numpy; float32 unless another dtype is given."""
 
-    def __init__(self, shape):
+    def __init__(self, shape, dtype=np.float32):
         self.shape = tuple(int(s) for s in shape)
+        dtype = np.dtype(dtype)
         n = int(np.prod(self.shape))
         self._ptr = _VP()
-        _check(load_library().ohs_host_alloc(C.byref(self._ptr), n * 4))
-        self.array = np.ctypeslib.as_array(C.cast(self._ptr, _f32p), shape=(n,)).reshape(self.shape)
+        _check(load_library().ohs_host_alloc(C.byref(self._ptr), n * dtype.itemsize))
+        raw = np.ctypeslib.as_array(C.cast(self._ptr, C.POINTER(C.c_uint8)), shape=(n * dtype.itemsize,))
+        self.array = raw.view(dtype).reshape(self.shape)
 
     def free(self):
         if self._ptr:
@@ -323,6 +328,40 @@ class Engine:
                 raise ValueError("out must be a writeable C-contiguous float32 array of shape %s" % (x.shape,))
         _check(self._L.ohs_process(self._h, x.ctypes.data, y.ctypes.data, x.shape[2], x.shape[2]))
         return y
+
+    def process_pcm(self, x, out_format: int, out=None) -> np.ndarray:
+        """Host flavour with integer PCM (ohs_process_pcm).  The input format follows the dtype: int16 [S, 2, n] is S16,
+        float32 [S, 2, n] is F32, uint8 [S, 2, 3n] is packed S24 (signals.pack_s24).  Returns int16 [S, 2, n] for
+        FMT_S16, uint8 [S, 2, 3n] for FMT_S24, float32 [S, 2, n] for FMT_F32 (or fills `out`, e.g. a PinnedBuffer's array)."""
+        x = np.asarray(x)
+        if x.ndim != 3 or x.shape[0] != self.n_streams or x.shape[1] != 2:
+            raise ValueError("x must be [n_streams, 2, frames], got %s" % (x.shape,))
+        if x.dtype == np.int16:
+            fmt, n = FMT_S16, x.shape[2]
+        elif x.dtype == np.float32:
+            fmt, n = FMT_F32, x.shape[2]
+        elif x.dtype == np.uint8 and x.shape[2] % 3 == 0:
+            fmt, n = FMT_S24, x.shape[2] // 3
+        else:
+            raise ValueError("process_pcm takes int16, float32 or packed 24-bit uint8 [S, 2, 3n] input, got %s %s" % (x.dtype, x.shape))
+        shape = {FMT_F32: (n, np.float32), FMT_S16: (n, np.int16), FMT_S24: (3 * n, np.uint8)}
+        if out_format not in shape:
+            raise ValueError("unknown sample format %r" % (out_format,))
+        x = np.ascontiguousarray(x)
+        want = ((self.n_streams, 2, shape[out_format][0]), np.dtype(shape[out_format][1]))
+        if out is None:
+            y = np.empty(*want)
+        else:
+            y = out
+            if not (isinstance(y, np.ndarray) and (y.shape, y.dtype) == want and y.flags["C_CONTIGUOUS"] and y.flags["WRITEABLE"]):
+                raise ValueError("out must be a writeable C-contiguous %s array of shape %s" % (want[1], want[0]))
+        _check(self._L.ohs_process_pcm(self._h, x.ctypes.data, fmt, y.ctypes.data, out_format, n, n))
+        return y
+
+    def process_device_pcm(self, d_in: int, in_format: int, d_out: int, out_format: int, n_frames: int, row_stride: int | None = None):
+        """Device flavour of process_pcm on raw device pointers; row_stride counts frames for both buffers."""
+        _check(self._L.ohs_process_device_pcm(self._h, d_in, in_format, d_out, out_format, n_frames,
+                                              n_frames if row_stride is None else row_stride))
 
     def process_fifo(self, x) -> np.ndarray:
         x = _f32(x)

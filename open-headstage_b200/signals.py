@@ -67,6 +67,42 @@ def synthetic_hrir_set(taps: int, decay: float, seed: int = 7) -> np.ndarray:
     return h.astype(np.float32)
 
 
+def pack_s24(q) -> np.ndarray:
+    """int32 samples in [-2^23, 2^23) -> packed 3-byte little-endian two's complement (WAV/FLAC 24-bit): the last axis
+    grows threefold, uint8."""
+    q = np.asarray(q, dtype=np.int32)
+    b = q.astype("<i4").view(np.uint8).reshape(q.shape + (4,))[..., :3]
+    return np.ascontiguousarray(b).reshape(q.shape[:-1] + (3 * q.shape[-1],))
+
+
+def unpack_s24(b) -> np.ndarray:
+    """Packed 24-bit bytes (last axis 3n) -> int32 samples, sign-extended."""
+    b = np.asarray(b, dtype=np.uint8)
+    t = b.reshape(b.shape[:-1] + (b.shape[-1] // 3, 3)).astype(np.int32)
+    v = t[..., 0] | (t[..., 1] << 8) | (t[..., 2] << 16)
+    return (v ^ 0x800000) - 0x800000
+
+
+# PCM formats of ohs_process_pcm (include/ohs.h): bits per sample
+PCM_BITS = {1: 16, 2: 24}
+
+
+def pcm_decode(q, fmt: int) -> np.ndarray:
+    """q * 2^-(b-1) as float32 (exact); q: int samples (S16) or int32 samples (S24, unpacked)."""
+    return (np.asarray(q).astype(np.float32) * np.float32(2.0 ** (1 - PCM_BITS[fmt]))).astype(np.float32)
+
+
+def pcm_encode(y, fmt: int) -> np.ndarray:
+    """The encode of include/ohs.h: v = y * 2^(b-1) in f32, round to nearest even, clamp to [-2^(b-1), 2^(b-1) - 1],
+    NaN -> 0.  int16 for S16, int32 (unpacked) for S24."""
+    b = PCM_BITS[fmt]
+    v = np.asarray(y, dtype=np.float32) * np.float32(2.0 ** (b - 1))
+    with np.errstate(invalid="ignore"):
+        r = np.clip(np.rint(v), -(2.0 ** (b - 1)), 2.0 ** (b - 1) - 1)
+    r = np.where(np.isnan(v), np.float32(0.0), r)
+    return r.astype(np.int16 if fmt == 1 else np.int32)
+
+
 # BASELINE.json configs -> engine parameters (SURVEY.md §8d table)
 CONFIGS = {
     1: dict(name="cfg1: 1 stereo stream, 48 kHz, SOFA 200-tap HRIR, block 512", n_streams=1, fs=48000.0, block=512, taps=200),
