@@ -93,16 +93,16 @@ struct ohs_engine {
     unsigned long long* d_trace = nullptr;  // ohs_debug_trace (OHS_TRACE builds)
     std::vector<float> h_ir_padded;         // [set][4][pmax*B] host mirror of d_ir, uploaded in one copy per commit
 
-    // host-pointer path
+    // host-pointer path (grow-only buffers: *_cap is the bytes allocated per buffer, see grow_buffers)
     float* d_stage[kPipe] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_in[kPipe] = {}, ev_comp[kPipe] = {}, ev_out[kPipe] = {};
-    size_t stage_frames = 0;
-    // ... and its integer-PCM form (ohs_process_pcm): the PCM rows of a chunk, both directions, beside d_stage
+    size_t stage_cap = 0;
+    // ... and its integer-PCM rows: the PCM rows of a chunk, both directions, beside d_stage
     unsigned char* d_pcm_stage[kPipe] = {nullptr, nullptr, nullptr};
-    size_t pcm_stage_bytes = 0;
+    size_t pcm_stage_cap = 0;
     // f32 rows of ohs_process_device_pcm's time chunks (decoded input, rendered in place)
     float* d_pcm_scratch = nullptr;
-    size_t pcm_scratch_frames = 0;
+    size_t pcm_scratch_cap = 0;
 
     // time-batched long-response path: spectra in time order and frequency-domain products of one sub-launch
     float2* d_zlin = nullptr;
@@ -137,7 +137,7 @@ struct ohs_engine {
     bool any_move = false;
     int* d_from_set = nullptr;
     int* d_sched = nullptr;
-    size_t sched_cap = 0;   // ints
+    size_t sched_cap = 0;   // bytes
 };
 
 namespace {
@@ -360,26 +360,32 @@ int check_audio_args(ohs_engine* h, const void* in, const void* out, size_t n_fr
     return OHS_OK;
 }
 
-// called once, from ohs_create (the only place the environment is consulted)
-// frames per staging chunk of the host-pointer path: whole blocks, about stage_bytes per buffer, at least one block
-size_t stage_chunk_frames(const ohs_engine* h, size_t n_frames) {
+size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
+
+// Frames per chunk of a call of n_frames: about budget_bytes of rows at bytes_per_sample, whole blocks, at least one
+// block.  The cap (the call rounded up to 16 frames) only sizes allocations: callers take min(chunk, frames left), so the
+// chunk boundaries are those of the uncapped rule.  The cap keeps every row pitch, round_up(n, 4) of f32 rows and
+// round_up(n, 16) of PCM rows, within an allocation of chunk frames (a block is a multiple of 16 frames).
+size_t chunk_frames(const ohs_engine* h, size_t n_frames, size_t budget_bytes, size_t bytes_per_sample) {
     const size_t rows = (size_t)h->cfg.n_streams * 2;
-    size_t chunk = h->stage_bytes / (rows * sizeof(float));
-    chunk = std::max<size_t>(h->B, (chunk / h->B) * h->B);
-    return std::min(chunk, (n_frames + 3) / 4 * 4);
+    const size_t chunk = std::max<size_t>(h->B, budget_bytes / (rows * bytes_per_sample) / h->B * h->B);
+    return std::min(chunk, round_up(n_frames, 16));
 }
 
-int ensure_stage_buffers(ohs_engine* h, size_t chunk) {
-    if (chunk <= h->stage_frames) return OHS_OK;
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
+// Grows the n buffers bufs[0..n) to `bytes` each unless `cap` (the bytes each holds) is enough already.  Work enqueued
+// earlier may still use the old buffers, hence the syncs.  `cap` is 0 from the first free until every allocation has
+// succeeded, so after a failed cudaMalloc the next call allocates again rather than use a freed or null buffer.
+template <typename T> int grow_buffers(ohs_engine* h, T** bufs, int n, size_t& cap, size_t bytes) {
+    if (bytes <= cap) return OHS_OK;
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     OHS_CUDA(cudaStreamSynchronize(h->d2h));
-    for (int i = 0; i < kPipe; ++i) {
-        if (h->d_stage[i]) OHS_CUDA(cudaFree(h->d_stage[i]));
-        h->d_stage[i] = nullptr;
-        OHS_CUDA(cudaMalloc(&h->d_stage[i], rows * chunk * sizeof(float)));
+    cap = 0;
+    for (int i = 0; i < n; ++i) {
+        if (bufs[i]) OHS_CUDA(cudaFree(bufs[i]));
+        bufs[i] = nullptr;
+        OHS_CUDA(cudaMalloc(&bufs[i], bytes));
     }
-    h->stage_frames = chunk;
+    cap = bytes;
     return OHS_OK;
 }
 
@@ -387,7 +393,6 @@ int ensure_stage_buffers(ohs_engine* h, size_t chunk) {
 size_t pcm_sample_bytes(int fmt) { return fmt == OHS_FMT_S16 ? 2 : fmt == OHS_FMT_S24 ? 3 : 4; }
 // frames in one 16-byte-aligned unit of the format: device rows start 16-byte aligned when the pitch is a multiple
 size_t pcm_align_frames(int fmt) { return fmt == OHS_FMT_S16 ? 8 : fmt == OHS_FMT_S24 ? 16 : 4; }
-size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
 int check_pcm_args(ohs_engine* h, const void* in, int in_format, const void* out, int out_format, size_t n_frames, size_t row_stride,
                    bool device) {
@@ -430,55 +435,13 @@ int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t p
     return OHS_OK;
 }
 
-// frames per chunk of ohs_process_pcm: about stage_bytes per copy of the wider side's rows (the default is a copy-size
-// optimum, tools/e2e_probe.py), whole blocks, at least one block
-size_t pcm_chunk_frames(const ohs_engine* h, size_t n_frames, size_t wide_bytes) {
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
-    size_t chunk = h->stage_bytes / (rows * wide_bytes);
-    chunk = std::max<size_t>(h->B, (chunk / h->B) * h->B);
-    return std::min(chunk, round_up(n_frames, 16));
-}
-
-int ensure_pcm_stage(ohs_engine* h, size_t bytes) {
-    if (bytes <= h->pcm_stage_bytes) return OHS_OK;
-    OHS_CUDA(cudaStreamSynchronize(h->stream));
-    OHS_CUDA(cudaStreamSynchronize(h->d2h));
-    for (int i = 0; i < kPipe; ++i) {
-        if (h->d_pcm_stage[i]) OHS_CUDA(cudaFree(h->d_pcm_stage[i]));
-        h->d_pcm_stage[i] = nullptr;
-        OHS_CUDA(cudaMalloc(&h->d_pcm_stage[i], bytes));
-    }
-    h->pcm_stage_bytes = bytes;
-    return OHS_OK;
-}
-
-// the staging ohs_process_pcm needs for calls of n_frames in any format pair (ohs_prepare): S16 gives the most frames
-// per chunk, the PCM rows of either integer format come to about stage_bytes
-int ensure_pcm_host_staging(ohs_engine* h, size_t n_frames) {
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
-    int rc = ensure_stage_buffers(h, pcm_chunk_frames(h, n_frames, 2));
-    if (rc) return rc;
-    return ensure_pcm_stage(h, rows * std::max(pcm_chunk_frames(h, n_frames, 2) * 2, pcm_chunk_frames(h, n_frames, 3) * 3));
-}
-
 // f32 scratch rows of ohs_process_device_pcm: whole blocks, at most 256 MiB (longer calls go through it in time chunks)
-size_t pcm_scratch_chunk(const ohs_engine* h, size_t n_frames) {
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
-    size_t chunk = ((size_t)256 << 20) / (rows * sizeof(float));
-    chunk = std::max<size_t>(h->B, (chunk / h->B) * h->B);
-    return std::min(chunk, round_up(n_frames, 4));
-}
-
+constexpr size_t kPcmScratchBytes = (size_t)256 << 20;
 int ensure_pcm_scratch(ohs_engine* h, size_t frames) {
-    if (frames <= h->pcm_scratch_frames) return OHS_OK;
-    OHS_CUDA(cudaStreamSynchronize(h->stream));
-    if (h->d_pcm_scratch) OHS_CUDA(cudaFree(h->d_pcm_scratch));
-    h->d_pcm_scratch = nullptr; h->pcm_scratch_frames = 0;
-    OHS_CUDA(cudaMalloc(&h->d_pcm_scratch, (size_t)h->cfg.n_streams * 2 * frames * sizeof(float)));
-    h->pcm_scratch_frames = frames;
-    return OHS_OK;
+    return grow_buffers(h, &h->d_pcm_scratch, 1, h->pcm_scratch_cap, (size_t)h->cfg.n_streams * 2 * frames * sizeof(float));
 }
 
+// called once, from ohs_create (the only place the environment is consulted)
 int pick_streams_per_cta(const ohs_engine* h) {
     if (const char* e = getenv("OHS_STREAMS_PER_CTA")) {
         const int g = atoi(e);
@@ -1138,14 +1101,16 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io) {
     if (rc) return rc;
     size_t per_launch = n_frames;
     if (host_io) {
-        per_launch = stage_chunk_frames(h, n_frames);
-        rc = ensure_stage_buffers(h, per_launch);
-        if (rc) return rc;
-        rc = ensure_pcm_host_staging(h, n_frames);   // ohs_process_pcm
-        if (rc) return rc;
-        per_launch = std::max(per_launch, pcm_chunk_frames(h, n_frames, 2));
+        // the widest chunk of ohs_process_pcm over every format pair: S16 has the most frames per chunk, which size the
+        // f32 slots; the PCM slots hold the larger of the S16 and S24 rows
+        const size_t rows = (size_t)h->cfg.n_streams * 2;
+        per_launch = chunk_frames(h, n_frames, h->stage_bytes, 2);
+        const size_t pcm_bytes = rows * std::max(per_launch * 2, chunk_frames(h, n_frames, h->stage_bytes, 3) * 3);
+        if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * per_launch * sizeof(float))) ||
+            (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, pcm_bytes)))
+            return rc;
     } else if (n_frames) {
-        rc = ensure_pcm_scratch(h, pcm_scratch_chunk(h, n_frames));   // ohs_process_device_pcm
+        rc = ensure_pcm_scratch(h, chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float)));   // ohs_process_device_pcm
         if (rc) return rc;
     }
     const int n_blocks = (int)((per_launch + h->B - 1) / h->B);
@@ -1223,13 +1188,8 @@ int process_device_impl(ohs_engine* h, const float* d_in, float* d_out, size_t n
             }
         }
         if (transition) {
-            if (S * K > h->sched_cap) {
-                OHS_CUDA(cudaStreamSynchronize(h->stream));   // an earlier launch may still read the old buffer
-                if (h->d_sched) OHS_CUDA(cudaFree(h->d_sched));
-                h->d_sched = nullptr; h->sched_cap = 0;
-                OHS_CUDA(cudaMalloc(&h->d_sched, sizeof(int) * S * K));
-                h->sched_cap = S * K;
-            }
+            rc = grow_buffers(h, &h->d_sched, 1, h->sched_cap, sizeof(int) * S * K);
+            if (rc) return rc;
             OHS_CUDA(cudaMemcpy2DAsync(h->d_sched, sizeof(int) * K, sets, sizeof(int) * sets_stride, sizeof(int) * K, S,
                                        cudaMemcpyHostToDevice, h->stream));
             p.block_set = h->d_sched; p.block_set_stride = (long long)K;
@@ -1297,7 +1257,7 @@ int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_forma
     }
     if (in_format == OHS_FMT_F32 && h->bypass)
         return launch_pcm(h, false, out_format, out, row_stride * bo, reinterpret_cast<float*>(src), row_stride, n_frames);
-    const size_t chunk = pcm_scratch_chunk(h, n_frames);
+    const size_t chunk = chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float));
     int rc = ensure_pcm_scratch(h, chunk);
     if (rc) return rc;
     float* x = h->d_pcm_scratch;
@@ -1553,64 +1513,14 @@ int ohs_host_free(void* p) {
     return OHS_OK;
 }
 
-// Host-pointer flavour: time chunks are staged through three HBM buffers; copy-in, kernel and copy-out of
-// consecutive chunks overlap on three CUDA streams.
-int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride) {
-    OHS_CHECK_HANDLE(h);
-    int rc = check_audio_args(h, in, out, n_frames, row_stride, false);
-    if (rc) return rc;
-    OHS_CUDA(cudaSetDevice(h->cfg.device));
-    if (n_frames == 0) return OHS_OK;
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
-    if (h->bypass) {
-        if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(out + r * row_stride, in + r * row_stride, n_frames * sizeof(float));
-        return OHS_OK;
-    }
-    // chunk: whole blocks, about 24 MiB per staging buffer, at least one block
-    // 24 MiB by default: measured best on PCIe Gen5 x16 with both directions busy (tools/e2e_probe.py)
-    const size_t chunk = stage_chunk_frames(h, n_frames);
-    rc = ensure_stage_buffers(h, chunk);
-    if (rc) return rc;
-    rc = commit_filters(h);
-    if (rc) return rc;
-    OHS_CUDA(cudaStreamSynchronize(h->stream));
-    size_t done = 0;
-    int idx = 0;
-    bool used[kPipe] = {false, false, false};
-    while (done < n_frames) {
-        const size_t n = std::min(chunk, n_frames - done);
-        const size_t pitch = (n + 3) / 4 * 4;  // device rows stay 16-byte aligned for a ragged EQ-only tail
-        const int b = idx % kPipe;
-        if (used[b]) OHS_CUDA(cudaStreamWaitEvent(h->h2d, h->ev_out[b], 0));  // buffer free once its copy-out finished
-        OHS_CUDA(cudaMemcpy2DAsync(h->d_stage[b], pitch * sizeof(float), in + done, row_stride * sizeof(float), n * sizeof(float), rows,
-                                   cudaMemcpyHostToDevice, h->h2d));
-        OHS_CUDA(cudaEventRecord(h->ev_in[b], h->h2d));
-        OHS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-        rc = ohs_process_device(h, h->d_stage[b], h->d_stage[b], n, pitch);
-        if (rc) return rc;
-        OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
-        OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
-        OHS_CUDA(cudaMemcpy2DAsync(out + done, row_stride * sizeof(float), h->d_stage[b], pitch * sizeof(float), n * sizeof(float), rows,
-                                   cudaMemcpyDeviceToHost, h->d2h));
-        OHS_CUDA(cudaEventRecord(h->ev_out[b], h->d2h));
-        used[b] = true;
-        done += n;
-        ++idx;
-    }
-    OHS_CUDA(cudaStreamSynchronize(h->d2h));
-    OHS_CUDA(cudaStreamSynchronize(h->stream));
-    return OHS_OK;
-}
-
-// ohs_process with integer PCM on either side: the same three-slot pipeline, the PCM rows crossing the link and converted
-// in HBM.  Per chunk: copy-in (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into
-// the f32 buffer, render there in place, encode back into the PCM buffer, copy-out.
+// Host-pointer flavour: time chunks are staged through three slots in HBM; copy-in, kernels and copy-out of consecutive
+// chunks overlap on three CUDA streams.  Integer PCM crosses the link as PCM and is converted in HBM.  Per chunk: copy-in
+// (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into the f32 buffer, render
+// there in place, encode back into the PCM buffer, copy-out.  ohs_process is the F32 -> F32 case.
 int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride) {
     OHS_CHECK_HANDLE(h);
     int rc = check_pcm_args(h, in, in_format, out, out_format, n_frames, row_stride, false);
     if (rc) return rc;
-    if (in_format == OHS_FMT_F32 && out_format == OHS_FMT_F32)
-        return ohs_process(h, static_cast<const float*>(in), static_cast<float*>(out), n_frames, row_stride);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     if (n_frames == 0) return OHS_OK;
     const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
@@ -1621,11 +1531,12 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
         return OHS_OK;
     }
     const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32;
-    const size_t chunk = pcm_chunk_frames(h, n_frames, std::max(bi, bo));
-    rc = ensure_stage_buffers(h, chunk);
-    if (rc) return rc;
-    rc = ensure_pcm_stage(h, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0));
-    if (rc) return rc;
+    // about stage_bytes per copy of the wider side's rows: 24 MiB by default, measured best on PCIe Gen5 x16 with both
+    // directions busy (tools/e2e_probe.py)
+    const size_t chunk = chunk_frames(h, n_frames, h->stage_bytes, std::max(bi, bo));
+    if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * chunk * sizeof(float))) ||
+        (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0))))
+        return rc;
     if (!h->bypass) {
         rc = commit_filters(h);
         if (rc) return rc;
@@ -1664,6 +1575,10 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     OHS_CUDA(cudaStreamSynchronize(h->d2h));
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     return OHS_OK;
+}
+
+int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride) {
+    return ohs_process_pcm(h, in, OHS_FMT_F32, out, OHS_FMT_F32, n_frames, row_stride);
 }
 
 // The reference's FIFO adaptation around whole engine blocks (src/dsp/convolution.rs:141-182): append the host block,
