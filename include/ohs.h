@@ -138,6 +138,8 @@ int ohs_eq_design(int filter_type, float fs, float fc, float q, float gain_db, f
 int ohs_eq_update_band(ohs_engine* h, int eq_set, int band, int filter_type, float fc, float q, float gain_db, int enabled);
 /* Same, with the five coefficients supplied as data. */
 int ohs_eq_set_band(ohs_engine* h, int eq_set, int band, const float coeffs[5], int enabled);
+/* Bind a stream (or OHS_ALL) to an EQ set from its next call on.  The stream's biquad state is kept: the new set's bands
+ * continue from the state the old set's bands left, as if update_band_coeffs had been called on every band. */
 int ohs_bind_stream_eq(ohs_engine* h, int stream, int eq_set);
 /* StereoParametricEQ::reset_all_bands_state (src/dsp/parametric_eq.rs:181-188; Plugin::reset src/lib.rs:1152-1154). */
 int ohs_eq_reset(ohs_engine* h);
