@@ -144,7 +144,7 @@ namespace {
 
 using namespace ohs;
 
-// moving: render_kernel_moving (p.from_set set, p.block_set optional)
+// moving: the moving-sources kernel, render_kernel<..., true> (p.from_set set, p.block_set optional)
 int launch_render(ohs_engine* h, const RenderParams& p, int first_stream = 0, bool moving = false) {
     // few blocks per launch: nothing overlaps inside the launch, so the variant built for latency runs it
     const bool latency = p.n_blocks <= h->latency_blocks;
@@ -1140,7 +1140,7 @@ namespace {
 
 // A multi-set engine with a delay line where some stream is bound to a one-partition set: render_kernel does not put
 // that stream's spectra into the delay line (it never reads them), but a later move to a longer set needs them, so
-// such calls run render_kernel_moving, which writes every block's.  Same outputs, more delay-line traffic.
+// such calls run the moving-sources kernel, which writes every block's.  Same outputs, more delay-line traffic.
 bool needs_full_ring(const ohs_engine* h) {
     if (h->pmax == 1 || h->cfg.n_hrir_sets == 1) return false;
     for (int set : h->h_stream_hrir) if (h->h_set_parts[set] == 1) return true;

@@ -44,8 +44,9 @@ constexpr int kMaxBands = 10;
 // stream-s/s) for more issue slots.
 // Placement weight of an EQ warp in units of a convolution warp (RenderSmem::place).  Round 2 re-measurement on config 2
 // (profiles/r02_ab_placement.txt): weight 3 -> (1, 1, 1, 4) convolution warps next to the three EQ warps, 16 warp
-// slots, 128 registers per thread, no spills: 1.081 M stream-s/s; weight 4 -> (0, 1, 1, 5), 20 warp slots, 96
-// registers, 360 bytes of spills in the convolution warps: 1.003 M; weight 5: 0.920 M.
+// slots, 128 registers per thread: 1.081 M stream-s/s; weight 4 -> (0, 1, 1, 5), 20 warp slots, 96 registers, 360
+// bytes of spills in the convolution warps: 1.003 M; weight 5: 0.920 M.  (ptxas 12.9 reports 128 registers and 224 B
+// of spill stores and loads for today's render_kernel<512, 7, 0>.)
 #ifndef OHS_EQ_WEIGHT
 #define OHS_EQ_WEIGHT 3
 #endif
@@ -88,7 +89,7 @@ struct RenderParams {
     int first_stream;           // CTA 0 renders streams first_stream .. first_stream+G-1 (set by the launcher)
     int io_first_stream;        // the stream whose rows sit at in/out row 0 (host staging by stream range), else 0
     unsigned long long* trace;  // OHS_TRACE builds: [CTA][16] clock64 stamps of the launch's milestones, else unused
-    // moving sources (render_kernel_moving only; DESIGN §10): the set of block t is block_set[s*block_set_stride + t],
+    // moving sources (render_kernel<..., true> only; DESIGN §10): the set of block t is block_set[s*block_set_stride + t],
     // or stream_hrir[s] for every block when block_set is null; from_set[s] is the set of the block before block 0
     const int* from_set;
     const int* block_set;
@@ -248,6 +249,16 @@ struct SmemCx {
     __device__ __forceinline__ void st(int i, float2 v) const { p[padi(i)] = v; }
     __device__ __forceinline__ void st2(int i, float2 a, float2 b) const {
         *reinterpret_cast<float4*>(p + padi(i)) = make_float4(a.x, a.y, b.x, b.y);
+    }
+};
+
+// the loads of SmemCx over an unpadded spectrum in global memory (a delay-line slot)
+struct GlobalCx {
+    const float2* p;
+    __device__ __forceinline__ float2 ld(int i) const { return p[i]; }
+    __device__ __forceinline__ void ld2(int i, float2& a, float2& b) const {
+        const float4 v = *reinterpret_cast<const float4*>(p + i);
+        a = make_float2(v.x, v.y); b = make_float2(v.z, v.w);
     }
 };
 
@@ -953,7 +964,7 @@ struct MixStore {
     }
 };
 
-// M: the moving-sources instantiation (render_kernel_moving).  Every block may name its own set; a block whose set
+// M: the moving-sources instantiation (render_kernel<..., true>).  Every block may name its own set; a block whose set
 // differs from the previous block's renders both sets' outputs from the one history and crossfades them (MixStore).
 template <int N, int G, int V, bool M = false>
 __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned char* smem, int stream0, int conv_index) {
@@ -1265,18 +1276,20 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
                 dstz[i >> 1] = make_float4(z0.x, z0.y, z1.x, z1.y);
             }
         }
-        // partition 0's spectra come from the resident shared-memory copy (plain LDS: the address space is known at
-        // compile time) or from global memory; one generic pointer for both would compile to generic loads
-        auto mac_partition0 = [&](const float4* fq) {
+        // partition 0 of filter table fq on top of the history in acc, with this block's spectrum read from z (zbuf, or
+        // moving: its delay-line slot), and the swapped product into wbuf.  The static path's table is the resident
+        // shared-memory copy (plain LDS: the address space is known at compile time) or global memory; one generic
+        // pointer for both would compile to generic loads
+        auto mac_partition0 = [&](const auto& z, const float4* fq) {
 #pragma unroll
             for (int m = 0; m < kPairs; ++m) {
                 const int k = 2 * (tid + m * T);
                 const int m0 = k ? N - k : N / 2, m1 = N - k - 1;
                 Operands o;
                 float2 u0, u1;
-                zbuf.ld2(k, u0, u1);
+                z.ld2(k, u0, u1);
                 o.uu = make_float4(u0.x, u0.y, u1.x, u1.y);
-                o.v0 = zbuf.ld(m0); o.v1 = zbuf.ld(m1);
+                o.v0 = z.ld(m0); o.v1 = z.ld(m1);
                 o.f0 = fq[fe(k)]; o.f1 = fq[fo(k + 1)]; o.g0 = fq[fe(m0)]; o.g1 = fq[fo(m1)];
                 mac_ops(acc[m], o, k);
                 // swap(re, im): the inverse transform is run as swap(FFT(swap(W)))
@@ -1320,7 +1333,7 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
                 }
             };
             stream_sync();
-            const float2* zs = fdl_s + (size_t)slot * N;
+            const GlobalCx zs{fdl_s + (size_t)slot * N};
 #pragma unroll 1
             for (int pass = trans ? 0 : 1; pass < 2; ++pass) {
                 const float4* fq = filt_g;
@@ -1333,15 +1346,7 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
                         for (int e = 0; e < 4; ++e) acc[m][e] = make_float2(0.f, 0.f);
                     if (np > 1) mac_history(fq, np);
                 }
-#pragma unroll
-                for (int m = 0; m < kPairs; ++m) {
-                    const int k = 2 * (tid + m * T);
-                    const int m0 = k ? N - k : N / 2, m1 = N - k - 1;
-                    mac_ops(acc[m], load_ops(zs, fq, k, m0, m1), k);
-                    wbuf.st2(k, make_float2(acc[m][0].y, acc[m][0].x), make_float2(acc[m][1].y, acc[m][1].x));
-                    wbuf.st(m0, make_float2(acc[m][2].y, acc[m][2].x));
-                    wbuf.st(m1, make_float2(acc[m][3].y, acc[m][3].x));
-                }
+                mac_partition0(zs, fq);
                 stream_sync();
                 fft_run<N, T>(tid, tw, zbuf.p, wbuf.p, wbuf, MixStore{out_l + (size_t)t * B - B, out_r + (size_t)t * B - B, gain, B, trans && pass == 1},
                               stream_sync, [&]() {});
@@ -1349,8 +1354,8 @@ __device__ __forceinline__ void conv_warps_main(const RenderParams& p, unsigned 
             }
             continue;
         }
-        if (SM::kFiltSmemBytes > 0 && p.filt_in_smem) mac_partition0(reinterpret_cast<const float4*>(smem + SM::kFiltOff));
-        else mac_partition0(filt_g);
+        if (SM::kFiltSmemBytes > 0 && p.filt_in_smem) mac_partition0(zbuf, reinterpret_cast<const float4*>(smem + SM::kFiltOff));
+        else mac_partition0(zbuf, filt_g);
         stream_sync();
         // ---- inverse FFT; keep the last B samples (overlap-save), ear sums are already inside W, apply gain
         fft_run<N, T>(tid, tw, zbuf.p, wbuf.p, wbuf, OutputStore{out_l + (size_t)t * B - B, out_r + (size_t)t * B - B, gain, B},
@@ -1377,7 +1382,9 @@ __device__ __forceinline__ int find_conv_index(int warp, std::integer_sequence<i
     return r;
 }
 
-template <int N, int G, int V = 0>
+// Moving: per-block HRIR sets with one-block crossfades (conv_warps_main<..., true>; DESIGN §10), instantiated
+// separately and launched only for calls that need it, so that the static instantiations carry none of its code
+template <int N, int G, int V = 0, bool Moving = false>
 __global__ void __maxnreg__((RenderSmem<N, G, V>::kMaxRegs)) render_kernel(const RenderParams p) {
     using SM = RenderSmem<N, G, V>;
     extern __shared__ __align__(16) unsigned char smem[];
@@ -1392,22 +1399,7 @@ __global__ void __maxnreg__((RenderSmem<N, G, V>::kMaxRegs)) render_kernel(const
     if (warp < SM::kEqWarps) { eq_warp_main<N, G, V>(p, smem, stream0, warp); return; }
     if (warp == SM::kStagerWarpId) { stager_warp_main<N, G, V>(p, smem, stream0); return; }
     const int conv_index = find_conv_index<N, G, V>(warp, std::make_integer_sequence<int, SM::kConvWarps>{});
-    if (conv_index >= 0) conv_warps_main<N, G, V>(p, smem, stream0, conv_index);  // other warp slots are placement padding
-}
-
-// Moving sources: the same kernel with per-block HRIR sets and one-block crossfades (conv_warps_main<..., true>).  A
-// kernel of its own, launched only for calls that need it, so that render_kernel's instantiations stay as they are.
-template <int N, int G, int V = 0>
-__global__ void __maxnreg__((RenderSmem<N, G, V>::kMaxRegs)) render_kernel_moving(const RenderParams p) {
-    using SM = RenderSmem<N, G, V>;
-    extern __shared__ __align__(16) unsigned char smem[];
-    const int stream0 = p.first_stream + blockIdx.x * G;
-    launch_dependents();
-    const int warp = threadIdx.x >> 5;
-    if (warp < SM::kEqWarps) { eq_warp_main<N, G, V>(p, smem, stream0, warp); return; }
-    if (warp == SM::kStagerWarpId) { stager_warp_main<N, G, V>(p, smem, stream0); return; }
-    const int conv_index = find_conv_index<N, G, V>(warp, std::make_integer_sequence<int, SM::kConvWarps>{});
-    if (conv_index >= 0) conv_warps_main<N, G, V, true>(p, smem, stream0, conv_index);
+    if (conv_index >= 0) conv_warps_main<N, G, V, Moving>(p, smem, stream0, conv_index);  // other warp slots are placement padding
 }
 
 }  // namespace ohs

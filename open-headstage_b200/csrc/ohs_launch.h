@@ -18,7 +18,7 @@ struct RenderLaunch {
     size_t min_smem_bytes; // EQ-only variant: ask for at least this much dynamic shared memory (keeps other kernels' CTAs off the SM)
     bool dependent;        // programmatic dependent launch: this grid may start while the previous launch on the stream
                            // drains; the kernel waits (griddepcontrol.wait) before it touches stream state
-    bool moving;           // render_kernel_moving: per-block HRIR sets with crossfaded transitions (variants 0 and 1)
+    bool moving;           // render_kernel<N, G, V, true>: per-block HRIR sets with crossfaded transitions (variants 0 and 1)
 };
 
 // cudaSuccess, or the CUDA error of the attribute call / launch; cudaErrorInvalidConfiguration if G does not fit

@@ -13,13 +13,12 @@ namespace {
 
 constexpr int N = OHS_RENDER_N;
 
-// Moving: render_kernel_moving (per-block HRIR sets, crossfaded transitions) instead of render_kernel
 template <int G, int V, bool Moving = false> cudaError_t launch_gv(const RenderLaunch& L, const RenderParams& p) {
     using SM = RenderSmem<N, G, V>;
     if constexpr (!SM::kFits) {
         return cudaErrorInvalidConfiguration;
     } else {
-        constexpr auto kernel = [] { if constexpr (Moving) return render_kernel_moving<N, G, V>; else return render_kernel<N, G, V>; }();
+        constexpr auto kernel = render_kernel<N, G, V, Moving>;
         // function attributes are per device; distinct handles may race here, so the flags are atomic (setting an
         // attribute twice is harmless)
         static std::atomic<unsigned char> attr_set[64];
@@ -49,29 +48,20 @@ template <int G, int V, bool Moving = false> cudaError_t launch_gv(const RenderL
 }
 
 // the latency variant (RenderSmem, V = 1) where it exists and fits, else the throughput variant; the EQ-only variant
-// (V = 2) on request.  The moving-sources kernel exists in the throughput and latency variants.
+// (V = 2) on request, for static launches only
 template <int G> cudaError_t launch_g(const RenderLaunch& L, const RenderParams& p) {
-    if (L.moving) {
-        if (L.variant == 2) return cudaErrorInvalidConfiguration;
-        if constexpr (N == 512) {
-            if constexpr (RenderSmem<N, G, 1>::kFits) {
-                if (L.variant == 1) return launch_gv<G, 1, true>(L, p);
-            }
-        }
-        return launch_gv<G, 0, true>(L, p);
-    }
     if constexpr (N == 512) {
         if (L.variant == 2) {
-            if constexpr (RenderSmem<N, G, 2>::kFits) return launch_gv<G, 2>(L, p);
-            else return cudaErrorInvalidConfiguration;
+            if constexpr (RenderSmem<N, G, 2>::kFits) { if (!L.moving) return launch_gv<G, 2>(L, p); }
+            return cudaErrorInvalidConfiguration;
         }
         if constexpr (RenderSmem<N, G, 1>::kFits) {
-            if (L.variant == 1) return launch_gv<G, 1>(L, p);
+            if (L.variant == 1) return L.moving ? launch_gv<G, 1, true>(L, p) : launch_gv<G, 1>(L, p);
         }
     } else {
         if (L.variant == 2) return cudaErrorInvalidConfiguration;
     }
-    return launch_gv<G, 0>(L, p);
+    return L.moving ? launch_gv<G, 0, true>(L, p) : launch_gv<G, 0>(L, p);
 }
 
 template <int G> constexpr int threads_g() {

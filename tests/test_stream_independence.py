@@ -11,7 +11,8 @@ Routes, forced the way the other GPU tests force them:
   R3  EQ-only mode (convolution off) with a ragged last block
   R4  the time-batched route (P >= 8, >= 8 blocks per call), its EQ pre-pass on CTAs of six streams that own their SM
       (>= 12 streams), on thin CTAs of three, and without the overlapped pipeline
-  R5  render_kernel_moving, which a multi-set engine with a delay line runs when some stream is bound to a one-partition set
+  R5  render_kernel<N, G, V, true>, the moving-sources kernel, which a multi-set engine with a delay line runs when some
+      stream is bound to a one-partition set
 Bindings derive from s % U and the inputs tile with period U, U prime to G, so that twin streams (same input, same
 bindings) sit in different CTAs and different slots; every CTA holds streams with different bindings.
 
