@@ -203,7 +203,8 @@ int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames
  *            time-batched route, pending moves, state); the engine state afterwards is the state after the f32 call on
  *            the decoded input
  *   encode   b = 16 / 24:  v = y * 2^(b-1) in f32 (exact for finite y), rounded to nearest with ties to even, clamped to
- *            [-2^(b-1), 2^(b-1) - 1]; NaN -> 0, +-inf -> the clamp bounds; no dither
+ *            [-2^(b-1), 2^(b-1) - 1]; NaN -> 0, +-inf -> the clamp bounds; dithered as ohs_set_dither says (below), off by
+ *            default
  * so out == encode(render(decode(in))) bit for bit.  OHS_FMT_F32 on a side means no conversion on that side; F32 -> F32
  * is ohs_process / ohs_process_device.  Bypass: out = encode(decode(in)) (equal formats: the bytes unchanged), state
  * untouched.  Checked before anything is enqueued (OHS_ERR_INVALID, engine untouched): an unknown format, n_frames not
@@ -215,7 +216,7 @@ int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames
  * route within round-off.  The device flavour decodes through f32 scratch rows of the engine (up to 256 MiB, allocated
  * on first use or by ohs_prepare; longer calls go through them in time chunks of whole blocks), except that a call with
  * f32 output decodes into the output rows and renders them in place.
- * Not provided: a PCM form of ohs_process_fifo or of ohs_process_device_scheduled, dither, a clip counter, S32 and F64. */
+ * Not provided: a PCM form of ohs_process_fifo or of ohs_process_device_scheduled, a clip counter, S32 and F64. */
 typedef enum ohs_sample_format {
     OHS_FMT_F32 = 0,   /* float, as everywhere else in this API */
     OHS_FMT_S16 = 1,   /* int16_t, little-endian */
@@ -226,6 +227,38 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
 /* device memory; the same contract as ohs_process_device */
 int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void* d_out, int out_format, size_t n_frames,
                            size_t row_stride);
+
+/* ---- dither of integer PCM output (an extension) -----------------------------------------------------------------
+ * TPDF dither, optionally with error-feedback noise shaping, for every encode to S16 or S24 by ohs_process_pcm and
+ * ohs_process_device_pcm, bypassed F32 -> S16 or S24 -> S16 calls included.  F32 output is never dithered.  Exact to the
+ * bit (numpy reference: signals.pcm_encode_dithered).  Row r = 2*stream + channel; b = 16 / 24; lo, hi = the clamp bounds.
+ *   position  a 64-bit counter p: ohs_set_dither sets it to 0; every successful call with an integer OUTPUT format moves it
+ *             on by n_frames (bypassed ones too); frame f of a call has position p0 + f.  So the noise does not depend on
+ *             how a render is cut into calls or into the chunks of a call.
+ *   noise     mix64(z) = SplitMix64's finaliser: z ^= z >> 30; z *= 0xBF58476D1CE4E5B9; z ^= z >> 27;
+ *             z *= 0x94D049BB133111EB; z ^= z >> 31 (all uint64, wrapping), phi = 0x9E3779B97F4A7C15,
+ *             K_r = mix64(seed + phi * (r + 1)), x = mix64(K_r + phi * (p + 1)),
+ *             u1 = x & (2^23 - 1), u2 = (x >> 32) & (2^23 - 1), d = (u1 + u2 - (2^23 - 1)) * 2^-23:
+ *             exact in f32, in (-1, 1) LSB, triangular (TPDF), variance 1/6 LSB^2
+ *   flat      (n_taps = 0)  v = y * 2^(b-1);  q = clamp(rint_even(v + d), lo, hi), v + d rounded in f32;  NaN -> 0
+ *   shaped    (n_taps = M)  taps h_1..h_M, per-row error history e_1..e_M (most recent first, zero after ohs_set_dither):
+ *             fb = h_M*e_M, then + h_(M-1)*e_(M-1), ..., + h_1*e_1 (oldest term first), w = v - fb,
+ *             q = clamp(rint_even(w + d), lo, hi), e = clamp(q - w, -1.5, 1.5) becomes e_1 and the others move one back;
+ *             every product and sum rounded on its own in f32.  NaN v: q = 0, e = 0; +-inf clamps as without dither.
+ *             So q = v + (1 - H(z)) e with H(z) = sum h_k z^-k: the white dither-plus-rounding error (1/4 LSB^2) shaped
+ *             by |1 - H|^2.  Without clipping |q - w| < 1.5 always; the clamp of e acts only on clipped samples and keeps
+ *             the loop from winding up there.
+ * Seed, mode and taps are configuration, like bindings; the position and the error history are state and travel in the
+ * state blob.  An equal-format bypass copies bytes and encodes nothing: the position moves on, the history stays.
+ * Several GPUs: each rank numbers its rows from 0, so give every rank a seed of its own. */
+#define OHS_DITHER_OFF 0       /* round and clamp only (the default) */
+#define OHS_DITHER_TPDF 1      /* TPDF dither, noise-shaped when n_taps > 0 */
+#define OHS_MAX_SHAPE_TAPS 9
+/* Sets mode, seed and taps (shape[0..n_taps) = h_1..h_M, copied), resets the position to 0 and zeroes the history, on the
+ * engine's stream (ordered after earlier calls).  Allocates the history (2 * n_streams * OHS_MAX_SHAPE_TAPS floats) for
+ * OHS_DITHER_TPDF; process calls never allocate for dither.  OHS_ERR_INVALID with the engine untouched: an unknown mode,
+ * n_taps outside 0..OHS_MAX_SHAPE_TAPS, taps with OHS_DITHER_OFF, a null shape with n_taps > 0, a non-finite tap. */
+int ohs_set_dither(ohs_engine* h, int mode, uint64_t seed, const float* shape, int n_taps);
 
 int ohs_sync(ohs_engine* h);
 /* The engine's cudaStream_t (as void*) so callers can order their own work / NCCL calls against it. */
@@ -274,9 +307,11 @@ int ohs_host_free(void* p);
 int ohs_debug_trace(ohs_engine* h, unsigned long long* d_stamps);
 
 /* ---- state export / import (chunked offline renders resume bit-exactly; SURVEY.md §5.4) ----------------------
- * The blob holds a self-describing header (geometry, ring head, byte count), the delay line, the overlap-save blocks,
- * the biquad states and whatever ohs_process_fifo has queued; import rejects a blob whose geometry, size or ring
- * head does not match this engine.  ohs_state_bytes is the size an export would need NOW (it grows with the FIFO). */
+ * The blob holds a self-describing header (geometry, ring head, flags, byte count), the delay line, the overlap-save
+ * blocks, the biquad states and whatever ohs_process_fifo has queued, and while dither is on (flags bit 0) the dither
+ * position (uint64) and error history (float[2 * n_streams][OHS_MAX_SHAPE_TAPS]) behind them; with dither off the blob
+ * is what it was before dither existed.  Import rejects a blob whose geometry, size, ring head or dither flag does not
+ * match this engine, and then leaves the engine untouched.  ohs_state_bytes is the size an export would need NOW (it grows with the FIFO). */
 int ohs_state_bytes(ohs_engine* h, size_t* bytes);
 int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes);
 int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes);

@@ -8,6 +8,6 @@ reference's `ConvolutionEngine` / `StereoParametricEQ`, and the seeded synthetic
 from . import autoeq, parallel, signals, sofa  # noqa: F401
 from ._build import build_host_inputs_tool, build_host_tests, build_library  # noqa: F401
 from .engine import (  # noqa: F401
-    ALLPASS, BANDPASS, FMT_F32, FMT_S16, FMT_S24, HIGHPASS, HIGHSHELF, LOWPASS, LOWSHELF, LSL, LSR, NOTCH, OHS_ALL, PEAK, RSL, RSR, SYMBOLS,
+    ALLPASS, BANDPASS, DITHER_OFF, DITHER_TPDF, FMT_F32, FMT_S16, FMT_S24, HIGHPASS, HIGHSHELF, LOWPASS, LOWSHELF, LSL, LSR, MAX_SHAPE_TAPS, NOTCH, OHS_ALL, PEAK, RSL, RSR, SYMBOLS,
     BandConfig, Comm, ConvolutionEngine, Engine, OhsError, PinnedBuffer, StereoParametricEQ, comm_unique_id, eq_design, load_library,
 )

@@ -103,6 +103,12 @@ struct ohs_engine {
     // f32 rows of ohs_process_device_pcm's time chunks (decoded input, rendered in place)
     float* d_pcm_scratch = nullptr;
     size_t pcm_scratch_cap = 0;
+    // dither of integer PCM output (ohs_set_dither): mode, seed and taps are configuration; the position (frames encoded
+    // since ohs_set_dither) and the per-row error history are state, carried by the state blob
+    int dither_mode = OHS_DITHER_OFF, dither_taps = 0;
+    unsigned long long dither_seed = 0, dither_pos = 0;
+    ohs::DitherTaps dither_h{};
+    float* d_dither_hist = nullptr;   // [2 * n_streams][OHS_MAX_SHAPE_TAPS], allocated by ohs_set_dither
 
     // time-batched long-response path: spectra in time order and frequency-domain products of one sub-launch
     float2* d_zlin = nullptr;
@@ -417,19 +423,48 @@ int check_pcm_args(ohs_engine* h, const void* in, int in_format, const void* out
     return OHS_OK;
 }
 
-// PCM rows <-> f32 rows on the engine's stream; pcm_pitch in bytes, f32_pitch in floats
-int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t pcm_pitch, float* f32, size_t f32_pitch, size_t n_frames) {
+static_assert(kShapeTaps == OHS_MAX_SHAPE_TAPS, "history rows of the shaped encode");
+
+// pcm_encode_shaped_kernel<Fmt, M> for the runtime tap count m (1..OHS_MAX_SHAPE_TAPS)
+template <int Fmt, int M = 1>
+void launch_encode_shaped(int m, cudaStream_t st, const float* f32, size_t f32_pitch, unsigned char* pcm, size_t pcm_pitch,
+                          size_t n_frames, int rows, unsigned long long seed, unsigned long long pos, const DitherTaps& taps,
+                          float* hist) {
+    if constexpr (M <= kShapeTaps) {
+        if (m != M)
+            return launch_encode_shaped<Fmt, M + 1>(m, st, f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist);
+        pcm_encode_shaped_kernel<Fmt, M><<<(rows + kShapeRows - 1) / kShapeRows, kShapeThreads, 0, st>>>(
+            f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist);
+    }
+}
+
+// PCM rows <-> f32 rows on the engine's stream; pcm_pitch in bytes, f32_pitch in floats.  An encode is dithered as
+// ohs_set_dither says, its first frame at dither position dither_pos + pos_offset (the frame's offset in the call).
+int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t pcm_pitch, float* f32, size_t f32_pitch, size_t n_frames,
+               size_t pos_offset = 0) {
     const size_t rows = (size_t)h->cfg.n_streams * 2;
     const size_t groups = (n_frames + pcm_align_frames(fmt) - 1) / pcm_align_frames(fmt), total = rows * groups;
     const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
+    const unsigned long long seed = h->dither_seed, pos = h->dither_pos + pos_offset;
+    const bool tpdf = h->dither_mode == OHS_DITHER_TPDF, shaped = tpdf && h->dither_taps > 0;
     if (decode && fmt == OHS_FMT_S16)
         pcm_decode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
     else if (decode)
         pcm_decode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
+    else if (shaped && fmt == OHS_FMT_S16)
+        launch_encode_shaped<kPcmS16>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
+                                      h->dither_h, h->d_dither_hist);
+    else if (shaped)
+        launch_encode_shaped<kPcmS24>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
+                                      h->dither_h, h->d_dither_hist);
+    else if (tpdf && fmt == OHS_FMT_S16)
+        pcm_encode_kernel<kPcmS16, true><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed, pos);
+    else if (tpdf)
+        pcm_encode_kernel<kPcmS24, true><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed, pos);
     else if (fmt == OHS_FMT_S16)
-        pcm_encode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total);
+        pcm_encode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
     else
-        pcm_encode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total);
+        pcm_encode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
     OHS_CUDA(cudaGetLastError());
     h->launches++;
     return OHS_OK;
@@ -902,7 +937,7 @@ int ohs_destroy(ohs_engine* h) {
     void* ptrs[] = {h->d_stream_hrir, h->d_stream_eq, h->d_stream_gain, h->d_filt, h->d_set_parts, h->d_set_list, h->d_set_flags,
                     h->d_fdl, h->d_prev, h->d_eqc, h->d_eqs, h->d_tw, h->d_ir, h->d_stage[0], h->d_stage[1], h->d_stage[2],
                     h->d_zlin, h->d_wlin, h->d_xf, h->d_from_set, h->d_sched, h->d_pcm_stage[0], h->d_pcm_stage[1],
-                    h->d_pcm_stage[2], h->d_pcm_scratch};
+                    h->d_pcm_stage[2], h->d_pcm_scratch, h->d_dither_hist};
     for (void* p : ptrs) if (p) cudaFree(p);
     for (int i = 0; i < kPipe; ++i) {
         if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
@@ -1068,6 +1103,28 @@ int ohs_eq_frequency_response(ohs_engine* h, int eq_set, float sample_rate, cons
 int ohs_set_eq_enable(ohs_engine* h, int enable) { OHS_CHECK_HANDLE(h); h->eq_enable = enable ? 1 : 0; return OHS_OK; }
 int ohs_set_conv_enable(ohs_engine* h, int enable) { OHS_CHECK_HANDLE(h); h->conv_enable = enable ? 1 : 0; return OHS_OK; }
 int ohs_set_bypass(ohs_engine* h, int bypass) { OHS_CHECK_HANDLE(h); h->bypass = bypass ? 1 : 0; return OHS_OK; }
+
+int ohs_set_dither(ohs_engine* h, int mode, uint64_t seed, const float* shape, int n_taps) {
+    OHS_CHECK_HANDLE(h);
+    if (mode != OHS_DITHER_OFF && mode != OHS_DITHER_TPDF) return fail(OHS_ERR_INVALID, "unknown dither mode %d", mode);
+    if (n_taps < 0 || n_taps > OHS_MAX_SHAPE_TAPS) return fail(OHS_ERR_INVALID, "n_taps %d outside 0..%d", n_taps, OHS_MAX_SHAPE_TAPS);
+    if (mode == OHS_DITHER_OFF && n_taps) return fail(OHS_ERR_INVALID, "noise-shaping taps need OHS_DITHER_TPDF");
+    if (n_taps && !shape) return fail(OHS_ERR_INVALID, "null shape with %d taps", n_taps);
+    for (int k = 0; k < n_taps; ++k)
+        if (!std::isfinite(shape[k])) return fail(OHS_ERR_INVALID, "shape[%d] is not finite", k);
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    const size_t hist_bytes = sizeof(float) * (size_t)h->cfg.n_streams * 2 * OHS_MAX_SHAPE_TAPS;
+    if (mode != OHS_DITHER_OFF && !h->d_dither_hist) OHS_CUDA(cudaMalloc(&h->d_dither_hist, hist_bytes));
+    // on the engine's stream: ordered after every encode enqueued before
+    if (h->d_dither_hist) OHS_CUDA(cudaMemsetAsync(h->d_dither_hist, 0, hist_bytes, h->stream));
+    h->dither_mode = mode;
+    h->dither_seed = seed;
+    h->dither_taps = n_taps;
+    h->dither_h = DitherTaps{};
+    for (int k = 0; k < n_taps; ++k) h->dither_h.h[k] = shape[k];
+    h->dither_pos = 0;
+    return OHS_OK;
+}
 
 int ohs_set_gain(ohs_engine* h, int stream, float gain) {
     OHS_CHECK_HANDLE(h);
@@ -1247,6 +1304,7 @@ int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_forma
     if (h->bypass && in_format == out_format) {
         if (in != out)
             OHS_CUDA(cudaMemcpy2DAsync(out, row_stride * bo, in, row_stride * bi, n_frames * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
+        h->dither_pos += n_frames;   // an integer output format: the position moves on, although nothing was encoded
         return OHS_OK;
     }
     if (out_format == OHS_FMT_F32) {   // decode straight into the output rows, render them in place
@@ -1255,21 +1313,24 @@ int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_forma
         if (rc || h->bypass) return rc;
         return process_device_impl(h, y, y, n_frames, row_stride, nullptr, 0);
     }
-    if (in_format == OHS_FMT_F32 && h->bypass)
-        return launch_pcm(h, false, out_format, out, row_stride * bo, reinterpret_cast<float*>(src), row_stride, n_frames);
-    const size_t chunk = chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float));
-    int rc = ensure_pcm_scratch(h, chunk);
-    if (rc) return rc;
-    float* x = h->d_pcm_scratch;
-    for (size_t f0 = 0; f0 < n_frames; f0 += chunk) {
-        const size_t n = std::min(chunk, n_frames - f0), pitch = round_up(n, 4);
-        if (in_format == OHS_FMT_F32)
-            OHS_CUDA(cudaMemcpy2DAsync(x, pitch * sizeof(float), src + f0 * bi, row_stride * bi, n * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
-        else if ((rc = launch_pcm(h, true, in_format, src + f0 * bi, row_stride * bi, x, pitch, n))) return rc;
-        if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
-        if ((rc = launch_pcm(h, false, out_format, out + f0 * bo, row_stride * bo, x, pitch, n))) return rc;
+    int rc = OHS_OK;
+    if (in_format == OHS_FMT_F32 && h->bypass) {
+        rc = launch_pcm(h, false, out_format, out, row_stride * bo, reinterpret_cast<float*>(src), row_stride, n_frames);
+    } else {
+        const size_t chunk = chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float));
+        if ((rc = ensure_pcm_scratch(h, chunk))) return rc;
+        float* x = h->d_pcm_scratch;
+        for (size_t f0 = 0; f0 < n_frames; f0 += chunk) {
+            const size_t n = std::min(chunk, n_frames - f0), pitch = round_up(n, 4);
+            if (in_format == OHS_FMT_F32)
+                OHS_CUDA(cudaMemcpy2DAsync(x, pitch * sizeof(float), src + f0 * bi, row_stride * bi, n * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
+            else if ((rc = launch_pcm(h, true, in_format, src + f0 * bi, row_stride * bi, x, pitch, n))) return rc;
+            if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
+            if ((rc = launch_pcm(h, false, out_format, out + f0 * bo, row_stride * bo, x, pitch, n, f0))) return rc;
+        }
     }
-    return OHS_OK;
+    if (rc == OHS_OK) h->dither_pos += n_frames;
+    return rc;
 }
 
 }  // namespace
@@ -1528,6 +1589,7 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     unsigned char* dst = static_cast<unsigned char*>(out);
     if (h->bypass && in_format == out_format) {
         if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(dst + r * row_stride * bo, src + r * row_stride * bi, n_frames * bi);
+        if (out_format != OHS_FMT_F32) h->dither_pos += n_frames;
         return OHS_OK;
     }
     const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32;
@@ -1560,7 +1622,7 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
         OHS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
         if (pcm_in && (rc = launch_pcm(h, true, in_format, q, pcm_pitch * bi, x, pitch, n))) return rc;
         if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
-        if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n))) return rc;
+        if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n, done))) return rc;
         OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
         OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
         if (pcm_out)
@@ -1574,6 +1636,7 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     }
     OHS_CUDA(cudaStreamSynchronize(h->d2h));
     OHS_CUDA(cudaStreamSynchronize(h->stream));
+    if (pcm_out) h->dither_pos += n_frames;
     return OHS_OK;
 }
 
@@ -1634,30 +1697,34 @@ int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames
 
 // ---- state export / import ----------------------------------------------------------------------------------
 // blob = StateHeader | delay line | overlap-save blocks | biquad states | FIFO residue (input rows, output rows)
+//        [ | dither position (uint64) | error history float[2S][OHS_MAX_SHAPE_TAPS] ]  when flags has kStateDither
 namespace {
 struct StateHeader {
     uint32_t magic;      // 'OHSS'
-    int32_t abi, n_streams, n_bands, pmax, block, head, reserved;
+    int32_t abi, n_streams, n_bands, pmax, block, head, flags;
     uint64_t fifo_in_len, fifo_out_len, total_bytes;
 };
 constexpr uint32_t kStateMagic = 0x5353484Fu;
-size_t state_need(const ohs_engine* h, size_t fifo_in, size_t fifo_out) {
+constexpr int32_t kStateDither = 1;   // the dither section follows the FIFO residue
+size_t dither_state_bytes(const ohs_engine* h) { return sizeof(uint64_t) + sizeof(float) * (size_t)h->cfg.n_streams * 2 * OHS_MAX_SHAPE_TAPS; }
+size_t state_need(const ohs_engine* h, size_t fifo_in, size_t fifo_out, bool dither) {
     const size_t S = h->cfg.n_streams;
     return sizeof(StateHeader) + sizeof(float2) * S * h->pmax * h->N + sizeof(float2) * S * h->B + sizeof(float4) * S * kMaxBands +
-           sizeof(float) * S * 2 * (fifo_in + fifo_out);
+           sizeof(float) * S * 2 * (fifo_in + fifo_out) + (dither ? dither_state_bytes(h) : 0);
 }
 }  // namespace
 
 int ohs_state_bytes(ohs_engine* h, size_t* bytes) {
     OHS_CHECK_HANDLE(h);
     if (!bytes) return fail(OHS_ERR_INVALID, "null output");
-    *bytes = state_need(h, h->fifo_in_len, h->fifo_out_len);
+    *bytes = state_need(h, h->fifo_in_len, h->fifo_out_len, h->dither_mode != OHS_DITHER_OFF);
     return OHS_OK;
 }
 
 int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
     OHS_CHECK_HANDLE(h);
-    const size_t need = state_need(h, h->fifo_in_len, h->fifo_out_len);
+    const bool dither = h->dither_mode != OHS_DITHER_OFF;
+    const size_t need = state_need(h, h->fifo_in_len, h->fifo_out_len, dither);
     if (!host_buf || bytes < need) return fail(OHS_ERR_INVALID, "state buffer too small (%zu < %zu)", bytes, need);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     int rc = commit_filters(h);
@@ -1667,7 +1734,7 @@ int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     unsigned char* p = (unsigned char*)host_buf;
     const size_t S = h->cfg.n_streams;
-    StateHeader hdr{kStateMagic, OHS_ABI_VERSION, h->cfg.n_streams, kMaxBands, h->pmax, h->B, h->head, 0,
+    StateHeader hdr{kStateMagic, OHS_ABI_VERSION, h->cfg.n_streams, kMaxBands, h->pmax, h->B, h->head, dither ? kStateDither : 0,
                     (uint64_t)h->fifo_in_len, (uint64_t)h->fifo_out_len, (uint64_t)need};
     memcpy(p, &hdr, sizeof(hdr)); p += sizeof(hdr);
     const size_t n0 = sizeof(float2) * S * h->pmax * h->N, n1 = sizeof(float2) * S * h->B, n2 = sizeof(float4) * S * kMaxBands;
@@ -1677,6 +1744,11 @@ int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
     // what ohs_process_fifo has queued (src/dsp/convolution.rs:73-76 input_buffer / output_buffer), row by row
     for (size_t r = 0; r < S * 2; ++r) { memcpy(p, h->fifo_in.data() + r * h->fifo_cap, h->fifo_in_len * sizeof(float)); p += h->fifo_in_len * sizeof(float); }
     for (size_t r = 0; r < S * 2; ++r) { memcpy(p, h->fifo_out.data() + r * h->fifo_cap, h->fifo_out_len * sizeof(float)); p += h->fifo_out_len * sizeof(float); }
+    if (dither) {
+        const uint64_t pos = h->dither_pos;
+        memcpy(p, &pos, sizeof(pos)); p += sizeof(pos);
+        OHS_CUDA(cudaMemcpy(p, h->d_dither_hist, dither_state_bytes(h) - sizeof(pos), cudaMemcpyDeviceToHost));
+    }
     return OHS_OK;
 }
 
@@ -1693,7 +1765,12 @@ int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes) {
     if (hdr.head < 0 || hdr.head >= h->pmax) return fail(OHS_ERR_INVALID, "state blob ring head %d outside 0..%d", hdr.head, h->pmax - 1);
     const size_t limit = (size_t)1 << 32;
     if (hdr.fifo_in_len > limit || hdr.fifo_out_len > limit) return fail(OHS_ERR_INVALID, "state blob FIFO lengths are implausible");
-    const size_t need = state_need(h, (size_t)hdr.fifo_in_len, (size_t)hdr.fifo_out_len);
+    if (hdr.flags & ~kStateDither) return fail(OHS_ERR_INVALID, "state blob has unknown flags 0x%x", (unsigned)hdr.flags);
+    const bool dither = (hdr.flags & kStateDither) != 0;
+    if (dither != (h->dither_mode != OHS_DITHER_OFF))
+        return fail(OHS_ERR_INVALID, dither ? "state blob carries dither state but this engine's dither is off"
+                                            : "state blob carries no dither state but this engine dithers (ohs_set_dither first)");
+    const size_t need = state_need(h, (size_t)hdr.fifo_in_len, (size_t)hdr.fifo_out_len, dither);
     if (hdr.total_bytes != need || bytes != need) return fail(OHS_ERR_INVALID, "state blob is %zu bytes, header says %llu, geometry needs %zu", bytes, (unsigned long long)hdr.total_bytes, need);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     int rc = commit_filters(h);  // pending set_ir would otherwise clear the imported history later
@@ -1712,6 +1789,12 @@ int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes) {
     for (size_t r = 0; r < S * 2; ++r) { memcpy(h->fifo_in.data() + r * cap, p, fi * sizeof(float)); p += fi * sizeof(float); }
     for (size_t r = 0; r < S * 2; ++r) { memcpy(h->fifo_out.data() + r * cap, p, fo * sizeof(float)); p += fo * sizeof(float); }
     h->fifo_in_len = fi; h->fifo_out_len = fo;
+    if (dither) {
+        uint64_t pos;
+        memcpy(&pos, p, sizeof(pos)); p += sizeof(pos);
+        OHS_CUDA(cudaMemcpy(h->d_dither_hist, p, dither_state_bytes(h) - sizeof(pos), cudaMemcpyHostToDevice));
+        h->dither_pos = pos;
+    }
     return OHS_OK;
 }
 

@@ -448,17 +448,68 @@ __global__ void __launch_bounds__(256) pcm_decode_kernel(const unsigned char* __
     }
 }
 
-// in: f32 rows (pitch in floats), out: PCM rows (pitch in bytes)
-template <int Fmt>
+// ---- dither (ohs_set_dither, include/ohs.h) ------------------------------------------------------------------------
+// The noise of row r at dither position p: x = mix64(K_r + phi * (p + 1)) with K_r = mix64(seed + phi * (r + 1)) (SplitMix64's
+// increment and finaliser), d = (u1 + u2 - (2^23 - 1)) * 2^-23 from the low 23 bits of each half of x: TPDF in (-1, 1) LSB,
+// exact in f32.  A stateless function of (seed, r, p), so the noise does not depend on how a render is cut into calls.
+constexpr unsigned long long kDitherPhi = 0x9E3779B97F4A7C15ull;
+constexpr int kShapeTaps = 9;   // OHS_MAX_SHAPE_TAPS: taps of the error-feedback filter, and history floats per row
+
+__device__ __forceinline__ unsigned long long dither_mix64(unsigned long long z) {
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+__device__ __forceinline__ unsigned long long dither_row_key(unsigned long long seed, size_t row) {
+    return dither_mix64(seed + kDitherPhi * (row + 1));
+}
+// the noise of the position whose phi * (p + 1) has been added to the row key
+__device__ __forceinline__ float dither_noise(unsigned long long keyed) {
+    const unsigned long long x = dither_mix64(keyed);
+    const int u1 = (int)(x & 0x7fffffu), u2 = (int)((x >> 32) & 0x7fffffu);
+    return (float)(u1 + u2 - 0x7fffff) * 0x1p-23f;
+}
+
+// flat TPDF: clamp(rint(v + d)) with v + d rounded on its own (no contraction into an FMA with the exact scaling); NaN -> 0
+template <int Fmt> __device__ __forceinline__ int pcm_quantise_dithered(float y, float d) {
+    using P = PcmTraits<Fmt>;
+    const float v = __fmul_rn(y, P::kEncode);
+    if (v != v) return 0;
+    return __float2int_rn(fminf(fmaxf(__fadd_rn(v, d), P::kLo), P::kHi));
+}
+
+// in: f32 rows (pitch in floats), out: PCM rows (pitch in bytes).  Dither: flat TPDF, the group's first frame at dither
+// position pos0 + f0 (the parameters behind `total` are read only then, so the undithered kernel is the plain encode).
+template <int Fmt, bool Dither = false>
 __global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict__ in, size_t in_pitch, unsigned char* __restrict__ out,
-                                                         size_t out_pitch, size_t n_frames, size_t groups, size_t total) {
+                                                         size_t out_pitch, size_t n_frames, size_t groups, size_t total,
+                                                         unsigned long long seed, unsigned long long pos0) {
     using P = PcmTraits<Fmt>;
     constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
     for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
         const size_t row = t / groups, f0 = (t - row * groups) * G;
         const float* src = in + row * in_pitch + f0;
         unsigned char* dst = out + row * out_pitch + f0 * NB;
-        if (f0 + G <= n_frames) {
+        if constexpr (Dither) {
+            unsigned long long z = dither_row_key(seed, row) + kDitherPhi * (pos0 + f0 + 1);
+            if (f0 + G <= n_frames) {
+                int q[G];
+#pragma unroll
+                for (int v = 0; v < G / 4; ++v) {
+                    const float4 y = reinterpret_cast<const float4*>(src)[v];
+                    const float ys[4] = {y.x, y.y, y.z, y.w};
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) { q[4 * v + j] = pcm_quantise_dithered<Fmt>(ys[j], dither_noise(z)); z += kDitherPhi; }
+                }
+                unsigned w[W];
+                pcm_pack<Fmt>(q, w);
+#pragma unroll
+                for (int v = 0; v < W / 4; ++v) reinterpret_cast<uint4*>(dst)[v] = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
+            } else {
+                for (size_t k = 0; f0 + k < n_frames; ++k, z += kDitherPhi)
+                    pcm_store_one<Fmt>(dst + k * NB, pcm_quantise_dithered<Fmt>(src[k], dither_noise(z)));
+            }
+        } else if (f0 + G <= n_frames) {
             int q[G];
 #pragma unroll
             for (int v = 0; v < G / 4; ++v) {
@@ -473,6 +524,165 @@ __global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict
         } else {
             for (size_t k = 0; f0 + k < n_frames; ++k) pcm_store_one<Fmt>(dst + k * NB, pcm_quantise<Fmt>(src[k]));
         }
+    }
+}
+
+// ---- noise-shaped encode: error feedback along each row ----------------------------------------------------------
+// One frame of row r (include/ohs.h): fb = h_M e_M + ... + h_1 e_1 summed oldest first, so the loop-carried chain through
+// the newest error e_1 is one multiply and one add; w = v - fb; q = clamp(rint(w + d)); e = clamp(q - w, -1.5, 1.5).
+// Every operation is rounded on its own (the build contracts to FMA by default; the numpy reference does not).
+struct DitherTaps { float h[kShapeTaps]; };   // h[k] = h_(k+1)
+
+// rint of a value already clamped to the format's range.  S16: |t| <= 2^15, so t + 1.5 * 2^23 lies in [2^23, 2^24), where the
+// f32 ulp is 1: the add rounds to nearest even and the subtraction is exact, two 4-cycle adds on the loop-carried chain
+// instead of FRND's trip through the conversion unit.  It gives +0 where rint gives -0 (t in [-0.5, 0]); a zero of the other
+// sign only ever meets nonzero values in sums (x + -0 = x + 0 = x) and gives zeros in products, so no q changes.
+template <int Fmt> __device__ __forceinline__ float rint_clamped(float t) {
+    if constexpr (Fmt == kPcmS16) return __fsub_rn(__fadd_rn(t, 12582912.0f), 12582912.0f);
+    else return rintf(t);
+}
+
+template <int Fmt, int M>
+__device__ __forceinline__ int shaped_step(float y, float d, const DitherTaps& t, float (&e)[M]) {
+    using P = PcmTraits<Fmt>;
+    const float v = __fmul_rn(y, P::kEncode);
+    float fb = __fmul_rn(t.h[M - 1], e[M - 1]);
+#pragma unroll
+    for (int k = M - 2; k >= 0; --k) fb = __fadd_rn(fb, __fmul_rn(t.h[k], e[k]));
+    const float w = __fsub_rn(v, fb);
+    const float qf = rint_clamped<Fmt>(fminf(fmaxf(__fadd_rn(w, d), P::kLo), P::kHi));   // clamping first is the same: integer bounds
+    // NaN v: q - w is NaN, and fmaxf / fminf return the other operand, so bounds of 0 give the error 0 without a select on
+    // the chain (v is known a frame ahead; finite or infinite v never makes q - w NaN)
+    const bool nan = v != v;
+    const float en = fminf(fmaxf(__fsub_rn(qf, w), nan ? 0.f : -1.5f), nan ? 0.f : 1.5f);
+#pragma unroll
+    for (int k = M - 1; k > 0; --k) e[k] = e[k - 1];
+    e[0] = en;
+    return nan ? 0 : __float2int_rn(qf);
+}
+
+__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// The recurrence runs in order along a row, so one thread owns one row: a CTA carries 32 rows in warp 0 and walks them
+// in tiles of kShapeT frames.  The f32 tiles arrive through shared memory (coalesced 16-byte cp.async, double-buffered:
+// tile k+1 loads while tile k is computed); warps 1-3 hash the noise of tile k+1 into shared memory meanwhile, which keeps the
+// ~25 integer instructions of a noise value out of warp 0's issue slots.  Warp 0 writes the packed integers of its row to a
+// byte tile that the whole CTA stores with 16-byte stores.  Tile rows are padded by 16 bytes, so that the 16-byte
+// accesses of eight lanes to eight rows (one shared-memory wavefront) fall on distinct banks.  The history e_1..e_M of a
+// row is read from hist[row][0..M) at the start of a launch and written back at its end.
+constexpr int kShapeT = 64, kShapeRows = 32, kShapeThreads = 128, kShapeStages = 2;
+
+template <int Fmt, int M>
+__global__ void __launch_bounds__(kShapeThreads) pcm_encode_shaped_kernel(const float* __restrict__ in, size_t in_pitch,
+                                                                        unsigned char* __restrict__ out, size_t out_pitch,
+                                                                        size_t n_frames, int rows, unsigned long long seed,
+                                                                        unsigned long long pos0, DitherTaps taps,
+                                                                        float* __restrict__ hist) {
+    using P = PcmTraits<Fmt>;
+    constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
+    constexpr int T = kShapeT, R = kShapeRows, NT = kShapeThreads, IP = T + 4, OP = T * NB + 16, C4 = T / 4, C16 = T * NB / 16;
+    static_assert(T % G == 0 && (IP / 4) % 8 == 1 && (OP / 16) % 2 == 1, "whole groups per tile; conflict-free 16-byte rows");
+    __shared__ __align__(16) float xs[kShapeStages][R][IP];   // f32 input rows
+    __shared__ __align__(16) float ds[2][R][IP];              // noise
+    __shared__ __align__(16) unsigned char qs[R][OP];         // packed output rows
+    __shared__ unsigned long long keys[R];
+    const int tid = threadIdx.x, r0 = blockIdx.x * R, nr = min(R, rows - r0);
+    const size_t n_tiles = (n_frames + T - 1) / T;
+    if (tid < R) keys[tid] = dither_row_key(seed, (size_t)(r0 + tid));
+    auto load = [&](size_t k) {
+        if (k < n_tiles) {
+            const size_t f0 = k * T;
+            const int nv = (int)((min((size_t)T, n_frames - f0) + 3) / 4);   // a row's last float4 is inside its pitch
+            for (int i = tid; i < R * C4; i += NT) {
+                const int r = i / C4, c = i - r * C4;
+                if (r < nr && c < nv) cp_async16(&xs[k % kShapeStages][r][4 * c], in + (size_t)(r0 + r) * in_pitch + f0 + 4 * c);
+            }
+        }
+        cp_async_commit();   // an empty group past the last tile keeps the wait counts uniform
+    };
+    auto noise = [&](size_t k) {   // warps 1-3: the noise of tile k (every frame of it; those past n_frames go unused)
+        const unsigned long long p = pos0 + k * T + 1;
+        for (int i = tid - 32; i < R * C4; i += NT - 32) {
+            const int r = i / C4, c = i - r * C4;
+            unsigned long long z = keys[r] + kDitherPhi * (p + 4 * c);
+            float4 d;
+            d.x = dither_noise(z); z += kDitherPhi;
+            d.y = dither_noise(z); z += kDitherPhi;
+            d.z = dither_noise(z); z += kDitherPhi;
+            d.w = dither_noise(z);
+            *reinterpret_cast<float4*>(&ds[k & 1][r][4 * c]) = d;
+        }
+    };
+    float e[M];
+    const bool owner = tid < nr;
+#pragma unroll
+    for (int k = 0; k < M; ++k) e[k] = owner ? hist[(size_t)(r0 + tid) * kShapeTaps + k] : 0.f;
+    load(0);
+    __syncthreads();   // keys
+    if (tid >= 32) noise(0);
+    for (size_t k = 0; k < n_tiles; ++k) {
+        load(k + 1);
+        cp_async_wait<1>();   // this thread's copies of tile k have landed ...
+        __syncthreads();      // ... and everybody's; the noise of tile k is written
+        const size_t f0 = k * T;
+        const int nf = (int)min((size_t)T, n_frames - f0);
+        if (owner) {
+            const float4* x = reinterpret_cast<const float4*>(xs[k % kShapeStages][tid]);
+            const float4* dn = reinterpret_cast<const float4*>(ds[k & 1][tid]);
+            unsigned char* o = qs[tid];
+            // a group's samples and noise are read one group ahead, so that the chain does not wait for shared memory
+            float xc[G], dc[G];
+            auto fetch = [&](int g, float (&xv)[G], float (&dv)[G]) {
+#pragma unroll
+                for (int v = 0; v < G / 4; ++v) {
+                    const float4 a = x[g / 4 + v], b = dn[g / 4 + v];
+                    xv[4 * v] = a.x; xv[4 * v + 1] = a.y; xv[4 * v + 2] = a.z; xv[4 * v + 3] = a.w;
+                    dv[4 * v] = b.x; dv[4 * v + 1] = b.y; dv[4 * v + 2] = b.z; dv[4 * v + 3] = b.w;
+                }
+            };
+            fetch(0, xc, dc);
+#pragma unroll 1
+            for (int g = 0; g < nf; g += G) {
+                float xn[G], dnx[G];
+                fetch(g + G < nf ? g + G : g, xn, dnx);
+                int q[G];
+                if (g + G <= nf) {
+#pragma unroll
+                    for (int j = 0; j < G; ++j) q[j] = shaped_step<Fmt, M>(xc[j], dc[j], taps, e);
+                } else {   // the call's last, partial group: only its frames step the filter
+#pragma unroll
+                    for (int j = 0; j < G; ++j) q[j] = g + j < nf ? shaped_step<Fmt, M>(xc[j], dc[j], taps, e) : 0;
+                }
+#pragma unroll
+                for (int j = 0; j < G; ++j) { xc[j] = xn[j]; dc[j] = dnx[j]; }
+                unsigned w[W];
+                pcm_pack<Fmt>(q, w);
+#pragma unroll
+                for (int v = 0; v < W / 4; ++v)
+                    *reinterpret_cast<uint4*>(o + g * NB + 16 * v) = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
+            }
+        } else if (tid >= 32 && k + 1 < n_tiles) {
+            noise(k + 1);
+        }
+        __syncthreads();   // the byte tile is complete
+        const int nb = nf * NB;
+        for (int i = tid; i < R * C16; i += NT) {
+            const int r = i / C16, c = i - r * C16;
+            if (r >= nr || 16 * c >= nb) continue;
+            unsigned char* dst = out + (size_t)(r0 + r) * out_pitch + f0 * NB + 16 * c;
+            const unsigned char* src = &qs[r][16 * c];
+            if (16 * c + 16 <= nb) *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(src);
+            else for (int b = 0; b < nb - 16 * c; ++b) dst[b] = src[b];   // nothing past n_frames is touched
+        }
+        __syncthreads();   // the byte tile and this tile's input stage are free again
+    }
+    if (owner) {
+#pragma unroll
+        for (int k = 0; k < M; ++k) hist[(size_t)(r0 + tid) * kShapeTaps + k] = e[k];
     }
 }
 

@@ -20,6 +20,8 @@ ABI_VERSION = 2   # OHS_ABI_VERSION of include/ohs.h this binding was written ag
 LSL, LSR, RSL, RSR = 0, 1, 2, 3
 PEAK, LOWSHELF, HIGHSHELF, LOWPASS, HIGHPASS, BANDPASS, NOTCH, ALLPASS = range(8)
 FMT_F32, FMT_S16, FMT_S24 = 0, 1, 2   # ohs_sample_format
+DITHER_OFF, DITHER_TPDF = 0, 1        # OHS_DITHER_*
+MAX_SHAPE_TAPS = 9                    # OHS_MAX_SHAPE_TAPS
 
 _f32p = C.POINTER(C.c_float)
 
@@ -70,6 +72,7 @@ SYMBOLS = [
     ("ohs_process_fifo", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t]),
     ("ohs_process_pcm", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_int, C.c_size_t, C.c_size_t]),
     ("ohs_process_device_pcm", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_int, C.c_size_t, C.c_size_t]),
+    ("ohs_set_dither", C.c_int, [_VP, C.c_int, C.c_uint64, _f32p, C.c_int]),
     ("ohs_sync", C.c_int, [_VP]),
     ("ohs_cuda_stream", C.c_int, [_VP, C.POINTER(_VP)]),
     ("ohs_launch_count", C.c_int, [_VP, C.POINTER(C.c_uint64)]),
@@ -362,6 +365,12 @@ class Engine:
         """Device flavour of process_pcm on raw device pointers; row_stride counts frames for both buffers."""
         _check(self._L.ohs_process_device_pcm(self._h, d_in, in_format, d_out, out_format, n_frames,
                                               n_frames if row_stride is None else row_stride))
+
+    def set_dither(self, mode: int, seed: int = 0, shape=()):
+        """Dither of integer PCM output (ohs_set_dither): DITHER_OFF or DITHER_TPDF, noise-shaped by the error-feedback taps
+        `shape` = (h_1, ..., h_M), M <= MAX_SHAPE_TAPS.  Resets the dither position and error history."""
+        h = _f32(shape).ravel()
+        _check(self._L.ohs_set_dither(self._h, mode, seed, h.ctypes.data_as(_f32p) if h.size else None, h.size))
 
     def process_fifo(self, x) -> np.ndarray:
         x = _f32(x)

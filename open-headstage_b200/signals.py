@@ -103,6 +103,77 @@ def pcm_encode(y, fmt: int) -> np.ndarray:
     return r.astype(np.int16 if fmt == 1 else np.int32)
 
 
+# Dither of integer PCM output (include/ohs.h, ohs_set_dither), exact to the bit: uint64 arithmetic wraps like C's
+_PHI = np.uint64(0x9E3779B97F4A7C15)
+
+
+def _mix64(z):
+    """SplitMix64's finaliser on uint64 arrays."""
+    z = np.asarray(z, np.uint64)
+    with np.errstate(over="ignore"):
+        z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    return z ^ (z >> np.uint64(31))
+
+
+def tpdf_noise(seed: int, rows, position: int, n: int) -> np.ndarray:
+    """The dither noise d of rows `rows` (r = 2*stream + channel) at positions position .. position + n - 1: float32
+    [len(rows), n], multiples of 2^-23 in (-1, 1)."""
+    r = np.atleast_1d(np.asarray(rows, np.uint64))
+    p = np.uint64(position) + np.arange(n, dtype=np.uint64)
+    with np.errstate(over="ignore"):
+        key = _mix64(np.uint64(seed) + _PHI * (r + np.uint64(1)))
+        x = _mix64(key[:, None] + _PHI * (p[None, :] + np.uint64(1)))
+    u1 = (x & np.uint64(0x7FFFFF)).astype(np.int64)
+    u2 = ((x >> np.uint64(32)) & np.uint64(0x7FFFFF)).astype(np.int64)
+    return ((u1 + u2 - 0x7FFFFF).astype(np.float32) * np.float32(2.0 ** -23)).astype(np.float32)
+
+
+def _shape_rows(v, d, h, e, lo, hi):
+    """The error-feedback recurrence on float32 rows v[R, n] with noise d[R, n], taps h[M] and history e[R, M] (most recent
+    first, updated in place).  Returns (q as float32, q - w before the error clamp)."""
+    m = len(h)
+    q = np.empty_like(v)
+    raw = np.empty_like(v)
+    lo, hi, lim = np.float32(lo), np.float32(hi), np.float32(1.5)
+    with np.errstate(invalid="ignore"):
+        for i in range(v.shape[1]):
+            fb = h[m - 1] * e[:, m - 1]
+            for k in range(m - 2, -1, -1):
+                fb = fb + h[k] * e[:, k]
+            w = v[:, i] - fb
+            qf = np.clip(np.rint(w + d[:, i]), lo, hi)
+            err = qf - w
+            nan = np.isnan(v[:, i])
+            q[:, i] = np.where(nan, np.float32(0.0), qf)
+            raw[:, i] = np.where(nan, np.float32(0.0), err)
+            e[:, 1:] = e[:, :-1]
+            e[:, 0] = np.where(nan, np.float32(0.0), np.clip(err, -lim, lim))
+    return q, raw
+
+
+def pcm_encode_dithered(y, fmt: int, seed: int, position: int, shape=(), state=None):
+    """The dithered encode of include/ohs.h (ohs_set_dither): y[..., n] float32 rows, row r = the flat index over the
+    leading axes (2*stream + channel for [S, 2, n]), frame f at dither position position + f.  shape = (h_1, ..., h_M)
+    noise-shapes; `state` is the error history [rows, M] (most recent first, None = zeros after ohs_set_dither).
+    Returns (q, state): int16 for S16, int32 (unpacked) for S24, and the history after the last frame."""
+    b = PCM_BITS[fmt]
+    y = np.asarray(y, dtype=np.float32)
+    v = (y.reshape(-1, y.shape[-1]) * np.float32(2.0 ** (b - 1))).astype(np.float32)
+    rows, n = v.shape
+    d = tpdf_noise(seed, np.arange(rows), position, n)
+    lo, hi = -(2.0 ** (b - 1)), 2.0 ** (b - 1) - 1
+    h = np.asarray(shape, np.float32).ravel()
+    e = np.zeros((rows, h.size), np.float32) if state is None else np.array(state, np.float32).reshape(rows, h.size)
+    if h.size == 0:
+        with np.errstate(invalid="ignore"):
+            q = np.clip(np.rint(v + d), lo, hi)
+        q = np.where(np.isnan(v), np.float32(0.0), q)
+    else:
+        q, _ = _shape_rows(v, d, h, e, lo, hi)
+    return q.astype(np.int16 if fmt == 1 else np.int32).reshape(y.shape), e
+
+
 # BASELINE.json configs -> engine parameters (SURVEY.md §8d table)
 CONFIGS = {
     1: dict(name="cfg1: 1 stereo stream, 48 kHz, SOFA 200-tap HRIR, block 512", n_streams=1, fs=48000.0, block=512, taps=200),
