@@ -271,13 +271,47 @@ int ohs_launch_count(ohs_engine* h, uint64_t* out);
 int ohs_enable_timing(ohs_engine* h, int enable);
 int ohs_last_kernel_ms(ohs_engine* h, float* ms);
 
+/* ---- listener buses: groups of streams mixed into one binaural bus each (an extension) ------------------------------
+ * A 5.1 or 7.1 file is 3 or 4 speaker pairs, one stream each (sofa.wire_speakers wires a pair to its own HRIR set); a
+ * listener's object scene is its sources, two mono sources per stream (below).  Either way a group of streams is summed
+ * into one stereo bus.  Partition the streams into n_groups contiguous groups: group g holds streams
+ * first[g] .. first[g+1]-1.  first is HOST memory with n_groups + 1 entries: first[0] == 0, strictly increasing,
+ * first[n_groups] == n_streams, 1 <= n_groups <= n_streams.  Default (and after ohs_create): one group holding every
+ * stream.  Like bindings, groups are configuration: not part of the state blob, and they change no stream's rendering.
+ * OHS_ERR_INVALID with the engine untouched for anything else.  The offsets are uploaded once, here, on the engine's
+ * stream (mixes enqueued before use the old ones).
+ * Bus layout everywhere: row 2*g + c (c 0 = left, 1 = right) at bus + (2*g + c) * bus_stride, and with f = first[g]
+ *   bus[g][c][n] = ((((+0) + y[f][c][n]) + y[f+1][c][n]) + y[f+2][c][n]) + ...
+ * in ascending stream order, every addition rounded to f32 (numpy reference: signals.mix_groups).  Starting from +0
+ * differs from starting with y[f] only where every term is -0: the bus is +0 there.
+ * Not provided: integer bus output and dither of buses (dither history rows are defined per stream row; sharing them
+ * with bus rows needs a definition of its own), grouped forms of ohs_process_fifo and ohs_process_device_scheduled (on
+ * the device, compose ohs_process_device_scheduled with ohs_mix_device), non-contiguous groups, and a mix fused into the
+ * render kernel (DESIGN §13). */
+int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups);
+/* The group count in force (bus rows = 2 * *out). */
+int ohs_num_groups(ohs_engine* h, int* out);
+
 /* Object mixdown (BASELINE config 4; an extension — the reference has no multi-source mode): sums the rendered
- * streams of this engine into one stereo bus, d_bus[c * bus_stride + n] = sum_s d_in[(s*2 + c) * row_stride + n].
+ * streams of each group (ohs_set_groups; by default one group of every stream) into its stereo bus, 2 * n_groups rows
+ * of the layout above: d_bus[(2*g + c) * bus_stride + n] = sum over s in group g of d_in[(s*2 + c) * row_stride + n].
  * Two mono sources ride in one stereo stream: source A as the left input with paths (LSL, LSR) = its (left-ear,
  * right-ear) HRIRs, source B as the right input with (RSL, RSR); the engine's output is already their binaural mix
  * (src/dsp/convolution.rs:229-230).  n_frames must be a multiple of 4; pointers 16-byte aligned.  Enqueues on the
- * engine's stream.  The per-GPU buses are then summed with NCCL (parallel.reduce_bus). */
+ * engine's stream; the bus padding is not touched.  The per-GPU buses are then summed with NCCL (parallel.reduce_bus, or
+ * ohs_reduce_bus over all 2 * n_groups * bus_stride floats: per-listener buses reduce across GPUs the same way). */
 int ohs_mix_device(ohs_engine* h, const float* d_in, float* d_bus, size_t n_frames, size_t row_stride, size_t bus_stride);
+/* Host memory.  Renders exactly what ohs_process_pcm(h, in, in_format, <rows>, OHS_FMT_F32, n_frames, row_stride) renders,
+ * cut into the same chunks (so the time-batched route too is bit-identical), and returns only the group buses:
+ * bus (host, f32) [2*n_groups][bus_stride], each chunk's buses mixed on the GPU so that only they cross PCIe back.
+ * Engine state afterwards == state after that ohs_process_pcm call (pending moves, EQ-only mode, gains and bindings
+ * behave as there).  Bypass: bus = mix(decode(in)), state untouched.  The dither position does not move (no integer
+ * output).  Checked before anything is enqueued (OHS_ERR_INVALID, engine untouched): the argument rules of
+ * ohs_process_pcm with F32 output (an unknown format, n_frames not a multiple of B while the convolution is on,
+ * row_stride < n_frames), a null bus, bus_stride < n_frames, a bus that overlaps the input bytes.  ohs_prepare(h, n, 1)
+ * also allocates the bus staging. */
+int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
+                        size_t bus_stride);
 
 /* ---- multi-GPU collectives (SURVEY.md 8e) -------------------------------------------------------------------------
  * Streams shard across GPUs with no data-path collective; NCCL is used for exactly two things, both available here so

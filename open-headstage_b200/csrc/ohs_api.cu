@@ -100,6 +100,9 @@ struct ohs_engine {
     // ... and its integer-PCM rows: the PCM rows of a chunk, both directions, beside d_stage
     unsigned char* d_pcm_stage[kPipe] = {nullptr, nullptr, nullptr};
     size_t pcm_stage_cap = 0;
+    // ... and ohs_process_grouped's bus rows of a chunk (2 * n_groups rows), beside d_stage
+    float* d_bus_stage[kPipe] = {nullptr, nullptr, nullptr};
+    size_t bus_stage_cap = 0;
     // f32 rows of ohs_process_device_pcm's time chunks (decoded input, rendered in place)
     float* d_pcm_scratch = nullptr;
     size_t pcm_scratch_cap = 0;
@@ -109,6 +112,11 @@ struct ohs_engine {
     unsigned long long dither_seed = 0, dither_pos = 0;
     ohs::DitherTaps dither_h{};
     float* d_dither_hist = nullptr;   // [2 * n_streams][OHS_MAX_SHAPE_TAPS], allocated by ohs_set_dither
+
+    // listener buses (ohs_set_groups): group g holds streams h_group_first[g] .. h_group_first[g+1]-1; configuration like the
+    // bindings, not state.  d_group_first is sized for n_streams groups.
+    std::vector<int> h_group_first;
+    int* d_group_first = nullptr;
 
     // time-batched long-response path: spectra in time order and frequency-domain products of one sub-launch
     float2* d_zlin = nullptr;
@@ -465,6 +473,20 @@ int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t p
         pcm_encode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
     else
         pcm_encode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
+    OHS_CUDA(cudaGetLastError());
+    h->launches++;
+    return OHS_OK;
+}
+
+int n_groups(const ohs_engine* h) { return (int)h->h_group_first.size() - 1; }
+
+// The group buses of f32 rows on the engine's stream: 2 * n_groups rows of `bus` (ohs_mix_device, ohs_process_grouped).
+// A plain launch, without the programmatic-serialization attribute: it starts once the render before it has finished.
+int launch_mix(ohs_engine* h, const float* in, size_t row_stride, float* bus, size_t bus_stride, size_t n_frames) {
+    const unsigned threads = 256;
+    const int rows = 2 * n_groups(h);
+    const dim3 grid((unsigned)(((n_frames + 3) / 4 + threads - 1) / threads), (unsigned)std::min(rows, 65535));
+    mix_streams_kernel<<<grid, threads, 0, h->stream>>>(in, bus, h->d_group_first, rows, n_frames, row_stride, bus_stride);
     OHS_CUDA(cudaGetLastError());
     h->launches++;
     return OHS_OK;
@@ -850,6 +872,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     const size_t per_path = (size_t)h->pmax * B;
 
     h->h_stream_hrir.assign(S, 0);
+    h->h_group_first = {0, S};
     h->h_move_to.assign(S, -1);
     h->h_stream_eq.assign(S, 0);
     h->h_gain.assign(S, 1.0f);
@@ -892,6 +915,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     h->filt_bytes = sizeof(float4) * (size_t)cfg->n_hrir_sets * h->pmax * h->N;
     OHS_TRY(cudaMalloc(&h->d_stream_hrir, sizeof(int) * S));
     OHS_TRY(cudaMalloc(&h->d_from_set, sizeof(int) * S));
+    OHS_TRY(cudaMalloc(&h->d_group_first, sizeof(int) * ((size_t)S + 1)));
     OHS_TRY(cudaMalloc(&h->d_stream_eq, sizeof(int) * S));
     OHS_TRY(cudaMalloc(&h->d_stream_gain, sizeof(float) * S));
     OHS_TRY(cudaMalloc(&h->d_filt, h->filt_bytes));
@@ -920,6 +944,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
         }
         OHS_TRY(cudaMemcpyAsync(h->d_tw, tw.data(), sizeof(float2) * h->N, cudaMemcpyHostToDevice, h->stream));
         OHS_TRY(cudaMemcpyAsync(h->d_set_parts, h->h_set_parts.data(), sizeof(int) * cfg->n_hrir_sets, cudaMemcpyHostToDevice, h->stream));
+        OHS_TRY(cudaMemcpyAsync(h->d_group_first, h->h_group_first.data(), sizeof(int) * 2, cudaMemcpyHostToDevice, h->stream));
         OHS_TRY(cudaStreamSynchronize(h->stream));
     }
 #undef OHS_TRY
@@ -937,7 +962,8 @@ int ohs_destroy(ohs_engine* h) {
     void* ptrs[] = {h->d_stream_hrir, h->d_stream_eq, h->d_stream_gain, h->d_filt, h->d_set_parts, h->d_set_list, h->d_set_flags,
                     h->d_fdl, h->d_prev, h->d_eqc, h->d_eqs, h->d_tw, h->d_ir, h->d_stage[0], h->d_stage[1], h->d_stage[2],
                     h->d_zlin, h->d_wlin, h->d_xf, h->d_from_set, h->d_sched, h->d_pcm_stage[0], h->d_pcm_stage[1],
-                    h->d_pcm_stage[2], h->d_pcm_scratch, h->d_dither_hist};
+                    h->d_pcm_stage[2], h->d_pcm_scratch, h->d_dither_hist, h->d_group_first, h->d_bus_stage[0],
+                    h->d_bus_stage[1], h->d_bus_stage[2]};
     for (void* p : ptrs) if (p) cudaFree(p);
     for (int i = 0; i < kPipe; ++i) {
         if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
@@ -1163,8 +1189,11 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io) {
         const size_t rows = (size_t)h->cfg.n_streams * 2;
         per_launch = chunk_frames(h, n_frames, h->stage_bytes, 2);
         const size_t pcm_bytes = rows * std::max(per_launch * 2, chunk_frames(h, n_frames, h->stage_bytes, 3) * 3);
+        // ohs_process_grouped's bus rows: its chunks are those of F32 output
+        const size_t bus_bytes = (size_t)2 * n_groups(h) * chunk_frames(h, n_frames, h->stage_bytes, sizeof(float)) * sizeof(float);
         if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * per_launch * sizeof(float))) ||
-            (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, pcm_bytes)))
+            (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, pcm_bytes)) ||
+            (rc = grow_buffers(h, h->d_bus_stage, kPipe, h->bus_stage_cap, bus_bytes)))
             return rc;
     } else if (n_frames) {
         rc = ensure_pcm_scratch(h, chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float)));   // ohs_process_device_pcm
@@ -1414,11 +1443,30 @@ int ohs_mix_device(ohs_engine* h, const float* d_in, float* d_bus, size_t n_fram
     if (row_stride < n_frames || bus_stride < n_frames) return fail(OHS_ERR_INVALID, "stride smaller than n_frames");
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     if (n_frames == 0) return OHS_OK;
-    const unsigned threads = 256;
-    dim3 grid((unsigned)((n_frames / 4 + threads - 1) / threads), 2);
-    mix_streams_kernel<<<grid, threads, 0, h->stream>>>(d_in, d_bus, h->cfg.n_streams, n_frames, row_stride, bus_stride);
-    OHS_CUDA(cudaGetLastError());
-    h->launches++;
+    return launch_mix(h, d_in, row_stride, d_bus, bus_stride, n_frames);
+}
+
+int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups) {
+    OHS_CHECK_HANDLE(h);
+    const int S = h->cfg.n_streams;
+    if (!first) return fail(OHS_ERR_INVALID, "null group offsets");
+    if (n_groups < 1 || n_groups > S) return fail(OHS_ERR_INVALID, "n_groups %d outside 1..%d", n_groups, S);
+    if (first[0] != 0 || first[n_groups] != S)
+        return fail(OHS_ERR_INVALID, "group offsets must run from 0 to n_streams %d (got %d .. %d)", S, first[0], first[n_groups]);
+    for (int g = 0; g < n_groups; ++g)
+        if (first[g + 1] <= first[g]) return fail(OHS_ERR_INVALID, "group %d is empty or the offsets decrease (%d, %d)", g, first[g], first[g + 1]);
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    std::vector<int> v(first, first + n_groups + 1);
+    // on the engine's stream: mixes enqueued before still read the old offsets (a pageable source is staged before returning)
+    OHS_CUDA(cudaMemcpyAsync(h->d_group_first, v.data(), sizeof(int) * v.size(), cudaMemcpyHostToDevice, h->stream));
+    h->h_group_first.swap(v);
+    return OHS_OK;
+}
+
+int ohs_num_groups(ohs_engine* h, int* out) {
+    OHS_CHECK_HANDLE(h);
+    if (!out) return fail(OHS_ERR_INVALID, "null output");
+    *out = n_groups(h);
     return OHS_OK;
 }
 
@@ -1574,20 +1622,26 @@ int ohs_host_free(void* p) {
     return OHS_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
 // Host-pointer flavour: time chunks are staged through three slots in HBM; copy-in, kernels and copy-out of consecutive
 // chunks overlap on three CUDA streams.  Integer PCM crosses the link as PCM and is converted in HBM.  Per chunk: copy-in
 // (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into the f32 buffer, render
-// there in place, encode back into the PCM buffer, copy-out.  ohs_process is the F32 -> F32 case.
-int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride) {
-    OHS_CHECK_HANDLE(h);
-    int rc = check_pcm_args(h, in, in_format, out, out_format, n_frames, row_stride, false);
-    if (rc) return rc;
+// there in place, encode back into the PCM buffer, copy-out.  ohs_process is the F32 -> F32 case.  With `bus`
+// (ohs_process_grouped: F32 output, `out` unused) the rendered rows are mixed into the slot's group buses instead, and
+// only those 2 * n_groups rows are copied out.  Arguments are validated by the caller.
+int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride,
+                      float* bus = nullptr, size_t bus_stride = 0) {
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     if (n_frames == 0) return OHS_OK;
+    int rc = OHS_OK;
     const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
+    const size_t bus_rows = (size_t)2 * n_groups(h);
     const unsigned char* src = static_cast<const unsigned char*>(in);
     unsigned char* dst = static_cast<unsigned char*>(out);
-    if (h->bypass && in_format == out_format) {
+    if (h->bypass && in_format == out_format && !bus) {
         if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(dst + r * row_stride * bo, src + r * row_stride * bi, n_frames * bi);
         if (out_format != OHS_FMT_F32) h->dither_pos += n_frames;
         return OHS_OK;
@@ -1597,7 +1651,8 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     // directions busy (tools/e2e_probe.py)
     const size_t chunk = chunk_frames(h, n_frames, h->stage_bytes, std::max(bi, bo));
     if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * chunk * sizeof(float))) ||
-        (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0))))
+        (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0))) ||
+        (bus && (rc = grow_buffers(h, h->d_bus_stage, kPipe, h->bus_stage_cap, bus_rows * chunk * sizeof(float)))))
         return rc;
     if (!h->bypass) {
         rc = commit_filters(h);
@@ -1613,6 +1668,7 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
         const int b = idx % kPipe;
         float* x = h->d_stage[b];
         unsigned char* q = h->d_pcm_stage[b];
+        float* g = h->d_bus_stage[b];
         if (used[b]) OHS_CUDA(cudaStreamWaitEvent(h->h2d, h->ev_out[b], 0));  // buffers free once their copy-out finished
         if (pcm_in)
             OHS_CUDA(cudaMemcpy2DAsync(q, pcm_pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
@@ -1623,9 +1679,13 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
         if (pcm_in && (rc = launch_pcm(h, true, in_format, q, pcm_pitch * bi, x, pitch, n))) return rc;
         if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
         if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n, done))) return rc;
+        if (bus && (rc = launch_mix(h, x, pitch, g, pitch, n))) return rc;
         OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
         OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
-        if (pcm_out)
+        if (bus)
+            OHS_CUDA(cudaMemcpy2DAsync(bus + done, bus_stride * sizeof(float), g, pitch * sizeof(float), n * sizeof(float), bus_rows,
+                                       cudaMemcpyDeviceToHost, h->d2h));
+        else if (pcm_out)
             OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, q, pcm_pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
         else
             OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, x, pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
@@ -1638,6 +1698,34 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     if (pcm_out) h->dither_pos += n_frames;
     return OHS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride) {
+    OHS_CHECK_HANDLE(h);
+    const int rc = check_pcm_args(h, in, in_format, out, out_format, n_frames, row_stride, false);
+    if (rc) return rc;
+    return process_host_impl(h, in, in_format, out, out_format, n_frames, row_stride);
+}
+
+int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
+                        size_t bus_stride) {
+    OHS_CHECK_HANDLE(h);
+    if (in_format != OHS_FMT_F32 && in_format != OHS_FMT_S16 && in_format != OHS_FMT_S24)
+        return fail(OHS_ERR_INVALID, "unknown sample format %d", in_format);
+    int rc = check_audio_args(h, in, bus, n_frames, row_stride, false);
+    if (rc) return rc;
+    if (bus_stride < n_frames) return fail(OHS_ERR_INVALID, "bus_stride %zu < n_frames %zu", bus_stride, n_frames);
+    // the decode or copy-in of a later chunk must not read what the copy-out of an earlier one has written
+    const size_t rows = (size_t)h->cfg.n_streams * 2, bus_rows = (size_t)2 * n_groups(h);
+    const uintptr_t a = (uintptr_t)in, b = (uintptr_t)bus;
+    const size_t na = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(in_format);
+    const size_t nb = ((bus_rows - 1) * bus_stride + n_frames) * sizeof(float);
+    if (a < b + nb && b < a + na) return fail(OHS_ERR_INVALID, "the bus overlaps the input");
+    return process_host_impl(h, in, in_format, nullptr, OHS_FMT_F32, n_frames, row_stride, bus, bus_stride);
 }
 
 int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride) {

@@ -333,21 +333,36 @@ __global__ void clear_history_kernel(float2* fdl, float2* prev, const int* strea
     for (size_t i = threadIdx.x; i < prev_per_stream; i += blockDim.x) q[i] = make_float2(0.f, 0.f);
 }
 
-// Object mixdown (BASELINE config 4): bus[c][n] = sum over streams of in[s][c][n].  Sequential f32 sum in stream order
-// (deterministic); one thread per four frames, rows read with coalesced 16-byte loads.
-__global__ void mix_streams_kernel(const float* __restrict__ in, float* __restrict__ bus, int n_streams, size_t n_frames,
-                                   size_t row_stride, size_t bus_stride) {
+// Group buses (ohs_set_groups; BASELINE config 4 is the single group of every stream): bus row 2g + c is the sum over the
+// streams first[g] .. first[g+1]-1 of in[s][c][n], a sequential f32 sum from +0 in stream order (deterministic).  One thread
+// per four frames and bus row: grid.x over 4-frame quads, grid.y over the 2G bus rows (rows past gridDim.y loop), so that
+// groups of three or four streams still fill the GPU; rows read with coalesced 16-byte loads.  A row's last, partial quad
+// (EQ-only calls of any length) is summed sample by sample, touching nothing past n_frames.
+__global__ void mix_streams_kernel(const float* __restrict__ in, float* __restrict__ bus, const int* __restrict__ group_first,
+                                   int n_rows, size_t n_frames, size_t row_stride, size_t bus_stride) {
     const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;  // float4 index inside a row
-    const int c = blockIdx.y;
     if (q * 4 >= n_frames) return;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    const float* row = in + (size_t)c * row_stride + q * 4;
+    for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+        const int g = r >> 1, c = r & 1;
+        const int s0 = group_first[g], s1 = group_first[g + 1];
+        const float* row = in + ((size_t)s0 * 2 + c) * row_stride + q * 4;
+        float* dst = bus + (size_t)r * bus_stride + q * 4;
+        if (q * 4 + 4 <= n_frames) {
+            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 4
-    for (int s = 0; s < n_streams; ++s) {
-        const float4 v = *reinterpret_cast<const float4*>(row + (size_t)s * 2 * row_stride);
-        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+            for (int s = s0; s < s1; ++s) {
+                const float4 v = *reinterpret_cast<const float4*>(row + (size_t)(s - s0) * 2 * row_stride);
+                acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+            }
+            *reinterpret_cast<float4*>(dst) = acc;
+        } else {
+            for (size_t k = 0; q * 4 + k < n_frames; ++k) {
+                float acc = 0.f;
+                for (int s = s0; s < s1; ++s) acc += row[(size_t)(s - s0) * 2 * row_stride + k];
+                dst[k] = acc;
+            }
+        }
     }
-    *reinterpret_cast<float4*>(bus + (size_t)c * bus_stride + q * 4) = acc;
 }
 
 // ---------------------------------------------------------------------------------------------------------------

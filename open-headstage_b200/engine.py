@@ -79,6 +79,9 @@ SYMBOLS = [
     ("ohs_enable_timing", C.c_int, [_VP, C.c_int]),
     ("ohs_last_kernel_ms", C.c_int, [_VP, C.POINTER(C.c_float)]),
     ("ohs_mix_device", C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_size_t, C.c_size_t]),
+    ("ohs_set_groups", C.c_int, [_VP, _VP, C.c_int]),
+    ("ohs_num_groups", C.c_int, [_VP, C.POINTER(C.c_int)]),
+    ("ohs_process_grouped", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_size_t, C.c_size_t, C.c_size_t]),
     ("ohs_comm_unique_id", C.c_int, [_VP]),
     ("ohs_comm_create", C.c_int, [C.POINTER(_VP), C.c_int, C.c_int, C.c_int, _VP]),
     ("ohs_comm_destroy", C.c_int, [_VP]),
@@ -132,6 +135,22 @@ def _check(rc: int):
 
 def _f32(a) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(a, dtype=np.float32))
+
+
+def _pcm_input(x, n_streams: int):
+    """The input of process_pcm / process_grouped: (contiguous array, ohs_sample_format, frames), the format from the dtype."""
+    x = np.asarray(x)
+    if x.ndim != 3 or x.shape[0] != n_streams or x.shape[1] != 2:
+        raise ValueError("x must be [n_streams, 2, frames], got %s" % (x.shape,))
+    if x.dtype == np.int16:
+        fmt, n = FMT_S16, x.shape[2]
+    elif x.dtype == np.float32:
+        fmt, n = FMT_F32, x.shape[2]
+    elif x.dtype == np.uint8 and x.shape[2] % 3 == 0:
+        fmt, n = FMT_S24, x.shape[2] // 3
+    else:
+        raise ValueError("process_pcm takes int16, float32 or packed 24-bit uint8 [S, 2, 3n] input, got %s %s" % (x.dtype, x.shape))
+    return np.ascontiguousarray(x), fmt, n
 
 
 def eq_design(filter_type: int, fs: float, fc: float, q: float, gain_db: float) -> np.ndarray:
@@ -336,21 +355,10 @@ class Engine:
         """Host flavour with integer PCM (ohs_process_pcm).  The input format follows the dtype: int16 [S, 2, n] is S16,
         float32 [S, 2, n] is F32, uint8 [S, 2, 3n] is packed S24 (signals.pack_s24).  Returns int16 [S, 2, n] for
         FMT_S16, uint8 [S, 2, 3n] for FMT_S24, float32 [S, 2, n] for FMT_F32 (or fills `out`, e.g. a PinnedBuffer's array)."""
-        x = np.asarray(x)
-        if x.ndim != 3 or x.shape[0] != self.n_streams or x.shape[1] != 2:
-            raise ValueError("x must be [n_streams, 2, frames], got %s" % (x.shape,))
-        if x.dtype == np.int16:
-            fmt, n = FMT_S16, x.shape[2]
-        elif x.dtype == np.float32:
-            fmt, n = FMT_F32, x.shape[2]
-        elif x.dtype == np.uint8 and x.shape[2] % 3 == 0:
-            fmt, n = FMT_S24, x.shape[2] // 3
-        else:
-            raise ValueError("process_pcm takes int16, float32 or packed 24-bit uint8 [S, 2, 3n] input, got %s %s" % (x.dtype, x.shape))
+        x, fmt, n = _pcm_input(x, self.n_streams)
         shape = {FMT_F32: (n, np.float32), FMT_S16: (n, np.int16), FMT_S24: (3 * n, np.uint8)}
         if out_format not in shape:
             raise ValueError("unknown sample format %r" % (out_format,))
-        x = np.ascontiguousarray(x)
         want = ((self.n_streams, 2, shape[out_format][0]), np.dtype(shape[out_format][1]))
         if out is None:
             y = np.empty(*want)
@@ -360,6 +368,39 @@ class Engine:
                 raise ValueError("out must be a writeable C-contiguous %s array of shape %s" % (want[1], want[0]))
         _check(self._L.ohs_process_pcm(self._h, x.ctypes.data, fmt, y.ctypes.data, out_format, n, n))
         return y
+
+    def set_groups(self, first):
+        """Listener buses (ohs_set_groups): group g holds streams first[g] .. first[g+1]-1, first[0] = 0, strictly increasing,
+        first[-1] = n_streams.  Used by process_grouped and mix_device."""
+        f = np.ascontiguousarray(np.asarray(first, dtype=np.int32).ravel())
+        if f.size < 2:
+            raise ValueError("first needs n_groups + 1 >= 2 entries, got %d" % f.size)
+        _check(self._L.ohs_set_groups(self._h, f.ctypes.data, f.size - 1))
+
+    @property
+    def n_groups(self) -> int:
+        """The group count in force, read from the library (ohs_num_groups)."""
+        n = C.c_int()
+        _check(self._L.ohs_num_groups(self._h, C.byref(n)))
+        return n.value
+
+    def process_grouped(self, x, out=None, bus_stride: int | None = None) -> np.ndarray:
+        """Host flavour returning only the group buses (ohs_process_grouped): renders what process_pcm(x, FMT_F32) renders
+        and returns the buses as float32 [n_groups, 2, n] (the input format follows the dtype, as in process_pcm).  `out`:
+        a writeable C-contiguous float32 [n_groups, 2, bus_stride] array (e.g. a PinnedBuffer's); the first n frames of
+        each of its rows are written and returned as a view."""
+        x, fmt, n = _pcm_input(x, self.n_streams)
+        bs = n if bus_stride is None else int(bus_stride)
+        want = (self.n_groups, 2, bs)
+        if out is None:
+            y = np.empty(want, np.float32)
+        else:
+            y = out
+            if not (isinstance(y, np.ndarray) and y.dtype == np.float32 and y.shape == want and y.flags["C_CONTIGUOUS"]
+                    and y.flags["WRITEABLE"]):
+                raise ValueError("out must be a writeable C-contiguous float32 array of shape %s" % (want,))
+        _check(self._L.ohs_process_grouped(self._h, x.ctypes.data, fmt, y.ctypes.data, n, n, bs))
+        return y[:, :, :n]
 
     def process_device_pcm(self, d_in: int, in_format: int, d_out: int, out_format: int, n_frames: int, row_stride: int | None = None):
         """Device flavour of process_pcm on raw device pointers; row_stride counts frames for both buffers."""
@@ -393,7 +434,8 @@ class Engine:
         _check(self._L.ohs_process_device_scheduled(self._h, d_in, d_out, n_frames, rs, sched.ctypes.data, sched.shape[1]))
 
     def mix_device(self, d_in: int, d_bus: int, n_frames: int, row_stride: int | None = None, bus_stride: int | None = None):
-        """Sum this engine's rendered streams into a stereo bus [2][bus_stride] (config 4 object mixdown)."""
+        """Sum the rendered streams of each group (set_groups; by default one group of every stream, the config 4 object
+        mixdown) into its stereo bus: 2 * n_groups rows [n_groups][2][bus_stride] at d_bus."""
         _check(self._L.ohs_mix_device(self._h, d_in, d_bus, n_frames, n_frames if row_stride is None else row_stride,
                                       n_frames if bus_stride is None else bus_stride))
 

@@ -174,6 +174,19 @@ def pcm_encode_dithered(y, fmt: int, seed: int, position: int, shape=(), state=N
     return q.astype(np.int16 if fmt == 1 else np.int32).reshape(y.shape), e
 
 
+def mix_groups(y, first) -> np.ndarray:
+    """The group buses of include/ohs.h (ohs_set_groups): y[S, 2, n] float32 rendered streams, group g = streams
+    first[g] .. first[g+1]-1.  Returns float32 [G, 2, n]: each group's rows summed from +0 in ascending stream order, every
+    addition rounded to f32 (a sequential sum; np.sum adds pairwise)."""
+    y = np.asarray(y, dtype=np.float32)
+    first = [int(f) for f in first]
+    out = np.zeros((len(first) - 1,) + y.shape[1:], np.float32)
+    for g in range(len(first) - 1):
+        for s in range(first[g], first[g + 1]):
+            out[g] = out[g] + y[s]
+    return out
+
+
 # BASELINE.json configs -> engine parameters (SURVEY.md §8d table)
 CONFIGS = {
     1: dict(name="cfg1: 1 stereo stream, 48 kHz, SOFA 200-tap HRIR, block 512", n_streams=1, fs=48000.0, block=512, taps=200),
