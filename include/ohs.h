@@ -27,7 +27,7 @@
  *   - the environment is read once, in ohs_create: OHS_STREAMS_PER_CTA (1..7, which render-kernel instantiation the
  *     handle uses; default: chosen from n_streams and the SM count), OHS_TIME_BATCH (0 = ohs_set_time_batch(h, 0)),
  *     OHS_STAGE_MB (staging chunk of the host-pointer path, default 24), OHS_PDL (0 = no programmatic dependent launches),
- *     OHS_TB_OVERLAP / OHS_TB_CHUNK / OHS_TB_EQ_G / OHS_TB_EQ_SMEM_KB (A/B switches of the time-batched route, INTEGRATION.md).
+ *     OHS_LATENCY_BLOCKS (launches of up to this many blocks run the render kernel's latency variant, default 2).
  */
 #ifndef OHS_H
 #define OHS_H

@@ -136,10 +136,6 @@ struct ohs_engine {
     cudaEvent_t ev_fwd[2] = {nullptr, nullptr};   // forward transforms have consumed a half of d_xf
     cudaEvent_t ev_call = nullptr;           // everything enqueued on the engine's stream before this call
     size_t eq_events_used = 0;
-    int tb_overlap = 1;      // OHS_TB_OVERLAP=0: EQ pre-pass on the engine's stream, one chunk per sub-launch (A/B)
-    int tb_eq_g = 0;         // OHS_TB_EQ_G: streams per CTA of the EQ pre-pass (A/B)
-    int tb_eq_smem_kb = -1;  // OHS_TB_EQ_SMEM_KB: dynamic shared memory its CTAs ask for at least (A/B; -1: by shape)
-    int tb_chunk = 0;        // OHS_TB_CHUNK=n: uniform chunks of n blocks instead of the ramped schedule (A/B)
 
     // FIFO adaptor (src/dsp/convolution.rs:141-182)
     std::vector<float> fifo_in, fifo_out;  // [row][cap]
@@ -165,15 +161,7 @@ int launch_render(ohs_engine* h, const RenderParams& p, int first_stream = 0, bo
     RenderLaunch L{h->G, h->cfg.device, h->stream, first_stream, latency ? 1 : 0, 0, h->dependent_launch, moving};
     RenderParams q = p;
     q.trace = h->d_trace;
-    cudaError_t e = cudaErrorInvalidValue;
-    switch (h->N) {
-        case 128: e = render_launch_128(L, q); break;
-        case 256: e = render_launch_256(L, q); break;
-        case 512: e = render_launch_512(L, q); break;
-        case 1024: e = render_launch_1024(L, q); break;
-        case 2048: e = render_launch_2048(L, q); break;
-        default: return fail(OHS_ERR_INVALID, "unsupported block size %d", h->B);
-    }
+    const cudaError_t e = with_transform_size(h->N, cudaErrorInvalidValue, [&](auto n) { return render_launch<n>(L, q); });
     if (e == cudaErrorInvalidConfiguration) { cudaGetLastError(); return fail(OHS_ERR_INVALID, "%d streams per CTA do not fit for block %d", h->G, h->B); }
     if (e != cudaSuccess) return fail(OHS_ERR_CUDA, "render kernel launch failed: %s", cudaGetErrorString(e));
     OHS_CUDA(cudaGetLastError());
@@ -181,46 +169,17 @@ int launch_render(ohs_engine* h, const RenderParams& p, int first_stream = 0, bo
     return OHS_OK;
 }
 
-bool render_fits(int N, int G) {
-    switch (N) {
-        case 128: return render_fits_128(G); case 256: return render_fits_256(G); case 512: return render_fits_512(G);
-        case 1024: return render_fits_1024(G); case 2048: return render_fits_2048(G);
-    }
-    return false;
-}
-
-// per-device "attribute already set" flags of the small kernels; handles on different threads may race here, hence
-// atomic (setting an attribute twice is harmless)
-struct AttrOnce {
-    std::atomic<unsigned char> done[64];
-    bool need(int dev) const { return dev >= 0 && dev < 64 && !done[dev].load(std::memory_order_acquire); }
-    void mark(int dev) { done[dev].store(1, std::memory_order_release); }
-};
-
 template <int N> int launch_setup_n(ohs_engine* h, int max_parts, int n_sets) {
     using SM = SetupSmem<N>;
-    static AttrOnce once;
-    const int dev = h->cfg.device;
-    if (once.need(dev)) {
-        OHS_CUDA(cudaFuncSetAttribute(setup_filters_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::kBytes));
-        once.mark(dev);
-    }
+    static OncePerDevice attrs;
+    OHS_CUDA(attrs.run(h->cfg.device, [] {
+        return cudaFuncSetAttribute(setup_filters_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::kBytes);
+    }));
     dim3 grid(max_parts, n_sets);
     setup_filters_kernel<N><<<grid, SM::T, SM::kBytes, h->stream>>>(h->d_ir, h->d_filt, h->d_tw, h->d_set_list, h->d_set_parts, h->pmax);
     OHS_CUDA(cudaGetLastError());
     h->launches++;
     return OHS_OK;
-}
-
-int launch_setup(ohs_engine* h, int max_parts, int n_sets) {
-    switch (h->N) {
-        case 128: return launch_setup_n<128>(h, max_parts, n_sets);
-        case 256: return launch_setup_n<256>(h, max_parts, n_sets);
-        case 512: return launch_setup_n<512>(h, max_parts, n_sets);
-        case 1024: return launch_setup_n<1024>(h, max_parts, n_sets);
-        case 2048: return launch_setup_n<2048>(h, max_parts, n_sets);
-    }
-    return fail(OHS_ERR_INVALID, "unsupported block size %d", h->B);
 }
 
 // the delay-line ring brought up to date from the time-ordered buffer (after time-batched calls), before anything reads
@@ -298,7 +257,7 @@ int commit_filters(ohs_engine* h) {
     OHS_CUDA(cudaMemcpyAsync(h->d_set_list, list.data(), sizeof(int) * list.size(), cudaMemcpyHostToDevice, h->stream));
     OHS_CUDA(cudaMemcpyAsync(h->d_set_flags, h->set_dirty.data(), n_sets, cudaMemcpyHostToDevice, h->stream));
     OHS_CUDA(cudaStreamSynchronize(h->stream));  // pageable sources (`list` is a local) must be consumed before returning
-    rc = launch_setup(h, max_parts, (int)list.size());
+    rc = with_transform_size(h->N, (int)OHS_ERR_INVALID, [&](auto n) { return launch_setup_n<n>(h, max_parts, (int)list.size()); });
     if (rc) return rc;
     // set_ir clears the history of the streams that use the set (src/dsp/convolution.rs:135-138)
     rc = clear_history(h, true);
@@ -500,9 +459,10 @@ int ensure_pcm_scratch(ohs_engine* h, size_t frames) {
 
 // called once, from ohs_create (the only place the environment is consulted)
 int pick_streams_per_cta(const ohs_engine* h) {
+    auto fits = [h](int g) { return with_transform_size(h->N, false, [g](auto n) { return render_fits<n>(g); }); };
     if (const char* e = getenv("OHS_STREAMS_PER_CTA")) {
         const int g = atoi(e);
-        if (g >= 1 && g <= kMaxG && render_fits(h->N, g)) return g;
+        if (g >= 1 && g <= kMaxG && fits(g)) return g;
     }
     cudaDeviceProp prop{};
     int sms = 148;
@@ -512,7 +472,7 @@ int pick_streams_per_cta(const ohs_engine* h) {
     // six chains exactly fill one EQ warp, several CTAs resident per SM (measured best on config 3).
     int g = (h->cfg.n_streams + sms - 1) / sms;
     g = (g > kMaxG) ? 3 : std::max(1, g);
-    while (g > 1 && !render_fits(h->N, g)) --g;
+    while (g > 1 && !fits(g)) --g;
     return g;
 }
 
@@ -525,12 +485,9 @@ constexpr int kTimeBatch = 8;  // consecutive blocks a bin_conv_kernel thread ac
 
 template <int N> int launch_inverse(ohs_engine* h, const float2* d_w, float* d_out, int K, size_t row_stride) {
     constexpr size_t smem = sizeof(float2) * 2 * padded_len(N);
-    static AttrOnce once;
-    const int dev = h->cfg.device;
-    if (smem > 48 * 1024 && once.need(dev)) {
-        OHS_CUDA(cudaFuncSetAttribute(inverse_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        once.mark(dev);
-    }
+    static OncePerDevice attrs;
+    if (smem > 48 * 1024)
+        OHS_CUDA(attrs.run(h->cfg.device, [] { return cudaFuncSetAttribute(inverse_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); }));
     inverse_kernel<N><<<dim3(K, h->cfg.n_streams), SetupSmem<N>::TX, smem, h->stream>>>(d_w, d_out, h->d_tw, h->d_stream_gain, K,
                                                                                       (long long)row_stride);
     OHS_CUDA(cudaGetLastError());
@@ -542,12 +499,9 @@ template <int N> int launch_inverse(ohs_engine* h, const float2* d_w, float* d_o
 template <int N> int launch_forward(ohs_engine* h, const float* xf, long long xf_stride, int t0, int k, long long zstride, int zbase) {
     // zbase: the time-ordered buffer's slot of the sub-launch's block 0
     constexpr size_t smem = sizeof(float2) * 2 * padded_len(N);
-    static AttrOnce once;
-    const int dev = h->cfg.device;
-    if (smem > 48 * 1024 && once.need(dev)) {
-        OHS_CUDA(cudaFuncSetAttribute(forward_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        once.mark(dev);
-    }
+    static OncePerDevice attrs;
+    if (smem > 48 * 1024)
+        OHS_CUDA(attrs.run(h->cfg.device, [] { return cudaFuncSetAttribute(forward_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); }));
     forward_kernel<N><<<dim3(k, h->cfg.n_streams), SetupSmem<N>::TX, smem, h->stream>>>(
         xf, xf_stride, t0, reinterpret_cast<const float*>(h->d_prev), h->d_zlin, zstride, zbase, h->zl_cap, h->d_tw);
     OHS_CUDA(cudaGetLastError());
@@ -567,21 +521,26 @@ template <int N> int launch_forward(ohs_engine* h, const float* xf, long long xf
 //   (4) the inverse transforms.
 // The delay-line ring, the overlap-save block and the EQ state end up exactly where the block-by-block path leaves
 // them, so the two can be mixed freely between calls.
-// whether a call of n_blocks takes the time-batched route
-bool time_batch_eligible(const ohs_engine* h, int n_blocks) {
-    return h->time_batch && h->conv_enable && h->pmax >= 8 && n_blocks >= kTimeBatch && h->cfg.n_streams <= 65535;  // (grid.y = stream)
-}
 
-// Scratch of the time-batched route for calls of n_blocks (ohs_prepare calls this ahead of time so that no allocation
-// happens inside a timed call).  1: does not fit the 2 GiB budget (the caller stays on the block-by-block kernel).
-int ensure_time_batch_scratch(ohs_engine* h, int n_blocks) {
+// Blocks per sub-launch a call of n_blocks needs on the time-batched route: as many as the 2 GiB budget holds, at most
+// 64 and at most n_blocks.  0: the call runs the block-by-block kernel (the route is off or does not apply, or fewer
+// than kTimeBatch blocks fit the budget).  Decided before anything is enqueued.
+size_t time_batch_blocks(const ohs_engine* h, int n_blocks) {
+    if (!h->time_batch || !h->conv_enable || h->pmax < 8 || n_blocks < kTimeBatch || h->cfg.n_streams > 65535)   // (grid.y = stream)
+        return 0;
     const size_t S = (size_t)h->cfg.n_streams, N = (size_t)h->N, hist = (size_t)h->pmax - 1;
     const size_t budget = (size_t)2 << 30;
     // per block: a spectrum and a product (8N bytes each) and the filtered rows in both halves of d_xf (2 * 2 * 4B = 8N)
     const size_t per_block = 3 * S * N * sizeof(float2), fixed = S * hist * N * sizeof(float2);
     size_t kc = fixed < budget ? (budget - fixed) / per_block : 0;
     kc = std::min<size_t>(std::min<size_t>(kc, 64), (size_t)n_blocks);
-    if (kc < (size_t)kTimeBatch) return 1;
+    return kc < (size_t)kTimeBatch ? 0 : kc;
+}
+
+// Scratch of the time-batched route for sub-launches of kc = time_batch_blocks(...) blocks, grow-only (ohs_prepare
+// calls this ahead of time so that no allocation happens inside a timed call)
+int ensure_time_batch_scratch(ohs_engine* h, size_t kc) {
+    const size_t S = (size_t)h->cfg.n_streams, N = (size_t)h->N, hist = (size_t)h->pmax - 1;
     if (kc > h->zlin_blocks) {
         { const int rc = ensure_ring(h); if (rc) return rc; }   // the history moves to the ring before its buffer goes
         h->zlin_valid = false;
@@ -614,12 +573,10 @@ int launch_bin_conv(ohs_engine* h, int zslot0, float2* w, int k, long long zstri
     const size_t S = (size_t)h->cfg.n_streams, N = (size_t)h->N;
     const dim3 blk(128);
     const unsigned gx = (unsigned)((N / 2 + 31) / 32), gz = (unsigned)((S + 3) / 4);
-    static AttrOnce once;
-    const int dev = h->cfg.device;
-    if (once.need(dev)) {
-        OHS_CUDA(cudaFuncSetAttribute(bin_conv_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * 16 * 128 * sizeof(float4))));
-        once.mark(dev);
-    }
+    static OncePerDevice attrs;
+    OHS_CUDA(attrs.run(h->cfg.device, [] {
+        return cudaFuncSetAttribute(bin_conv_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * 16 * 128 * sizeof(float4)));
+    }));
     // 16 blocks per thread (half the spectrum and filter traffic per FMA) from 16 blocks per launch on: measured faster
     // than 8 at K = 16 (0.529 vs 0.560 ms), 32, 64 and 128 on config 5
     if (k >= 16)
@@ -633,9 +590,9 @@ int launch_bin_conv(ohs_engine* h, int zslot0, float2* w, int k, long long zstri
     return OHS_OK;
 }
 
-// EQ pre-pass of `frames` frames of every stream on `stream`: rows in (stride in_stride) -> rows out (stride out_stride)
+// EQ pre-pass of `frames` frames of every stream on the EQ stream: rows in (stride in_stride) -> rows out (stride out_stride)
 int launch_eq_prepass(ohs_engine* h, const RenderParams& base, const float* d_in, long long in_stride, float* d_out, long long out_stride,
-                      size_t frames, cudaStream_t stream) {
+                      size_t frames) {
     constexpr int kB = 256;   // the EQ-only variant exists for N = 512; the chain does not care how its rows are cut into blocks
     RenderParams q = base;
     q.in = d_in; q.out = d_out; q.row_stride = in_stride; q.out_row_stride = out_stride;
@@ -648,48 +605,39 @@ int launch_eq_prepass(ohs_engine* h, const RenderParams& base, const float* d_in
     // the per-bin kernel's FMA-saturated warps every instruction of the biquad chain waits for its issue slot and the
     // chain, the route's critical path, runs 2.5x slower (measured; config 5 at 256 blocks per call: 4.95 ms with 43 SMs
     // owned, 5.65 ms with thin CTAs of three streams sharing 86 SMs, 5.82 ms with twelve streams = two EQ warps per
-    // partition on 22 SMs).  Few streams or one stream of work: thin CTAs of three.
-    const bool own_sm = stream != h->stream && h->cfg.n_streams >= 12;
-    const int g = (h->tb_eq_g > 0) ? h->tb_eq_g : (own_sm ? 6 : 3);
-    const size_t min_smem = (h->tb_eq_smem_kb >= 0) ? (size_t)h->tb_eq_smem_kb << 10 : (own_sm ? (size_t)200 << 10 : 0);
+    // partition on 22 SMs).  Fewer than twelve streams: thin CTAs of three.
+    const bool own_sm = h->cfg.n_streams >= 12;
     // no programmatic dependent launch here: the next chunk's CTAs, started early, would sit on SMs of their own (they
     // cannot share one with this chunk's) and take them from the transforms of the chunk before
-    RenderLaunch L{g, h->cfg.device, stream, 0, 2, min_smem, false};
-    const cudaError_t e = render_launch_512(L, q);
+    RenderLaunch L{own_sm ? 6 : 3, h->cfg.device, h->eq_stream, 0, 2, own_sm ? (size_t)200 << 10 : 0, false};
+    const cudaError_t e = render_launch<512>(L, q);
     if (e != cudaSuccess) return fail(OHS_ERR_CUDA, "EQ pre-pass launch failed: %s", cudaGetErrorString(e));
     h->launches++;
     return OHS_OK;
 }
 
-int process_time_batched(ohs_engine* h, RenderParams p, const float* d_in, float* d_out, size_t row_stride) {
+// the time-batched route for a call that needs sub-launches of `fit` = time_batch_blocks(h, p.n_blocks) blocks
+int process_time_batched(ohs_engine* h, RenderParams p, size_t fit, const float* d_in, float* d_out, size_t row_stride) {
     const size_t S = (size_t)h->cfg.n_streams, N = (size_t)h->N, hist = (size_t)h->pmax - 1, B = (size_t)h->B;
-    {
-        const int rc = ensure_time_batch_scratch(h, p.n_blocks);
-        if (rc) return rc;   // 1: caller falls back to the block-by-block kernel
-    }
+    { const int rc = ensure_time_batch_scratch(h, fit); if (rc) return rc; }
+    // sub-launches as long as the scratch allows: after a longer call, more than this call's own fit
     const size_t kc = h->zlin_blocks;
     const long long zstride = (long long)((hist + kc) * N);
     const long long xstride = (long long)(kc * B);               // frames between the rows of a half of d_xf
     const size_t xhalf = S * 2 * kc * B;                         // floats per half
     const int total = p.n_blocks;
     const bool eq_on = p.eq_enable != 0;
-    const bool overlap = eq_on && h->tb_overlap;
-    cudaStream_t eqs = overlap ? h->eq_stream : h->stream;
     const int n_sub = (total + (int)kc - 1) / (int)kc;
     // chunks of sub-launch j: (first block inside the sub-launch, blocks).  The EQ pre-pass of a chunk runs beside the
     // transforms of the chunk before it, so what a call cannot hide is the pre-pass of its first chunk and the transforms of
     // its last: the first sub-launch ramps up (16, 16, 32), the last one ramps down (32, 16, 16), everything between goes
     // in the largest pieces.  (Chunks of 8 were measured and lose: the per-bin kernel's 8-block form takes 128 us per
     // chunk against 187 us for 16 blocks; config 5 at 64 blocks per call: 1.39 ms with 16-16-16-16, 1.50 ms with
-    // 8-8-16-16-8-8, 1.61 ms un-overlapped.)
+    // 8-8-16-16-8-8, 1.61 ms un-overlapped.)  With the EQ off there is nothing to overlap: one chunk per sub-launch.
     auto chunks_of = [&](int j, std::vector<std::pair<int, int>>& out) {
         out.clear();
         const int k = std::min<int>((int)kc, total - j * (int)kc);
-        if (!overlap) { out.emplace_back(0, k); return; }
-        if (h->tb_chunk > 0) {
-            for (int at = 0; at < k; at += h->tb_chunk) out.emplace_back(at, std::min(h->tb_chunk, k - at));
-            return;
-        }
+        if (!eq_on) { out.emplace_back(0, k); return; }
         std::vector<int> head, tail;
         int rest = k;
         if (j == 0) for (int c : {16, 16, 32}) if (rest >= 2 * c) { head.push_back(c); rest -= c; }
@@ -699,17 +647,6 @@ int process_time_batched(ohs_engine* h, RenderParams p, const float* d_in, float
         if (rest > 0) { out.emplace_back(at, rest); at += rest; }
         for (size_t i = tail.size(); i-- > 0;) { out.emplace_back(at, tail[i]); at += tail[i]; }
     };
-#ifdef OHS_TB_TRACE   // debug builds only: a timing event behind every kernel of the route, printed as a timeline per call
-    struct Mark { cudaEvent_t ev; const char* what; int a, b; };
-    std::vector<Mark> marks;
-    auto mark = [&](cudaStream_t st, const char* what, int a, int b) {
-        cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); marks.push_back({e, what, a, b});
-    };
-#define OHS_TB_MARK(st, what, a, b) mark(st, what, a, b)
-#else
-#define OHS_TB_MARK(st, what, a, b) do { } while (0)
-#endif
-    OHS_TB_MARK(h->stream, "call", 0, 0);
     std::vector<std::vector<std::pair<int, int>>> chunks(n_sub);
     std::vector<std::vector<cudaEvent_t>> done_ev(n_sub);
     for (int j = 0; j < n_sub; ++j) chunks_of(j, chunks[j]);
@@ -725,33 +662,28 @@ int process_time_batched(ohs_engine* h, RenderParams p, const float* d_in, float
     h->eq_events_used = 0;
     // enqueue the EQ pre-pass of sub-launch j (its chunks back to back on the EQ stream, an event behind each)
     auto enqueue_eq = [&](int j) -> int {
-        if (!eq_on) return OHS_OK;
         float* xf = h->d_xf + (size_t)(j & 1) * xhalf;
-        if (overlap && j >= 2) OHS_CUDA(cudaStreamWaitEvent(eqs, h->ev_fwd[j & 1], 0));   // sub-launch j-2's transforms have read this half
+        if (j >= 2) OHS_CUDA(cudaStreamWaitEvent(h->eq_stream, h->ev_fwd[j & 1], 0));   // sub-launch j-2's transforms have read this half
         for (const auto& c : chunks[j]) {
             const size_t f0 = ((size_t)j * kc + c.first) * B;
-            int rc = launch_eq_prepass(h, p, d_in + f0, (long long)row_stride, xf + (size_t)c.first * B, xstride, (size_t)c.second * B, eqs);
+            int rc = launch_eq_prepass(h, p, d_in + f0, (long long)row_stride, xf + (size_t)c.first * B, xstride, (size_t)c.second * B);
             if (rc) return rc;
-            OHS_TB_MARK(eqs, "eq", j, c.first);
-            if (overlap) {
-                cudaEvent_t ev;
-                rc = next_event(&ev);
-                if (rc) return rc;
-                OHS_CUDA(cudaEventRecord(ev, eqs));
-                done_ev[j].push_back(ev);
-            }
+            cudaEvent_t ev;
+            rc = next_event(&ev);
+            if (rc) return rc;
+            OHS_CUDA(cudaEventRecord(ev, h->eq_stream));
+            done_ev[j].push_back(ev);
         }
         return OHS_OK;
     };
-    if (overlap) {
+    if (eq_on) {
         // the EQ stream starts behind everything already enqueued on the engine's stream (EQ state, input rows)
         OHS_CUDA(cudaEventRecord(h->ev_call, h->stream));
-        OHS_CUDA(cudaStreamWaitEvent(eqs, h->ev_call, 0));
+        OHS_CUDA(cudaStreamWaitEvent(h->eq_stream, h->ev_call, 0));
         for (int j = 0; j < std::min(2, n_sub); ++j) { const int rc = enqueue_eq(j); if (rc) return rc; }
     }
     for (int j = 0; j < n_sub; ++j) {
         const int k = std::min<int>((int)kc, total - j * (int)kc);
-        if (!overlap) { const int rc = enqueue_eq(j); if (rc) return rc; }
         if (!h->zlin_valid) {
             // the route changes here (first call, or block-by-block calls since the last time-batched one): the ring's
             // history goes behind the next block's slot; between time-batched sub-launches and calls nothing is copied
@@ -760,51 +692,30 @@ int process_time_batched(ohs_engine* h, RenderParams p, const float* d_in, float
             OHS_CUDA(cudaGetLastError());
             h->launches++;
             h->zlin_valid = true;
-            OHS_TB_MARK(h->stream, "gather", j, 0);
         }
         const int zb = h->zl_base;   // slot of this sub-launch's block 0
         // filtered rows of this sub-launch: a half of d_xf (with the EQ off, a copy of the input rows: the transforms read
         // a block's predecessor too, which an in-place call has overwritten with output by then)
-        const float* xf = h->d_xf + (size_t)(j & 1) * xhalf;
-        const long long xs = xstride;
+        float* xf = h->d_xf + (size_t)(j & 1) * xhalf;
         if (!eq_on)
-            OHS_CUDA(cudaMemcpy2DAsync(h->d_xf + (size_t)(j & 1) * xhalf, (size_t)xstride * sizeof(float), d_in + (size_t)j * kc * B,
-                                       row_stride * sizeof(float), (size_t)k * B * sizeof(float), S * 2, cudaMemcpyDeviceToDevice, h->stream));
+            OHS_CUDA(cudaMemcpy2DAsync(xf, (size_t)xstride * sizeof(float), d_in + (size_t)j * kc * B, row_stride * sizeof(float),
+                                       (size_t)k * B * sizeof(float), S * 2, cudaMemcpyDeviceToDevice, h->stream));
         float* out_j = d_out + (size_t)j * kc * B;
         for (size_t ci = 0; ci < chunks[j].size(); ++ci) {
             const int c0 = chunks[j][ci].first, ck = chunks[j][ci].second;
-            if (overlap) OHS_CUDA(cudaStreamWaitEvent(h->stream, done_ev[j][ci], 0));
-            int rc;
-            switch (h->N) {
-                case 128: rc = launch_forward<128>(h, xf, xs, c0, ck, zstride, zb); break;
-                case 256: rc = launch_forward<256>(h, xf, xs, c0, ck, zstride, zb); break;
-                case 512: rc = launch_forward<512>(h, xf, xs, c0, ck, zstride, zb); break;
-                case 1024: rc = launch_forward<1024>(h, xf, xs, c0, ck, zstride, zb); break;
-                case 2048: rc = launch_forward<2048>(h, xf, xs, c0, ck, zstride, zb); break;
-                default: rc = fail(OHS_ERR_INVALID, "unsupported transform size %d", h->N);
-            }
-            if (rc) return rc;
-            OHS_TB_MARK(h->stream, "forward", j, c0);
+            if (eq_on) OHS_CUDA(cudaStreamWaitEvent(h->stream, done_ev[j][ci], 0));
             float2* w = h->d_wlin + S * (size_t)c0 * N;
-            rc = launch_bin_conv(h, (zb + c0) % h->zl_cap, w, ck, zstride);
+            const int rc = with_transform_size(h->N, (int)OHS_ERR_INVALID, [&](auto n) {
+                int r = launch_forward<n>(h, xf, xstride, c0, ck, zstride, zb);
+                if (!r) r = launch_bin_conv(h, (zb + c0) % h->zl_cap, w, ck, zstride);
+                return r ? r : launch_inverse<n>(h, w, out_j + (size_t)c0 * B, ck, row_stride);
+            });
             if (rc) return rc;
-            OHS_TB_MARK(h->stream, "bin_conv", j, c0);
-            float* out_c = out_j + (size_t)c0 * B;
-            switch (h->N) {
-                case 128: rc = launch_inverse<128>(h, w, out_c, ck, row_stride); break;
-                case 256: rc = launch_inverse<256>(h, w, out_c, ck, row_stride); break;
-                case 512: rc = launch_inverse<512>(h, w, out_c, ck, row_stride); break;
-                case 1024: rc = launch_inverse<1024>(h, w, out_c, ck, row_stride); break;
-                case 2048: rc = launch_inverse<2048>(h, w, out_c, ck, row_stride); break;
-                default: rc = fail(OHS_ERR_INVALID, "unsupported transform size %d", h->N);
-            }
-            if (rc) return rc;
-            OHS_TB_MARK(h->stream, "inverse", j, c0);
         }
         // overlap-save history of the next sub-launch or call: this one's last filtered block
-        OHS_CUDA(cudaMemcpy2DAsync(h->d_prev, B * sizeof(float), xf + (size_t)(k - 1) * B, (size_t)xs * sizeof(float), B * sizeof(float),
+        OHS_CUDA(cudaMemcpy2DAsync(h->d_prev, B * sizeof(float), xf + (size_t)(k - 1) * B, (size_t)xstride * sizeof(float), B * sizeof(float),
                                    S * 2, cudaMemcpyDeviceToDevice, h->stream));
-        if (overlap) {
+        if (eq_on) {
             OHS_CUDA(cudaEventRecord(h->ev_fwd[j & 1], h->stream));
             if (j + 2 < n_sub) { const int rc = enqueue_eq(j + 2); if (rc) return rc; }
         }
@@ -812,16 +723,6 @@ int process_time_batched(ohs_engine* h, RenderParams p, const float* d_in, float
         h->zl_base = (zb + k) % h->zl_cap;
         h->ring_valid = false;   // the spectra of these blocks exist in the time-ordered buffer only (ensure_ring)
     }
-#ifdef OHS_TB_TRACE
-    cudaStreamSynchronize(h->stream);
-    if (h->eq_stream) cudaStreamSynchronize(h->eq_stream);
-    for (const Mark& m : marks) {
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, marks[0].ev, m.ev);
-        fprintf(stderr, "tb_trace %-8s sub %d block %2d done at %8.1f us\n", m.what, m.a, m.b, ms * 1e3);
-    }
-    for (const Mark& m : marks) cudaEventDestroy(m.ev);
-#endif
     return OHS_OK;
 }
 
@@ -861,10 +762,6 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     h->pmax = (cfg->max_taps + B - 1) / B;
     h->G = pick_streams_per_cta(h);
     if (const char* e = getenv("OHS_TIME_BATCH")) h->time_batch = atoi(e) != 0;
-    if (const char* e = getenv("OHS_TB_OVERLAP")) h->tb_overlap = atoi(e) != 0;
-    if (const char* e = getenv("OHS_TB_EQ_G")) { const int g = atoi(e); if (g == 3 || g == 6) h->tb_eq_g = g; }
-    if (const char* e = getenv("OHS_TB_EQ_SMEM_KB")) { const int k = atoi(e); if (k >= 0 && k <= 227) h->tb_eq_smem_kb = k; }
-    if (const char* e = getenv("OHS_TB_CHUNK")) { const int c = atoi(e); if (c >= 1 && c <= 64) h->tb_chunk = c; }
     if (const char* e = getenv("OHS_STAGE_MB")) { const long mb = atol(e); if (mb >= 1 && mb <= 4096) h->stage_bytes = (size_t)mb << 20; }
     if (const char* e = getenv("OHS_PDL")) h->dependent_launch = atoi(e) != 0;
     if (const char* e = getenv("OHS_LATENCY_BLOCKS")) h->latency_blocks = atoi(e);
@@ -935,13 +832,7 @@ int ohs_create(const ohs_config* cfg, ohs_engine** out) {
     OHS_TRY(cudaMemsetAsync(h->d_ir, 0, sizeof(float) * (size_t)cfg->n_hrir_sets * 4 * per_path, h->stream));
     {
         std::vector<float2> tw(h->N);
-        switch (h->N) {
-            case 128: fill_twiddles<128>(tw.data()); break;
-            case 256: fill_twiddles<256>(tw.data()); break;
-            case 512: fill_twiddles<512>(tw.data()); break;
-            case 1024: fill_twiddles<1024>(tw.data()); break;
-            case 2048: fill_twiddles<2048>(tw.data()); break;
-        }
+        with_transform_size(h->N, false, [&](auto n) { fill_twiddles<n>(tw.data()); return true; });
         OHS_TRY(cudaMemcpyAsync(h->d_tw, tw.data(), sizeof(float2) * h->N, cudaMemcpyHostToDevice, h->stream));
         OHS_TRY(cudaMemcpyAsync(h->d_set_parts, h->h_set_parts.data(), sizeof(int) * cfg->n_hrir_sets, cudaMemcpyHostToDevice, h->stream));
         OHS_TRY(cudaMemcpyAsync(h->d_group_first, h->h_group_first.data(), sizeof(int) * 2, cudaMemcpyHostToDevice, h->stream));
@@ -1199,11 +1090,8 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io) {
         rc = ensure_pcm_scratch(h, chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float)));   // ohs_process_device_pcm
         if (rc) return rc;
     }
-    const int n_blocks = (int)((per_launch + h->B - 1) / h->B);
-    if (time_batch_eligible(h, n_blocks)) {
-        rc = ensure_time_batch_scratch(h, n_blocks);
-        if (rc < 0) return rc;
-    }
+    const size_t tb = time_batch_blocks(h, (int)((per_launch + h->B - 1) / h->B));
+    if (tb && (rc = ensure_time_batch_scratch(h, tb))) return rc;
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     return OHS_OK;
 }
@@ -1303,13 +1191,11 @@ int process_device_impl(ohs_engine* h, const float* d_in, float* d_out, size_t n
     if (h->timing) OHS_CUDA(cudaEventRecord(h->ev_k0, h->stream));
     // long responses over many blocks: convolve along time per bin instead of re-reading the delay line every block
     // (one set per stream and call: a call with a transition runs the block-by-block kernel)
-    bool batched = !transition && time_batch_eligible(h, p.n_blocks);
-    if (batched) {
-        rc = process_time_batched(h, p, d_in, d_out, row_stride);
-        if (rc < 0) return rc;
-        batched = (rc == 0);
-    }
-    if (!batched) {
+    const size_t tb = transition ? 0 : time_batch_blocks(h, p.n_blocks);
+    if (tb) {
+        rc = process_time_batched(h, p, tb, d_in, d_out, row_stride);
+        if (rc) return rc;
+    } else {
         if (h->conv_enable) { rc = ensure_ring(h); if (rc) return rc; }   // the kernel reads and extends the delay-line ring
         const bool moving = transition || (h->conv_enable && needs_full_ring(h));
         if (moving && !p.from_set) p.from_set = h->d_stream_hrir;

@@ -588,13 +588,15 @@ def test_time_batched_long_response(block, taps, n_streams, n_blocks, monkeypatc
 
 
 @pytest.mark.parametrize("case", ["in_place", "eq_off", "disabled_band", "ragged_prepass", "own_sm"])
-def test_time_batched_pipeline_variants(case, monkeypatch):
+def test_time_batched_pipeline_variants(case):
     """The time-batched route's EQ pre-pass pipeline through ohs_process_device: several sub-launches and chunks per call
-    (150 blocks: 8+8+16+32, 64, 22), in place; the EQ off (the transforms read a copy of the input rows); a disabled band
-    (the pre-pass leaves its continuous chain); block 64 with a chunk that is not a whole number of the pre-pass's
-    256-frame rows; 14 streams, which select the pre-pass's production shape (render_kernel<512,6,2>: six streams per
-    CTA on an SM of its own, here two full CTAs and a partial one).  Each against the oracle, and the overlapped pipeline against the same kernels run on one stream
-    (OHS_TB_OVERLAP=0): bit-identical."""
+    (calls of 16 and 134 blocks, the second in sub-launches of 16+16+32, 64 and 6 blocks), in place; the EQ off (the
+    transforms read a copy of the input rows); a disabled band (the pre-pass leaves its continuous chain); block 64 with
+    a chunk that is not a whole number of the pre-pass's 256-frame rows; 14 streams, which select the pre-pass's
+    production shape (render_kernel<512,6,2>: six streams per CTA on an SM of its own, here two full CTAs and a partial
+    one).  Each against the oracle, and two fresh engines fed the same calls bit-identical: the pre-pass runs on a stream
+    of its own, and a missing wait between it and the engine's stream would let the transforms read rows it has not
+    written yet."""
     import torch
 
     block, taps, n_streams, n_blocks = {"in_place": (128, 1500, 5, 150), "eq_off": (128, 1100, 4, 70), "disabled_band": (256, 2100, 4, 30),
@@ -607,9 +609,8 @@ def test_time_batched_pipeline_variants(case, monkeypatch):
     if case == "disabled_band":
         enabled[4] = 0
     ref = oracle_render(x, block, h, None if case == "eq_off" else coeffs, None if case == "eq_off" else enabled, 0.7)
-    outs = {}
-    for overlap in ("1", "0"):
-        monkeypatch.setenv("OHS_TB_OVERLAP", overlap)
+    outs = []
+    for _ in range(2):
         e = ohs.Engine(n_streams, block, taps)
         e.set_hrir_set(h); e.set_gain(0.7)
         if case != "eq_off":
@@ -623,9 +624,9 @@ def test_time_batched_pipeline_variants(case, monkeypatch):
         e.process_device(buf.data_ptr(), dst.data_ptr(), cut, row_stride=n)
         e.process_device(buf.data_ptr() + 4 * cut, dst.data_ptr() + 4 * cut, n - cut, row_stride=n)
         e.sync()
-        outs[overlap] = dst.cpu().numpy()
-        assert float(np.max(np.abs(outs[overlap] - ref))) <= TOL, (case, overlap)
-    assert np.array_equal(outs["0"], outs["1"])
+        outs.append(dst.cpu().numpy())
+    assert float(np.max(np.abs(outs[0] - ref))) <= TOL, case
+    assert np.array_equal(outs[0], outs[1])
 
 
 def test_time_batched_history_stays_in_the_circular_buffer():

@@ -9,8 +9,8 @@ Routes, forced the way the other GPU tests force them:
       memory), single-partition sets (fused path) and multi-partition sets
   R2  latency render_kernel<512, G, 1>: calls of one and two blocks
   R3  EQ-only mode (convolution off) with a ragged last block
-  R4  the time-batched route (P >= 8, >= 8 blocks per call), its EQ pre-pass on CTAs of six streams that own their SM
-      (>= 12 streams), on thin CTAs of three, and without the overlapped pipeline
+  R4  the time-batched route (P >= 8, >= 8 blocks per call), its EQ pre-pass on its own stream, on CTAs of six streams
+      that own their SM (>= 12 streams) and on thin CTAs of three
   R5  render_kernel<N, G, V, true>, the moving-sources kernel, which a multi-set engine with a delay line runs when some
       stream is bound to a one-partition set
 Bindings derive from s % U and the inputs tile with period U, U prime to G, so that twin streams (same input, same
@@ -97,7 +97,6 @@ class Route:
     g: int = 0                    # OHS_STREAMS_PER_CTA (0: the engine picks)
     conv: bool = True
     host: bool = False            # ohs_process instead of ohs_process_device
-    env: tuple = ()
 
     @property
     def n(self):
@@ -107,7 +106,7 @@ class Route:
     def pre_g(self):
         """streams per CTA of the kernel that holds the EQ chains: the render kernel, or the time-batched pre-pass"""
         if min(self.parts) >= 8:
-            return 6 if self.n_streams >= 12 and ("OHS_TB_OVERLAP", "0") not in self.env else 3
+            return 6 if self.n_streams >= 12 else 3
         return self.g
 
 
@@ -130,7 +129,6 @@ ROUTES = {
     "r3_b1024_ragged": Route(1024, 15, 11, (1, 1, 1), (1500, 2 * 1024 + 29), g=2, conv=False),
     "r4_own_sm": Route(128, 16, 11, (8, 9, 11), (16 * 128, 12 * 128)),
     "r4_thin": Route(128, 8, 5, (8, 9, 11), (16 * 128, 12 * 128)),
-    "r4_no_overlap": Route(128, 16, 11, (8, 9, 11), (16 * 128, 12 * 128), env=(("OHS_TB_OVERLAP", "0"),)),
     "r5_moving": Route(256, 16, 11, (1, 3, 2), (3 * 256, 4 * 256), g=3),
 }
 CONV_ROUTES = [k for k, r in ROUTES.items() if r.conv]
@@ -141,8 +139,6 @@ ISOLATION_ROUTES = ["r1_g3_b256_p3_host", "r1_g2_b1024_p3", "r1_g2_b256_p1", "r2
 def configure(monkeypatch, route):
     if route.g:
         monkeypatch.setenv("OHS_STREAMS_PER_CTA", str(route.g))
-    for k, v in route.env:
-        monkeypatch.setenv(k, v)
 
 
 def make_engine(route, n_bands=10, eq=True, sets=None, bind=True):
