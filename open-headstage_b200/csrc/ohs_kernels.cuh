@@ -12,9 +12,9 @@
 //   * EQ warps: band-systolic in time.  Lane l*6 + c owns bands 2l and 2l+1 of chain c = (stream, channel); at step s
 //     band A filters sample s-4l with the input shuffled over from lane l-1 three steps earlier, band B filters sample
 //     s-4l-1 with band A's previous output.  Every band's recurrence stays strictly sequential in the reference's
-//     operation order with explicitly rounded, never-contracted scalar ops: bit-exact.  (Packed f32x2 was measured
-//     slower, and ptxas 12.9 contracts mul.f32x2+add.f32x2 into FFMA2 even under -fmad=false.)  The chain runs
-//     continuously across the blocks of a launch.
+//     operation order with explicitly rounded, never-contracted ops: bit-exact.  Where several CTAs share an SM the two
+//     bands of a lane run as one packed f32x2 chain (RenderSmem::kEqPacked).  The chain runs continuously across the
+//     blocks of a launch.
 //   * convolution warps, T = max(32, N/16) threads per stream (one warp at N = 512): left + i*right go through ONE
 //     complex N = 2B point Stockham FFT in shared memory (radix 8/4/2 in registers, two adjacent butterflies per thread
 //     so every shared-memory access is 128-bit), the frequency-domain delay line keeps that packed spectrum Z, and the
@@ -46,7 +46,9 @@ constexpr int kMaxBands = 10;
 // (profiles/r02_ab_placement.txt): weight 3 -> (1, 1, 1, 4) convolution warps next to the three EQ warps, 16 warp
 // slots, 128 registers per thread: 1.081 M stream-s/s; weight 4 -> (0, 1, 1, 5), 20 warp slots, 96 registers, 360
 // bytes of spills in the convolution warps: 1.003 M; weight 5: 0.920 M.  (ptxas 12.9 reports 128 registers and 224 B
-// of spill stores and loads for today's render_kernel<512, 7, 0>.)
+// of spill stores and loads for today's render_kernel<512, 7, 0>.)  Weight 1 -> (1, 1, 2, 3), 12 warp slots, 168
+// registers: 0.977 M, and 0.884 M with the packed EQ step (profiles/eq_packed_f32x2_ab.txt); weight 2 places config 2
+// like weight 3.
 #ifndef OHS_EQ_WEIGHT
 #define OHS_EQ_WEIGHT 3
 #endif
@@ -94,6 +96,10 @@ struct RenderParams {
     const int* from_set;
     const int* block_set;
     long long block_set_stride;
+    // operands of the EQ warps' packed biquad step (df2t_step2): kernel parameters, so that ptxas cannot fold them into
+    // a contraction of the separately rounded products and sums
+    float one = 1.f;
+    float neg_zero = -0.f;
 };
 
 #ifdef OHS_TRACE
@@ -393,6 +399,11 @@ template <int N, int G, int V = 0> struct RenderSmem {
 #else
     static constexpr int kEqBpl = (N >= 1024 || V == 2) ? 1 : 2;
 #endif
+    // Two bands per lane as one packed f32x2 chain (df2t_step2) where several CTAs share an SM (N <= 256: config 3),
+    // whose warps compete for issue slots: config 3 870 k against 823 k stream-s/s with the scalar pair of chains.
+    // Where one CTA owns the SM (N = 512) the scalar form is faster: its two independent chains per lane hide each
+    // other's latency (config 2 1.084 M against 0.988 M packed, K = 1 496 k against 480 k; DESIGN §4.5).
+    static constexpr bool kEqPacked = kEqBpl == 2 && N < 512;
     // lane skew of the systolic chain in steps (= steps per unrolled iteration).  One band per lane runs a step in half
     // the time, too fast for a 3-step shuffle flight: skew 8
     static constexpr int kEqSkewSteps = (B >= 128) ? (kEqBpl == 1 ? 8 : kEqSkew) : 4;
@@ -492,14 +503,43 @@ template <int N, int G, int V = 0> struct RenderSmem {
 // One DF2T step, reference operation order (biquad 0.4.2 DirectForm2Transposed::run behind
 // src/dsp/parametric_eq.rs:116-122):   out = s1 + b0*x;  s1 = (s2 + b1*x) - a1*out;  s2 = b2*x - a2*out
 // Explicit round-to-nearest intrinsics: every product and sum is rounded separately and is never contracted into an
-// FMA (Rust does not contract; the cascade's output moves by 3.8e-4 if it is).  Left and right are two independent
-// scalar chains in the same lane, which gives the in-order warp the instruction-level parallelism to cover the
-// 4-cycle FP32 latency.  (The packed f32x2 form has half the instructions but one chain; measured slower, and ptxas
-// 12.9 contracts mul.f32x2 + add.f32x2 into FFMA2 even under -fmad=false.)
+// FMA (Rust does not contract; the cascade's output moves by 3.8e-4 if it is).  With two bands per lane, bands A and
+// B are two independent scalar chains in the same lane, which gives the in-order warp the instruction-level
+// parallelism to cover the 4-cycle FP32 latency, or one packed chain (df2t_step2, RenderSmem::kEqPacked).
 __device__ __forceinline__ float df2t_step(float x, float& s1, float& s2, float b0, float b1, float b2, float a1, float a2) {
     const float out = __fadd_rn(s1, __fmul_rn(b0, x));
     s1 = __fsub_rn(__fadd_rn(s2, __fmul_rn(b1, x)), __fmul_rn(a1, out));
     s2 = __fsub_rn(__fmul_rn(b2, x), __fmul_rn(a2, out));
+    return out;
+}
+// the same step with the rounded input products b0*x, b1*x, b2*x given
+__device__ __forceinline__ float df2t_step_products(float p0, float p1, float p2, float& s1, float& s2, float a1, float a2) {
+    const float out = __fadd_rn(s1, p0);
+    s1 = __fsub_rn(__fadd_rn(s2, p1), __fmul_rn(a1, out));
+    s2 = __fsub_rn(p2, __fmul_rn(a2, out));
+    return out;
+}
+
+// Packed f32x2 pairs {band A, band B} (low word = A), one FFMA2 per op pair.
+typedef unsigned long long f32x2;
+__device__ __forceinline__ f32x2 pk2(float lo, float hi) { f32x2 d; asm("mov.b64 %0, {%1, %2};" : "=l"(d) : "f"(lo), "f"(hi)); return d; }
+__device__ __forceinline__ void unpk2(f32x2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
+__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) {
+    f32x2 d;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
+    return d;
+}
+// df2t_step on two bands at once, in the same operation order and with the same rounding: every product is
+// fma(b, x, -0) (= the rounded product, signed zeros included) and every sum fma(a, 1, c), with 1 and -0 run-time
+// values (RenderParams::one, ::neg_zero).  ptxas 12.9 contracts mul.rn.f32x2 + add.rn.f32x2 into one FFMA2 even under
+// -fmad=false, and would do the same to these if it saw the constants.  The subtractions add the product with the
+// negated a1, a2 (na1, na2): -(a1*out) rounds to exactly the negated rounded product.  Half the FP32 instructions of
+// two scalar steps for the same FP32-pipe time, but one dependent chain where the scalar form has two.
+__device__ __forceinline__ f32x2 df2t_step2(f32x2 x, f32x2& s1, f32x2& s2, f32x2 b0, f32x2 b1, f32x2 b2, f32x2 na1, f32x2 na2,
+                                            f32x2 one, f32x2 nz) {
+    const f32x2 out = fma2(fma2(b0, x, nz), one, s1);
+    s1 = fma2(fma2(fma2(b1, x, nz), one, s2), one, fma2(na1, out, nz));
+    s2 = fma2(fma2(b2, x, nz), one, fma2(na2, out, nz));
     return out;
 }
 
@@ -508,15 +548,17 @@ __device__ __forceinline__ float df2t_step(float x, float& s1, float& s2, float 
 //     step s:  band A filters sample s - 4l      (input: lane l-1's band-B output of step s-3, by SHFL; l = 0: the input row)
 //              band B filters sample s - 4l - 1  (input: this lane's band-A output of step s-1)
 // so the last band (l = 4, B) runs 17 samples behind the first.  A shuffled output is consumed three steps later, which
-// covers its latency (26 cycles alone, more while the convolution warps load the shared-memory pipe), and the two bands
-// of a lane are two independent dependent-chains that cover each other's 4-cycle FP32 latency.  Every band's
-// recurrence is the strictly sequential reference recurrence (see df2t_step): bit-exact.
+// covers its latency (26 cycles alone, more while the convolution warps load the shared-memory pipe).  The two bands
+// of a lane are two independent dependent-chains that cover each other's 4-cycle FP32 latency, or, where
+// RenderSmem::kEqPacked, one packed {A, B} chain (df2t_step2) whose band B takes the low word of the previous step's
+// output pair.  Every band's recurrence is the strictly sequential reference recurrence (see df2t_step): bit-exact.
 template <bool V> struct Flag { static constexpr bool value = V; };
 template <int N, int G, int V>
 __device__ __forceinline__ void eq_warp_main(const RenderParams& p, unsigned char* smem, int stream0, int w) {
     using SM = RenderSmem<N, G, V>;
     constexpr int B = SM::B;
     constexpr int BPL = SM::kEqBpl;                    // bands per lane
+    constexpr bool kPacked = SM::kEqPacked;            // the two bands as one f32x2 chain (df2t_step2)
     constexpr int LPC = kMaxBands / BPL;               // lanes per chain
     constexpr int CPW = SM::kEqCpw;                    // chains per warp
     // lane skew in steps = steps per unrolled iteration.  One band per lane runs a step in half the time, too fast for
@@ -570,6 +612,12 @@ __device__ __forceinline__ void eq_warp_main(const RenderParams& p, unsigned cha
         const float* st = reinterpret_cast<const float*>(p.eqs + (size_t)s * kMaxBands + band_b);
         bs1 = st[ch]; bs2 = st[2 + ch];
     }
+    // kPacked: coefficients and state as {A, B} pairs, a1 and a2 negated (df2t_step2)
+    const f32x2 one2 = pk2(p.one, p.one), nz2 = pk2(p.neg_zero, p.neg_zero);
+    const f32x2 b0p = pk2(ab0, bb0), b1p = pk2(ab1, bb1), b2p = pk2(ab2, bb2), na1p = pk2(-aa1, -ba1), na2p = pk2(-aa2, -ba2);
+    f32x2 s1p = pk2(as1, bs1), s2p = pk2(as2, bs2);
+    // scalar two-band lanes: band A's coefficients b0, b1, b2 in both words, for its products of two steps at once
+    const f32x2 ab0d = pk2(ab0, ab0), ab1d = pk2(ab1, ab1), ab2d = pk2(ab2, ab2);
     bar_sync(kBarInitEq, 32 + SM::kEqThreads);   // the staging warp has initialised the mbarriers
 
     OHS_STAMP_IF(threadIdx.x == 0, p, 2);
@@ -624,12 +672,28 @@ __device__ __forceinline__ void eq_warp_main(const RenderParams& p, unsigned cha
     // SelLater: the block's last iteration; the next block's rows may not have landed, the raw shuffled values stay in
     // xsel and seed_inputs() completes them after the stage wait.
     auto fast_iter = [&](auto sel, const In& in, const In& nx, int i0, float* dst) {
+        f32x2 pa0, pa1, pa2;   // scalar two-band lanes: band A's products b*x of steps u and u+1 (u even), low word = u
 #pragma unroll
         for (int u = 0; u < DL; ++u) {
             if constexpr (BPL == 2) {
-                const float xa = xsel[u];
-                const float y = df2t_step(ya_prev, bs1, bs2, bb0, bb1, bb2, ba1, ba2);   // band B on band A's previous output
-                ya_prev = df2t_step(xa, as1, as2, ab0, ab1, ab2, aa1, aa2);
+                // band A on xsel[u], band B on band A's previous output
+                float y;
+                if constexpr (kPacked) {
+                    unpk2(df2t_step2(pk2(xsel[u], ya_prev), s1p, s2p, b0p, b1p, b2p, na1p, na2p, one2, nz2), ya_prev, y);
+                } else {
+                    // Band A's inputs are chosen steps ahead and its products lie off its recurrence: they are formed
+                    // for two steps at once by FFMA2 against -0 (= the rounded products), one instruction for two
+                    // FMULs.  xsel[u + 1] is final here: it was written one to three steps ago.
+                    if (u % 2 == 0) {
+                        const f32x2 x2 = pk2(xsel[u], xsel[u + 1]);
+                        pa0 = fma2(ab0d, x2, nz2); pa1 = fma2(ab1d, x2, nz2); pa2 = fma2(ab2d, x2, nz2);
+                    }
+                    float q0, q1, q2, unused;
+                    if (u % 2 == 0) { unpk2(pa0, q0, unused); unpk2(pa1, q1, unused); unpk2(pa2, q2, unused); }
+                    else { unpk2(pa0, unused, q0); unpk2(pa1, unused, q1); unpk2(pa2, unused, q2); }
+                    y = df2t_step(ya_prev, bs1, bs2, bb0, bb1, bb2, ba1, ba2);
+                    ya_prev = df2t_step_products(q0, q1, q2, as1, as2, aa1, aa2);
+                }
                 const float r = __shfl_sync(0xffffffffu, y, src_lane);   // band A's input DL-1 steps from now
                 if (u == 0) xsel[DL - 1] = first ? in_at(in, DL - 1) : r;
                 else xsel[u - 1] = (decltype(sel)::value && first) ? in_at(nx, u - 1) : r;
@@ -662,16 +726,33 @@ __device__ __forceinline__ void eq_warp_main(const RenderParams& p, unsigned cha
             const bool act_a = lane_valid && na >= 0 && na < nb, act_b = lane_valid && nbi >= 0 && nbi < nb;
             const float xa = xsel[u];
             if constexpr (BPL == 2) {
-                float t1 = bs1, t2 = bs2;
-                float y = df2t_step(ya_prev, t1, t2, bb0, bb1, bb2, ba1, ba2);
-                const bool upd_b = act_b && en_b;
-                bs1 = upd_b ? t1 : bs1; bs2 = upd_b ? t2 : bs2;
-                y = upd_b ? y : ya_prev;
-                t1 = as1; t2 = as2;
-                float ya = df2t_step(xa, t1, t2, ab0, ab1, ab2, aa1, aa2);
-                const bool upd_a = act_a && en_a;
-                as1 = upd_a ? t1 : as1; as2 = upd_a ? t2 : as2;
-                ya_prev = upd_a ? ya : xa;
+                float y;
+                if constexpr (kPacked) {
+                    const bool upd_a = act_a && en_a, upd_b = act_b && en_b;
+                    f32x2 t1 = s1p, t2 = s2p;
+                    float ya;
+                    unpk2(df2t_step2(pk2(xa, ya_prev), t1, t2, b0p, b1p, b2p, na1p, na2p, one2, nz2), ya, y);
+                    // commit each half of the pair on its own band's condition
+                    auto commit = [&](f32x2& s, f32x2 t) {
+                        float sa, sb, ta, tb;
+                        unpk2(s, sa, sb); unpk2(t, ta, tb);
+                        s = pk2(upd_a ? ta : sa, upd_b ? tb : sb);
+                    };
+                    commit(s1p, t1); commit(s2p, t2);
+                    y = upd_b ? y : ya_prev;
+                    ya_prev = upd_a ? ya : xa;
+                } else {
+                    float t1 = bs1, t2 = bs2;
+                    y = df2t_step(ya_prev, t1, t2, bb0, bb1, bb2, ba1, ba2);
+                    const bool upd_b = act_b && en_b;
+                    bs1 = upd_b ? t1 : bs1; bs2 = upd_b ? t2 : bs2;
+                    y = upd_b ? y : ya_prev;
+                    t1 = as1; t2 = as2;
+                    float ya = df2t_step(xa, t1, t2, ab0, ab1, ab2, aa1, aa2);
+                    const bool upd_a = act_a && en_a;
+                    as1 = upd_a ? t1 : as1; as2 = upd_a ? t2 : as2;
+                    ya_prev = upd_a ? ya : xa;
+                }
                 const float r = __shfl_sync(0xffffffffu, y, src_lane);
                 if (u == 0) xsel[DL - 1] = first ? in_at(in, DL - 1) : r;
                 else xsel[u - 1] = first ? in_at(nx, u - 1) : r;
@@ -814,6 +895,7 @@ __device__ __forceinline__ void eq_warp_main(const RenderParams& p, unsigned cha
             bar_arrive(kBarFull0 + (t & 1), SM::kFullCount);
         }
     }
+    if constexpr (kPacked) { unpk2(s1p, as1, bs1); unpk2(s2p, as2, bs2); }
     if (has_a) { float* st = reinterpret_cast<float*>(p.eqs + (size_t)s * kMaxBands + band_a); st[ch] = as1; st[2 + ch] = as2; }
     if (has_b) { float* st = reinterpret_cast<float*>(p.eqs + (size_t)s * kMaxBands + band_b); st[ch] = bs1; st[2 + ch] = bs2; }
     OHS_STAMP_IF(threadIdx.x == 0, p, 8);
