@@ -230,8 +230,10 @@ int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void*
 
 /* ---- dither of integer PCM output (an extension) -----------------------------------------------------------------
  * TPDF dither, optionally with error-feedback noise shaping, for every encode to S16 or S24 by ohs_process_pcm and
- * ohs_process_device_pcm, bypassed F32 -> S16 or S24 -> S16 calls included.  F32 output is never dithered.  Exact to the
- * bit (numpy reference: signals.pcm_encode_dithered).  Row r = 2*stream + channel; b = 16 / 24; lo, hi = the clamp bounds.
+ * ohs_process_device_pcm, bypassed F32 -> S16 or S24 -> S16 calls included, and for the integer buses of
+ * ohs_process_grouped_pcm and ohs_mix_device_pcm (their rows numbered from 2 * n_streams on, below at ohs_set_groups).
+ * F32 output is never dithered.  Exact to the bit (numpy reference: signals.pcm_encode_dithered).  Row r =
+ * 2*stream + channel; b = 16 / 24; lo, hi = the clamp bounds.
  *   position  a 64-bit counter p: ohs_set_dither sets it to 0; every successful call with an integer OUTPUT format moves it
  *             on by n_frames (bypassed ones too); frame f of a call has position p0 + f.  So the noise does not depend on
  *             how a render is cut into calls or into the chunks of a call.
@@ -255,7 +257,8 @@ int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void*
 #define OHS_DITHER_TPDF 1      /* TPDF dither, noise-shaped when n_taps > 0 */
 #define OHS_MAX_SHAPE_TAPS 9
 /* Sets mode, seed and taps (shape[0..n_taps) = h_1..h_M, copied), resets the position to 0 and zeroes the history, on the
- * engine's stream (ordered after earlier calls).  Allocates the history (2 * n_streams * OHS_MAX_SHAPE_TAPS floats) for
+ * engine's stream (ordered after earlier calls).  Allocates the history (4 * n_streams * OHS_MAX_SHAPE_TAPS floats: stream
+ * rows, then the bus rows of ohs_set_groups) for
  * OHS_DITHER_TPDF; process calls never allocate for dither.  OHS_ERR_INVALID with the engine untouched: an unknown mode,
  * n_taps outside 0..OHS_MAX_SHAPE_TAPS, taps with OHS_DITHER_OFF, a null shape with n_taps > 0, a non-finite tap. */
 int ohs_set_dither(ohs_engine* h, int mode, uint64_t seed, const float* shape, int n_taps);
@@ -284,10 +287,17 @@ int ohs_last_kernel_ms(ohs_engine* h, float* ms);
  *   bus[g][c][n] = ((((+0) + y[f][c][n]) + y[f+1][c][n]) + y[f+2][c][n]) + ...
  * in ascending stream order, every addition rounded to f32 (numpy reference: signals.mix_groups).  Starting from +0
  * differs from starting with y[f] only where every term is -0: the bus is +0 there.
- * Not provided: integer bus output and dither of buses (dither history rows are defined per stream row; sharing them
- * with bus rows needs a definition of its own), grouped forms of ohs_process_fifo and ohs_process_device_scheduled (on
- * the device, compose ohs_process_device_scheduled with ohs_mix_device), non-contiguous groups, and a mix fused into the
- * render kernel (DESIGN §13). */
+ * Integer buses (ohs_process_grouped_pcm, ohs_mix_device_pcm): bus row 2*g + c is encoded exactly as ohs_process_pcm
+ * encodes a stream row, from the f32 bus above, and dithered as ohs_set_dither says with these rules of its own:
+ *   row number  bus row 2*g + c has dither row number 2*n_streams + 2*g + c, so K = mix64(seed + phi * (2S + 2g + c + 1)):
+ *               its noise never repeats a stream row's (the same keys as stream rows 2g + c under the seed seed + phi * 2S)
+ *   position    the engine's one position p: every successful call with an integer bus format moves it on by n_frames
+ *               (bypassed ones too), frame f of the call at p0 + f; calls with an F32 bus leave it alone
+ *   history     every bus row has its own e_1..e_M, zeroed by ohs_set_dither and by ohs_set_groups (on the engine's stream,
+ *               ordered like the offsets), carried by the state blob (flags bit 1)
+ * Not provided: grouped forms of ohs_process_fifo and ohs_process_device_scheduled (on the device, compose
+ * ohs_process_device_scheduled with ohs_mix_device or ohs_mix_device_pcm), non-contiguous groups, and a mix fused into the
+ * render kernel (DESIGN §13, §14). */
 int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups);
 /* The group count in force (bus rows = 2 * *out). */
 int ohs_num_groups(ohs_engine* h, int* out);
@@ -312,6 +322,20 @@ int ohs_mix_device(ohs_engine* h, const float* d_in, float* d_bus, size_t n_fram
  * also allocates the bus staging. */
 int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
                         size_t bus_stride);
+/* ohs_process_grouped with the buses delivered in bus_format (OHS_FMT_F32: exactly ohs_process_grouped).  Host memory;
+ * bus row r at byte r * bus_stride * bytes(bus_format).  Renders what ohs_process_grouped renders, in the same chunks, and
+ * leaves the same engine state, plus the dither position and bus history of an integer bus (above): each chunk's buses are
+ * mixed, dithered and encoded in one launch on the GPU, and only the 2 or 3 bytes per bus sample cross PCIe back.  Bypass:
+ * bus = encode(mix(decode(in))), dithered, and the position moves on.  OHS_ERR_INVALID with the engine untouched: the
+ * argument rules of ohs_process_grouped, an unknown bus format, and a bus whose bytes overlap the input. */
+int ohs_process_grouped_pcm(ohs_engine* h, const void* in, int in_format, void* bus, int bus_format, size_t n_frames,
+                            size_t row_stride, size_t bus_stride);
+/* Device memory: f32 stream rows -> the group buses in bus_format, one launch on the engine's stream (no f32 bus in
+ * between).  OHS_FMT_F32 is exactly ohs_mix_device.  An integer bus takes the alignment rules of ohs_mix_device plus
+ * bus_stride a multiple of 8 (S16) or 16 (S24) frames, else OHS_ERR_ALIGNMENT; an unknown format is OHS_ERR_INVALID.  The
+ * rendered rows usually come from ohs_process_device on the same engine, which leaves the position alone. */
+int ohs_mix_device_pcm(ohs_engine* h, const float* d_in, void* d_bus, int bus_format, size_t n_frames, size_t row_stride,
+                       size_t bus_stride);
 
 /* ---- multi-GPU collectives (SURVEY.md 8e) -------------------------------------------------------------------------
  * Streams shard across GPUs with no data-path collective; NCCL is used for exactly two things, both available here so
@@ -344,8 +368,11 @@ int ohs_debug_trace(ohs_engine* h, unsigned long long* d_stamps);
  * The blob holds a self-describing header (geometry, ring head, flags, byte count), the delay line, the overlap-save
  * blocks, the biquad states and whatever ohs_process_fifo has queued, and while dither is on (flags bit 0) the dither
  * position (uint64) and error history (float[2 * n_streams][OHS_MAX_SHAPE_TAPS]) behind them; with dither off the blob
- * is what it was before dither existed.  Import rejects a blob whose geometry, size, ring head or dither flag does not
- * match this engine, and then leaves the engine untouched.  ohs_state_bytes is the size an export would need NOW (it grows with the FIFO). */
+ * is what it was before dither existed.  Flags bit 1, only while dither is on and a bus has been encoded since the last
+ * ohs_set_dither, ohs_set_groups or import: int32 n_groups, int32 0, float[2 * n_groups][OHS_MAX_SHAPE_TAPS] (the bus
+ * rows' history) behind the dither section.  Import rejects a blob whose geometry, size, ring head or dither flag does
+ * not match this engine, bit 1 without bit 0 or with another group count, and then leaves the engine untouched; a blob
+ * without bit 1 zeroes the bus rows' history.  ohs_state_bytes is the size an export would need NOW (it grows with the FIFO). */
 int ohs_state_bytes(ohs_engine* h, size_t* bytes);
 int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes);
 int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes);

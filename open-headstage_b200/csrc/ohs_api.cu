@@ -100,7 +100,8 @@ struct ohs_engine {
     // ... and its integer-PCM rows: the PCM rows of a chunk, both directions, beside d_stage
     unsigned char* d_pcm_stage[kPipe] = {nullptr, nullptr, nullptr};
     size_t pcm_stage_cap = 0;
-    // ... and ohs_process_grouped's bus rows of a chunk (2 * n_groups rows), beside d_stage
+    // ... and ohs_process_grouped_pcm's bus rows of a chunk (2 * n_groups rows), beside d_stage: f32 rows, or the packed PCM
+    // rows of an integer bus (pitch round_up(n, 16) frames, never more bytes than the f32 rows of the same chunk)
     float* d_bus_stage[kPipe] = {nullptr, nullptr, nullptr};
     size_t bus_stage_cap = 0;
     // f32 rows of ohs_process_device_pcm's time chunks (decoded input, rendered in place)
@@ -111,7 +112,8 @@ struct ohs_engine {
     int dither_mode = OHS_DITHER_OFF, dither_taps = 0;
     unsigned long long dither_seed = 0, dither_pos = 0;
     ohs::DitherTaps dither_h{};
-    float* d_dither_hist = nullptr;   // [2 * n_streams][OHS_MAX_SHAPE_TAPS], allocated by ohs_set_dither
+    float* d_dither_hist = nullptr;   // [4 * n_streams][OHS_MAX_SHAPE_TAPS], allocated by ohs_set_dither: stream rows, then bus rows
+    bool bus_hist_live = false;       // a bus has been encoded since ohs_set_dither, ohs_set_groups or a state import
 
     // listener buses (ohs_set_groups): group g holds streams h_group_first[g] .. h_group_first[g+1]-1; configuration like the
     // bindings, not state.  d_group_first is sized for n_streams groups.
@@ -392,52 +394,72 @@ int check_pcm_args(ohs_engine* h, const void* in, int in_format, const void* out
 
 static_assert(kShapeTaps == OHS_MAX_SHAPE_TAPS, "history rows of the shaped encode");
 
-// pcm_encode_shaped_kernel<Fmt, M> for the runtime tap count m (1..OHS_MAX_SHAPE_TAPS)
-template <int Fmt, int M = 1>
+// pcm_encode_shaped_kernel<Fmt, M, Mix> for the runtime tap count m (1..OHS_MAX_SHAPE_TAPS)
+template <int Fmt, bool Mix, int M = 1>
 void launch_encode_shaped(int m, cudaStream_t st, const float* f32, size_t f32_pitch, unsigned char* pcm, size_t pcm_pitch,
                           size_t n_frames, int rows, unsigned long long seed, unsigned long long pos, const DitherTaps& taps,
-                          float* hist) {
+                          float* hist, const int* group_first) {
     if constexpr (M <= kShapeTaps) {
         if (m != M)
-            return launch_encode_shaped<Fmt, M + 1>(m, st, f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist);
-        pcm_encode_shaped_kernel<Fmt, M><<<(rows + kShapeRows - 1) / kShapeRows, kShapeThreads, 0, st>>>(
-            f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist);
+            return launch_encode_shaped<Fmt, Mix, M + 1>(m, st, f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist,
+                                                         group_first);
+        pcm_encode_shaped_kernel<Fmt, M, Mix><<<(rows + kShapeRows - 1) / kShapeRows, kShapeThreads, 0, st>>>(
+            f32, f32_pitch, pcm, pcm_pitch, n_frames, rows, seed, pos, taps, hist, group_first);
     }
 }
 
+int n_groups(const ohs_engine* h) { return (int)h->h_group_first.size() - 1; }
+// the bus rows' error history: behind the 2 * n_streams stream rows, room for 2 * n_streams bus rows
+float* bus_hist(const ohs_engine* h) { return h->d_dither_hist + (size_t)h->cfg.n_streams * 2 * kShapeTaps; }
+size_t bus_hist_bytes(const ohs_engine* h) { return sizeof(float) * (size_t)h->cfg.n_streams * 2 * kShapeTaps; }
+
+// The encode of f32 rows into PCM rows, dithered as ohs_set_dither says.  Mix: the rows are the 2 * n_groups bus rows, each
+// the sum of its group's stream rows of `f32` (pcm_encode_kernel / pcm_encode_shaped_kernel with Mix): dither row numbers
+// from 2 * n_streams on, i.e. the key hash with the seed seed + phi * 2S, and the error history behind the streams' rows.
+template <int Fmt, bool Mix>
+void launch_encode(ohs_engine* h, unsigned char* pcm, size_t pcm_pitch, const float* f32, size_t f32_pitch, size_t n_frames,
+                   unsigned long long pos) {
+    const size_t S2 = (size_t)h->cfg.n_streams * 2, rows = Mix ? (size_t)2 * n_groups(h) : S2;
+    const size_t groups = (n_frames + PcmTraits<Fmt>::kGroup - 1) / PcmTraits<Fmt>::kGroup, total = rows * groups;
+    const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
+    const unsigned long long seed = h->dither_seed + (Mix ? kDitherPhi * S2 : 0ull);
+    float* hist = h->d_dither_hist ? h->d_dither_hist + (Mix ? S2 * kShapeTaps : 0) : nullptr;
+    const int* gf = Mix ? h->d_group_first : nullptr;
+    if (h->dither_mode == OHS_DITHER_TPDF && h->dither_taps > 0)
+        launch_encode_shaped<Fmt, Mix>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
+                                       h->dither_h, hist, gf);
+    else if (h->dither_mode == OHS_DITHER_TPDF)
+        pcm_encode_kernel<Fmt, true, Mix><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed,
+                                                                             pos, gf);
+    else
+        pcm_encode_kernel<Fmt, false, Mix><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0,
+                                                                              0, gf);
+}
+
 // PCM rows <-> f32 rows on the engine's stream; pcm_pitch in bytes, f32_pitch in floats.  An encode is dithered as
-// ohs_set_dither says, its first frame at dither position dither_pos + pos_offset (the frame's offset in the call).
+// ohs_set_dither says, its first frame at dither position dither_pos + pos_offset (the frame's offset in the call).  mix:
+// an encode of the group buses of the f32 stream rows into 2 * n_groups PCM bus rows (launch_encode).
 int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t pcm_pitch, float* f32, size_t f32_pitch, size_t n_frames,
-               size_t pos_offset = 0) {
+               size_t pos_offset = 0, bool mix = false) {
     const size_t rows = (size_t)h->cfg.n_streams * 2;
     const size_t groups = (n_frames + pcm_align_frames(fmt) - 1) / pcm_align_frames(fmt), total = rows * groups;
     const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
-    const unsigned long long seed = h->dither_seed, pos = h->dither_pos + pos_offset;
-    const bool tpdf = h->dither_mode == OHS_DITHER_TPDF, shaped = tpdf && h->dither_taps > 0;
+    const unsigned long long pos = h->dither_pos + pos_offset;
     if (decode && fmt == OHS_FMT_S16)
         pcm_decode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
     else if (decode)
         pcm_decode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
-    else if (shaped && fmt == OHS_FMT_S16)
-        launch_encode_shaped<kPcmS16>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
-                                      h->dither_h, h->d_dither_hist);
-    else if (shaped)
-        launch_encode_shaped<kPcmS24>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
-                                      h->dither_h, h->d_dither_hist);
-    else if (tpdf && fmt == OHS_FMT_S16)
-        pcm_encode_kernel<kPcmS16, true><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed, pos);
-    else if (tpdf)
-        pcm_encode_kernel<kPcmS24, true><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed, pos);
     else if (fmt == OHS_FMT_S16)
-        pcm_encode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
+        mix ? launch_encode<kPcmS16, true>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos)
+            : launch_encode<kPcmS16, false>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos);
     else
-        pcm_encode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0, 0);
+        mix ? launch_encode<kPcmS24, true>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos)
+            : launch_encode<kPcmS24, false>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos);
     OHS_CUDA(cudaGetLastError());
     h->launches++;
+    if (mix) h->bus_hist_live = true;
     return OHS_OK;
 }
-
-int n_groups(const ohs_engine* h) { return (int)h->h_group_first.size() - 1; }
 
 // The group buses of f32 rows on the engine's stream: 2 * n_groups rows of `bus` (ohs_mix_device, ohs_process_grouped).
 // A plain launch, without the programmatic-serialization attribute: it starts once the render before it has finished.
@@ -1030,7 +1052,7 @@ int ohs_set_dither(ohs_engine* h, int mode, uint64_t seed, const float* shape, i
     for (int k = 0; k < n_taps; ++k)
         if (!std::isfinite(shape[k])) return fail(OHS_ERR_INVALID, "shape[%d] is not finite", k);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
-    const size_t hist_bytes = sizeof(float) * (size_t)h->cfg.n_streams * 2 * OHS_MAX_SHAPE_TAPS;
+    const size_t hist_bytes = sizeof(float) * (size_t)h->cfg.n_streams * 4 * OHS_MAX_SHAPE_TAPS;   // stream rows, then bus rows (G <= S)
     if (mode != OHS_DITHER_OFF && !h->d_dither_hist) OHS_CUDA(cudaMalloc(&h->d_dither_hist, hist_bytes));
     // on the engine's stream: ordered after every encode enqueued before
     if (h->d_dither_hist) OHS_CUDA(cudaMemsetAsync(h->d_dither_hist, 0, hist_bytes, h->stream));
@@ -1040,6 +1062,7 @@ int ohs_set_dither(ohs_engine* h, int mode, uint64_t seed, const float* shape, i
     h->dither_h = DitherTaps{};
     for (int k = 0; k < n_taps; ++k) h->dither_h.h[k] = shape[k];
     h->dither_pos = 0;
+    h->bus_hist_live = false;
     return OHS_OK;
 }
 
@@ -1080,7 +1103,8 @@ int ohs_prepare(ohs_engine* h, size_t n_frames, int host_io) {
         const size_t rows = (size_t)h->cfg.n_streams * 2;
         per_launch = chunk_frames(h, n_frames, h->stage_bytes, 2);
         const size_t pcm_bytes = rows * std::max(per_launch * 2, chunk_frames(h, n_frames, h->stage_bytes, 3) * 3);
-        // ohs_process_grouped's bus rows: its chunks are those of F32 output
+        // ohs_process_grouped_pcm's bus rows: its chunks are those of F32 output, and an integer bus's packed rows
+        // (round_up(n, 16) frames of at most 3 bytes) fit in the f32 rows' bytes
         const size_t bus_bytes = (size_t)2 * n_groups(h) * chunk_frames(h, n_frames, h->stage_bytes, sizeof(float)) * sizeof(float);
         if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * per_launch * sizeof(float))) ||
             (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, pcm_bytes)) ||
@@ -1332,6 +1356,28 @@ int ohs_mix_device(ohs_engine* h, const float* d_in, float* d_bus, size_t n_fram
     return launch_mix(h, d_in, row_stride, d_bus, bus_stride, n_frames);
 }
 
+int ohs_mix_device_pcm(ohs_engine* h, const float* d_in, void* d_bus, int bus_format, size_t n_frames, size_t row_stride,
+                       size_t bus_stride) {
+    OHS_CHECK_HANDLE(h);
+    if (bus_format != OHS_FMT_F32 && bus_format != OHS_FMT_S16 && bus_format != OHS_FMT_S24)
+        return fail(OHS_ERR_INVALID, "unknown bus format %d", bus_format);
+    if (bus_format == OHS_FMT_F32) return ohs_mix_device(h, d_in, static_cast<float*>(d_bus), n_frames, row_stride, bus_stride);
+    if (!d_in || !d_bus) return fail(OHS_ERR_INVALID, "null audio pointer");
+    const size_t align = pcm_align_frames(bus_format);
+    if (n_frames % 4 || row_stride % 4 || bus_stride % align || (((uintptr_t)d_in | (uintptr_t)d_bus) & 15u))
+        return fail(OHS_ERR_ALIGNMENT, "mixdown needs 16-byte aligned pointers, n_frames and row_stride multiples of 4 and bus_stride a "
+                                       "multiple of %zu frames", align);
+    if (row_stride < n_frames || bus_stride < n_frames) return fail(OHS_ERR_INVALID, "stride smaller than n_frames");
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    if (n_frames) {
+        const int rc = launch_pcm(h, false, bus_format, static_cast<unsigned char*>(d_bus), bus_stride * pcm_sample_bytes(bus_format),
+                                  const_cast<float*>(d_in), row_stride, n_frames, 0, true);
+        if (rc) return rc;
+    }
+    h->dither_pos += n_frames;
+    return OHS_OK;
+}
+
 int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups) {
     OHS_CHECK_HANDLE(h);
     const int S = h->cfg.n_streams;
@@ -1345,6 +1391,9 @@ int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups) {
     std::vector<int> v(first, first + n_groups + 1);
     // on the engine's stream: mixes enqueued before still read the old offsets (a pageable source is staged before returning)
     OHS_CUDA(cudaMemcpyAsync(h->d_group_first, v.data(), sizeof(int) * v.size(), cudaMemcpyHostToDevice, h->stream));
+    // a new partition makes the old bus rows' error history meaningless: zeroed, in the same order as the offsets
+    if (h->d_dither_hist) OHS_CUDA(cudaMemsetAsync(bus_hist(h), 0, bus_hist_bytes(h), h->stream));
+    h->bus_hist_live = false;
     h->h_group_first.swap(v);
     return OHS_OK;
 }
@@ -1516,23 +1565,27 @@ namespace {
 // chunks overlap on three CUDA streams.  Integer PCM crosses the link as PCM and is converted in HBM.  Per chunk: copy-in
 // (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into the f32 buffer, render
 // there in place, encode back into the PCM buffer, copy-out.  ohs_process is the F32 -> F32 case.  With `bus`
-// (ohs_process_grouped: F32 output, `out` unused) the rendered rows are mixed into the slot's group buses instead, and
-// only those 2 * n_groups rows are copied out.  Arguments are validated by the caller.
+// (ohs_process_grouped_pcm: F32 output, `out` unused) the rendered rows are mixed into the slot's group buses instead,
+// encoded to bus_format in the same launch for an integer bus, and only those 2 * n_groups rows are copied out.  Arguments
+// are validated by the caller.
 int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride,
-                      float* bus = nullptr, size_t bus_stride = 0) {
+                      void* bus = nullptr, int bus_format = OHS_FMT_F32, size_t bus_stride = 0) {
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     if (n_frames == 0) return OHS_OK;
     int rc = OHS_OK;
     const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
-    const size_t bus_rows = (size_t)2 * n_groups(h);
+    const size_t bus_rows = (size_t)2 * n_groups(h), bb = pcm_sample_bytes(bus_format);
     const unsigned char* src = static_cast<const unsigned char*>(in);
     unsigned char* dst = static_cast<unsigned char*>(out);
+    unsigned char* bus_dst = static_cast<unsigned char*>(bus);
+    // the output words this call delivers: an integer format moves the dither position on
+    const bool int_out = bus ? bus_format != OHS_FMT_F32 : out_format != OHS_FMT_F32;
     if (h->bypass && in_format == out_format && !bus) {
         if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(dst + r * row_stride * bo, src + r * row_stride * bi, n_frames * bi);
-        if (out_format != OHS_FMT_F32) h->dither_pos += n_frames;
+        if (int_out) h->dither_pos += n_frames;
         return OHS_OK;
     }
-    const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32;
+    const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32, pcm_bus = bus && bus_format != OHS_FMT_F32;
     // about stage_bytes per copy of the wider side's rows: 24 MiB by default, measured best on PCIe Gen5 x16 with both
     // directions busy (tools/e2e_probe.py)
     const size_t chunk = chunk_frames(h, n_frames, h->stage_bytes, std::max(bi, bo));
@@ -1555,6 +1608,7 @@ int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, i
         float* x = h->d_stage[b];
         unsigned char* q = h->d_pcm_stage[b];
         float* g = h->d_bus_stage[b];
+        unsigned char* gq = reinterpret_cast<unsigned char*>(g);   // an integer bus: packed rows, pcm_pitch frames each
         if (used[b]) OHS_CUDA(cudaStreamWaitEvent(h->h2d, h->ev_out[b], 0));  // buffers free once their copy-out finished
         if (pcm_in)
             OHS_CUDA(cudaMemcpy2DAsync(q, pcm_pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
@@ -1565,12 +1619,15 @@ int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, i
         if (pcm_in && (rc = launch_pcm(h, true, in_format, q, pcm_pitch * bi, x, pitch, n))) return rc;
         if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
         if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n, done))) return rc;
-        if (bus && (rc = launch_mix(h, x, pitch, g, pitch, n))) return rc;
+        if (pcm_bus && (rc = launch_pcm(h, false, bus_format, gq, pcm_pitch * bb, x, pitch, n, done, true))) return rc;
+        if (bus && !pcm_bus && (rc = launch_mix(h, x, pitch, g, pitch, n))) return rc;
         OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
         OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
-        if (bus)
-            OHS_CUDA(cudaMemcpy2DAsync(bus + done, bus_stride * sizeof(float), g, pitch * sizeof(float), n * sizeof(float), bus_rows,
-                                       cudaMemcpyDeviceToHost, h->d2h));
+        if (pcm_bus)
+            OHS_CUDA(cudaMemcpy2DAsync(bus_dst + done * bb, bus_stride * bb, gq, pcm_pitch * bb, n * bb, bus_rows, cudaMemcpyDeviceToHost,
+                                       h->d2h));
+        else if (bus)
+            OHS_CUDA(cudaMemcpy2DAsync(bus_dst + done * bb, bus_stride * bb, g, pitch * bb, n * bb, bus_rows, cudaMemcpyDeviceToHost, h->d2h));
         else if (pcm_out)
             OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, q, pcm_pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
         else
@@ -1582,7 +1639,7 @@ int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, i
     }
     OHS_CUDA(cudaStreamSynchronize(h->d2h));
     OHS_CUDA(cudaStreamSynchronize(h->stream));
-    if (pcm_out) h->dither_pos += n_frames;
+    if (int_out) h->dither_pos += n_frames;
     return OHS_OK;
 }
 
@@ -1597,11 +1654,11 @@ int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int
     return process_host_impl(h, in, in_format, out, out_format, n_frames, row_stride);
 }
 
-int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
-                        size_t bus_stride) {
+int ohs_process_grouped_pcm(ohs_engine* h, const void* in, int in_format, void* bus, int bus_format, size_t n_frames, size_t row_stride,
+                            size_t bus_stride) {
     OHS_CHECK_HANDLE(h);
-    if (in_format != OHS_FMT_F32 && in_format != OHS_FMT_S16 && in_format != OHS_FMT_S24)
-        return fail(OHS_ERR_INVALID, "unknown sample format %d", in_format);
+    for (int f : {in_format, bus_format})
+        if (f != OHS_FMT_F32 && f != OHS_FMT_S16 && f != OHS_FMT_S24) return fail(OHS_ERR_INVALID, "unknown sample format %d", f);
     int rc = check_audio_args(h, in, bus, n_frames, row_stride, false);
     if (rc) return rc;
     if (bus_stride < n_frames) return fail(OHS_ERR_INVALID, "bus_stride %zu < n_frames %zu", bus_stride, n_frames);
@@ -1609,9 +1666,14 @@ int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus
     const size_t rows = (size_t)h->cfg.n_streams * 2, bus_rows = (size_t)2 * n_groups(h);
     const uintptr_t a = (uintptr_t)in, b = (uintptr_t)bus;
     const size_t na = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(in_format);
-    const size_t nb = ((bus_rows - 1) * bus_stride + n_frames) * sizeof(float);
+    const size_t nb = ((bus_rows - 1) * bus_stride + n_frames) * pcm_sample_bytes(bus_format);
     if (a < b + nb && b < a + na) return fail(OHS_ERR_INVALID, "the bus overlaps the input");
-    return process_host_impl(h, in, in_format, nullptr, OHS_FMT_F32, n_frames, row_stride, bus, bus_stride);
+    return process_host_impl(h, in, in_format, nullptr, OHS_FMT_F32, n_frames, row_stride, bus, bus_format, bus_stride);
+}
+
+int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
+                        size_t bus_stride) {
+    return ohs_process_grouped_pcm(h, in, in_format, bus, OHS_FMT_F32, n_frames, row_stride, bus_stride);
 }
 
 int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride) {
@@ -1672,6 +1734,7 @@ int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames
 // ---- state export / import ----------------------------------------------------------------------------------
 // blob = StateHeader | delay line | overlap-save blocks | biquad states | FIFO residue (input rows, output rows)
 //        [ | dither position (uint64) | error history float[2S][OHS_MAX_SHAPE_TAPS] ]  when flags has kStateDither
+//        [ | n_groups (int32) | 0 (int32) | bus error history float[2G][OHS_MAX_SHAPE_TAPS] ]  when flags has kStateBus
 namespace {
 struct StateHeader {
     uint32_t magic;      // 'OHSS'
@@ -1680,25 +1743,31 @@ struct StateHeader {
 };
 constexpr uint32_t kStateMagic = 0x5353484Fu;
 constexpr int32_t kStateDither = 1;   // the dither section follows the FIFO residue
+constexpr int32_t kStateBus = 2;      // the bus section follows the dither section (dither on and a bus encoded)
 size_t dither_state_bytes(const ohs_engine* h) { return sizeof(uint64_t) + sizeof(float) * (size_t)h->cfg.n_streams * 2 * OHS_MAX_SHAPE_TAPS; }
+size_t bus_state_floats(int groups) { return (size_t)groups * 2 * OHS_MAX_SHAPE_TAPS; }
 size_t state_need(const ohs_engine* h, size_t fifo_in, size_t fifo_out, bool dither) {
     const size_t S = h->cfg.n_streams;
     return sizeof(StateHeader) + sizeof(float2) * S * h->pmax * h->N + sizeof(float2) * S * h->B + sizeof(float4) * S * kMaxBands +
            sizeof(float) * S * 2 * (fifo_in + fifo_out) + (dither ? dither_state_bytes(h) : 0);
 }
+// the blob carries the bus rows' history only while it means something: dither on and a bus encoded since it was zeroed
+bool bus_state(const ohs_engine* h) { return h->dither_mode != OHS_DITHER_OFF && h->bus_hist_live; }
+size_t bus_state_bytes(int groups) { return 2 * sizeof(int32_t) + sizeof(float) * bus_state_floats(groups); }
 }  // namespace
 
 int ohs_state_bytes(ohs_engine* h, size_t* bytes) {
     OHS_CHECK_HANDLE(h);
     if (!bytes) return fail(OHS_ERR_INVALID, "null output");
-    *bytes = state_need(h, h->fifo_in_len, h->fifo_out_len, h->dither_mode != OHS_DITHER_OFF);
+    *bytes = state_need(h, h->fifo_in_len, h->fifo_out_len, h->dither_mode != OHS_DITHER_OFF) + (bus_state(h) ? bus_state_bytes(n_groups(h)) : 0);
     return OHS_OK;
 }
 
 int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
     OHS_CHECK_HANDLE(h);
-    const bool dither = h->dither_mode != OHS_DITHER_OFF;
-    const size_t need = state_need(h, h->fifo_in_len, h->fifo_out_len, dither);
+    const bool dither = h->dither_mode != OHS_DITHER_OFF, bus = bus_state(h);
+    const int G = n_groups(h);
+    const size_t need = state_need(h, h->fifo_in_len, h->fifo_out_len, dither) + (bus ? bus_state_bytes(G) : 0);
     if (!host_buf || bytes < need) return fail(OHS_ERR_INVALID, "state buffer too small (%zu < %zu)", bytes, need);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     int rc = commit_filters(h);
@@ -1708,7 +1777,8 @@ int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
     OHS_CUDA(cudaStreamSynchronize(h->stream));
     unsigned char* p = (unsigned char*)host_buf;
     const size_t S = h->cfg.n_streams;
-    StateHeader hdr{kStateMagic, OHS_ABI_VERSION, h->cfg.n_streams, kMaxBands, h->pmax, h->B, h->head, dither ? kStateDither : 0,
+    StateHeader hdr{kStateMagic, OHS_ABI_VERSION, h->cfg.n_streams, kMaxBands, h->pmax, h->B, h->head,
+                    (dither ? kStateDither : 0) | (bus ? kStateBus : 0),
                     (uint64_t)h->fifo_in_len, (uint64_t)h->fifo_out_len, (uint64_t)need};
     memcpy(p, &hdr, sizeof(hdr)); p += sizeof(hdr);
     const size_t n0 = sizeof(float2) * S * h->pmax * h->N, n1 = sizeof(float2) * S * h->B, n2 = sizeof(float4) * S * kMaxBands;
@@ -1722,6 +1792,12 @@ int ohs_state_export(ohs_engine* h, void* host_buf, size_t bytes) {
         const uint64_t pos = h->dither_pos;
         memcpy(p, &pos, sizeof(pos)); p += sizeof(pos);
         OHS_CUDA(cudaMemcpy(p, h->d_dither_hist, dither_state_bytes(h) - sizeof(pos), cudaMemcpyDeviceToHost));
+        p += dither_state_bytes(h) - sizeof(pos);
+    }
+    if (bus) {
+        const int32_t head[2] = {G, 0};
+        memcpy(p, head, sizeof(head)); p += sizeof(head);
+        OHS_CUDA(cudaMemcpy(p, bus_hist(h), sizeof(float) * bus_state_floats(G), cudaMemcpyDeviceToHost));
     }
     return OHS_OK;
 }
@@ -1739,12 +1815,21 @@ int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes) {
     if (hdr.head < 0 || hdr.head >= h->pmax) return fail(OHS_ERR_INVALID, "state blob ring head %d outside 0..%d", hdr.head, h->pmax - 1);
     const size_t limit = (size_t)1 << 32;
     if (hdr.fifo_in_len > limit || hdr.fifo_out_len > limit) return fail(OHS_ERR_INVALID, "state blob FIFO lengths are implausible");
-    if (hdr.flags & ~kStateDither) return fail(OHS_ERR_INVALID, "state blob has unknown flags 0x%x", (unsigned)hdr.flags);
-    const bool dither = (hdr.flags & kStateDither) != 0;
+    if (hdr.flags & ~(kStateDither | kStateBus)) return fail(OHS_ERR_INVALID, "state blob has unknown flags 0x%x", (unsigned)hdr.flags);
+    const bool dither = (hdr.flags & kStateDither) != 0, bus = (hdr.flags & kStateBus) != 0;
+    if (bus && !dither) return fail(OHS_ERR_INVALID, "state blob carries bus dither history without dither state");
     if (dither != (h->dither_mode != OHS_DITHER_OFF))
         return fail(OHS_ERR_INVALID, dither ? "state blob carries dither state but this engine's dither is off"
                                             : "state blob carries no dither state but this engine dithers (ohs_set_dither first)");
-    const size_t need = state_need(h, (size_t)hdr.fifo_in_len, (size_t)hdr.fifo_out_len, dither);
+    size_t need = state_need(h, (size_t)hdr.fifo_in_len, (size_t)hdr.fifo_out_len, dither);
+    const int G = n_groups(h);
+    if (bus) {
+        int32_t head[2] = {0, 0};
+        if (bytes >= need + sizeof(head)) memcpy(head, (const unsigned char*)host_buf + need, sizeof(head));
+        if (head[0] != G || head[1] != 0)
+            return fail(OHS_ERR_INVALID, "state blob's bus history is for %d groups, this engine has %d", head[0], G);
+        need += bus_state_bytes(G);
+    }
     if (hdr.total_bytes != need || bytes != need) return fail(OHS_ERR_INVALID, "state blob is %zu bytes, header says %llu, geometry needs %zu", bytes, (unsigned long long)hdr.total_bytes, need);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
     int rc = commit_filters(h);  // pending set_ir would otherwise clear the imported history later
@@ -1767,8 +1852,13 @@ int ohs_state_import(ohs_engine* h, const void* host_buf, size_t bytes) {
         uint64_t pos;
         memcpy(&pos, p, sizeof(pos)); p += sizeof(pos);
         OHS_CUDA(cudaMemcpy(h->d_dither_hist, p, dither_state_bytes(h) - sizeof(pos), cudaMemcpyHostToDevice));
+        p += dither_state_bytes(h) - sizeof(pos);
         h->dither_pos = pos;
+        // the bus rows' history: the blob's, or zeros for a blob written before any bus encode
+        if (bus) OHS_CUDA(cudaMemcpy(bus_hist(h), p + 2 * sizeof(int32_t), sizeof(float) * bus_state_floats(G), cudaMemcpyHostToDevice));
+        else OHS_CUDA(cudaMemset(bus_hist(h), 0, bus_hist_bytes(h)));
     }
+    h->bus_hist_live = bus;
     return OHS_OK;
 }
 

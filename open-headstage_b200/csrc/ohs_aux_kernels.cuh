@@ -493,25 +493,67 @@ template <int Fmt> __device__ __forceinline__ int pcm_quantise_dithered(float y,
     return __float2int_rn(fminf(fmaxf(__fadd_rn(v, d), P::kLo), P::kHi));
 }
 
+// Mixed encode (bus rows, ohs_process_grouped_pcm / ohs_mix_device_pcm): row r of the output is bus row 2g + c, and its f32
+// samples are the group's stream rows in[(2s + c)], s = group_first[g] .. group_first[g+1]-1, summed from +0 in ascending
+// stream order (mix_streams_kernel's sum, bit for bit).  group_sum1: one frame, `src` at the group's first stream row;
+// the ns rows sit 2 * pitch apart.
+__device__ __forceinline__ float group_sum1(const float* src, int ns, size_t pitch) {
+    float acc = 0.f;
+    for (int s = 0; s < ns; ++s) acc += src[(size_t)s * 2 * pitch];
+    return acc;
+}
+
 // in: f32 rows (pitch in floats), out: PCM rows (pitch in bytes).  Dither: flat TPDF, the group's first frame at dither
 // position pos0 + f0 (the parameters behind `total` are read only then, so the undithered kernel is the plain encode).
-template <int Fmt, bool Dither = false>
+// Mix: `total` counts the groups of the bus rows, and a thread sums its frames of the group's stream rows into registers
+// first (the f32 bus is never stored); group_first is read only then.
+template <int Fmt, bool Dither = false, bool Mix = false>
 __global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict__ in, size_t in_pitch, unsigned char* __restrict__ out,
                                                          size_t out_pitch, size_t n_frames, size_t groups, size_t total,
-                                                         unsigned long long seed, unsigned long long pos0) {
+                                                         unsigned long long seed, unsigned long long pos0,
+                                                         const int* __restrict__ group_first) {
     using P = PcmTraits<Fmt>;
     constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
     for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
         const size_t row = t / groups, f0 = (t - row * groups) * G;
         const float* src = in + row * in_pitch + f0;
         unsigned char* dst = out + row * out_pitch + f0 * NB;
+        // the samples of the thread's frames: the row itself, or (Mix) the group sums, all G of them in registers
+        [[maybe_unused]] float4 mixed[G / 4];
+        [[maybe_unused]] int ns = 0;
+        if constexpr (Mix) {
+            const int g = (int)(row >> 1), s0 = group_first[g];
+            ns = group_first[g + 1] - s0;
+            src = in + ((size_t)s0 * 2 + (row & 1)) * in_pitch + f0;
+            if (f0 + G <= n_frames) {
+#pragma unroll
+                for (int v = 0; v < G / 4; ++v) mixed[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 2
+                for (int s = 0; s < ns; ++s) {
+                    const float* r = src + (size_t)s * 2 * in_pitch;
+#pragma unroll
+                    for (int v = 0; v < G / 4; ++v) {
+                        const float4 x = reinterpret_cast<const float4*>(r)[v];
+                        mixed[v].x += x.x; mixed[v].y += x.y; mixed[v].z += x.z; mixed[v].w += x.w;
+                    }
+                }
+            }
+        }
+        auto sample4 = [&](int v) -> float4 {
+            if constexpr (Mix) return mixed[v];
+            else return reinterpret_cast<const float4*>(src)[v];
+        };
+        auto sample1 = [&](size_t k) -> float {
+            if constexpr (Mix) return group_sum1(src + k, ns, in_pitch);
+            else return src[k];
+        };
         if constexpr (Dither) {
             unsigned long long z = dither_row_key(seed, row) + kDitherPhi * (pos0 + f0 + 1);
             if (f0 + G <= n_frames) {
                 int q[G];
 #pragma unroll
                 for (int v = 0; v < G / 4; ++v) {
-                    const float4 y = reinterpret_cast<const float4*>(src)[v];
+                    const float4 y = sample4(v);
                     const float ys[4] = {y.x, y.y, y.z, y.w};
 #pragma unroll
                     for (int j = 0; j < 4; ++j) { q[4 * v + j] = pcm_quantise_dithered<Fmt>(ys[j], dither_noise(z)); z += kDitherPhi; }
@@ -522,13 +564,13 @@ __global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict
                 for (int v = 0; v < W / 4; ++v) reinterpret_cast<uint4*>(dst)[v] = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
             } else {
                 for (size_t k = 0; f0 + k < n_frames; ++k, z += kDitherPhi)
-                    pcm_store_one<Fmt>(dst + k * NB, pcm_quantise_dithered<Fmt>(src[k], dither_noise(z)));
+                    pcm_store_one<Fmt>(dst + k * NB, pcm_quantise_dithered<Fmt>(sample1(k), dither_noise(z)));
             }
         } else if (f0 + G <= n_frames) {
             int q[G];
 #pragma unroll
             for (int v = 0; v < G / 4; ++v) {
-                const float4 y = reinterpret_cast<const float4*>(src)[v];
+                const float4 y = sample4(v);
                 q[4 * v] = pcm_quantise<Fmt>(y.x); q[4 * v + 1] = pcm_quantise<Fmt>(y.y);
                 q[4 * v + 2] = pcm_quantise<Fmt>(y.z); q[4 * v + 3] = pcm_quantise<Fmt>(y.w);
             }
@@ -537,7 +579,7 @@ __global__ void __launch_bounds__(256) pcm_encode_kernel(const float* __restrict
 #pragma unroll
             for (int v = 0; v < W / 4; ++v) reinterpret_cast<uint4*>(dst)[v] = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
         } else {
-            for (size_t k = 0; f0 + k < n_frames; ++k) pcm_store_one<Fmt>(dst + k * NB, pcm_quantise<Fmt>(src[k]));
+            for (size_t k = 0; f0 + k < n_frames; ++k) pcm_store_one<Fmt>(dst + k * NB, pcm_quantise<Fmt>(sample1(k)));
         }
     }
 }
@@ -589,14 +631,17 @@ template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile(
 // byte tile that the whole CTA stores with 16-byte stores.  Tile rows are padded by 16 bytes, so that the 16-byte
 // accesses of eight lanes to eight rows (one shared-memory wavefront) fall on distinct banks.  The history e_1..e_M of a
 // row is read from hist[row][0..M) at the start of a launch and written back at its end.
+// Mix: the CTA's rows are bus rows, and each f32 tile holds the group sums instead of copies: warps 1-3 build
+// tile k+1 (plain loads and stores to shared memory) before its noise, while warp 0 runs the recurrence on tile k, and all
+// four warps build tile 0.  group_first is read only then.
 constexpr int kShapeT = 64, kShapeRows = 32, kShapeThreads = 128, kShapeStages = 2;
 
-template <int Fmt, int M>
+template <int Fmt, int M, bool Mix = false>
 __global__ void __launch_bounds__(kShapeThreads) pcm_encode_shaped_kernel(const float* __restrict__ in, size_t in_pitch,
                                                                         unsigned char* __restrict__ out, size_t out_pitch,
                                                                         size_t n_frames, int rows, unsigned long long seed,
                                                                         unsigned long long pos0, DitherTaps taps,
-                                                                        float* __restrict__ hist) {
+                                                                        float* __restrict__ hist, const int* __restrict__ group_first) {
     using P = PcmTraits<Fmt>;
     constexpr int G = P::kGroup, NB = P::kBytes, W = G * NB / 4;
     constexpr int T = kShapeT, R = kShapeRows, NT = kShapeThreads, IP = T + 4, OP = T * NB + 16, C4 = T / 4, C16 = T * NB / 16;
@@ -619,6 +664,43 @@ __global__ void __launch_bounds__(kShapeThreads) pcm_encode_shaped_kernel(const 
         }
         cp_async_commit();   // an empty group past the last tile keeps the wait counts uniform
     };
+    // Mix: tile k of the bus rows from the stream rows.  A thread owns up to J float4 columns and walks their streams
+    // together, so that J independent 16-byte loads are in flight per stream step: one column at a time left the
+    // build, not the recurrence, on the critical path.
+    auto build = [&](size_t k, int i0, int step) {
+        constexpr int J = (R * C4 + (NT - 32) - 1) / (NT - 32);   // columns per thread of warps 1-3 (all warps: fewer)
+        const size_t f0 = k * T;
+        const int nv = (int)((min((size_t)T, n_frames - f0) + 3) / 4);
+        const float* src[J];
+        int ns[J], nmax = 0;
+        float4 acc[J];
+#pragma unroll
+        for (int j = 0; j < J; ++j) {
+            const int i = i0 + j * step, r = i / C4, c = i - r * C4;
+            src[j] = in; ns[j] = 0; acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (i < R * C4 && r < nr && c < nv) {
+                const int row = r0 + r, s0 = group_first[row >> 1];
+                ns[j] = group_first[(row >> 1) + 1] - s0;
+                src[j] = in + ((size_t)s0 * 2 + (row & 1)) * in_pitch + f0 + 4 * c;
+            }
+            nmax = max(nmax, ns[j]);
+        }
+#pragma unroll 2
+        for (int s = 0; s < nmax; ++s) {
+#pragma unroll
+            for (int j = 0; j < J; ++j)
+                if (s < ns[j]) {
+                    const float4 v = *reinterpret_cast<const float4*>(src[j] + (size_t)s * 2 * in_pitch);
+                    acc[j].x += v.x; acc[j].y += v.y; acc[j].z += v.z; acc[j].w += v.w;
+                }
+        }
+#pragma unroll
+        for (int j = 0; j < J; ++j)
+            if (ns[j]) {
+                const int i = i0 + j * step, r = i / C4, c = i - r * C4;
+                *reinterpret_cast<float4*>(&xs[k % kShapeStages][r][4 * c]) = acc[j];
+            }
+    };
     auto noise = [&](size_t k) {   // warps 1-3: the noise of tile k (every frame of it; those past n_frames go unused)
         const unsigned long long p = pos0 + k * T + 1;
         for (int i = tid - 32; i < R * C4; i += NT - 32) {
@@ -636,12 +718,15 @@ __global__ void __launch_bounds__(kShapeThreads) pcm_encode_shaped_kernel(const 
     const bool owner = tid < nr;
 #pragma unroll
     for (int k = 0; k < M; ++k) e[k] = owner ? hist[(size_t)(r0 + tid) * kShapeTaps + k] : 0.f;
-    load(0);
-    __syncthreads();   // keys
+    if constexpr (Mix) build(0, tid, NT);
+    else load(0);
+    __syncthreads();   // keys (Mix: and tile 0)
     if (tid >= 32) noise(0);
     for (size_t k = 0; k < n_tiles; ++k) {
-        load(k + 1);
-        cp_async_wait<1>();   // this thread's copies of tile k have landed ...
+        if constexpr (!Mix) {
+            load(k + 1);
+            cp_async_wait<1>();   // this thread's copies of tile k have landed ...
+        }
         __syncthreads();      // ... and everybody's; the noise of tile k is written
         const size_t f0 = k * T;
         const int nf = (int)min((size_t)T, n_frames - f0);
@@ -681,6 +766,7 @@ __global__ void __launch_bounds__(kShapeThreads) pcm_encode_shaped_kernel(const 
                     *reinterpret_cast<uint4*>(o + g * NB + 16 * v) = make_uint4(w[4 * v], w[4 * v + 1], w[4 * v + 2], w[4 * v + 3]);
             }
         } else if (tid >= 32 && k + 1 < n_tiles) {
+            if constexpr (Mix) build(k + 1, tid - 32, NT - 32);
             noise(k + 1);
         }
         __syncthreads();   // the byte tile is complete

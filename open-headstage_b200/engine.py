@@ -82,6 +82,8 @@ SYMBOLS = [
     ("ohs_set_groups", C.c_int, [_VP, _VP, C.c_int]),
     ("ohs_num_groups", C.c_int, [_VP, C.POINTER(C.c_int)]),
     ("ohs_process_grouped", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_size_t, C.c_size_t, C.c_size_t]),
+    ("ohs_process_grouped_pcm", C.c_int, [_VP, _VP, C.c_int, _VP, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t]),
+    ("ohs_mix_device_pcm", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t]),
     ("ohs_comm_unique_id", C.c_int, [_VP]),
     ("ohs_comm_create", C.c_int, [C.POINTER(_VP), C.c_int, C.c_int, C.c_int, _VP]),
     ("ohs_comm_destroy", C.c_int, [_VP]),
@@ -151,6 +153,17 @@ def _pcm_input(x, n_streams: int):
     else:
         raise ValueError("process_pcm takes int16, float32 or packed 24-bit uint8 [S, 2, 3n] input, got %s %s" % (x.dtype, x.shape))
     return np.ascontiguousarray(x), fmt, n
+
+
+def _pcm_rows(shape, fmt: int):
+    """The (shape, dtype) of PCM rows [*shape, n] in `fmt`: int16 [.., n] (S16), packed uint8 [.., 3n] (S24), float32 (F32)."""
+    if fmt == FMT_F32:
+        return tuple(shape), np.dtype(np.float32)
+    if fmt == FMT_S16:
+        return tuple(shape), np.dtype(np.int16)
+    if fmt == FMT_S24:
+        return tuple(shape[:-1]) + (3 * shape[-1],), np.dtype(np.uint8)
+    raise ValueError("unknown sample format %r" % (fmt,))
 
 
 def eq_design(filter_type: int, fs: float, fc: float, q: float, gain_db: float) -> np.ndarray:
@@ -356,10 +369,7 @@ class Engine:
         float32 [S, 2, n] is F32, uint8 [S, 2, 3n] is packed S24 (signals.pack_s24).  Returns int16 [S, 2, n] for
         FMT_S16, uint8 [S, 2, 3n] for FMT_S24, float32 [S, 2, n] for FMT_F32 (or fills `out`, e.g. a PinnedBuffer's array)."""
         x, fmt, n = _pcm_input(x, self.n_streams)
-        shape = {FMT_F32: (n, np.float32), FMT_S16: (n, np.int16), FMT_S24: (3 * n, np.uint8)}
-        if out_format not in shape:
-            raise ValueError("unknown sample format %r" % (out_format,))
-        want = ((self.n_streams, 2, shape[out_format][0]), np.dtype(shape[out_format][1]))
+        want = _pcm_rows((self.n_streams, 2, n), out_format)
         if out is None:
             y = np.empty(*want)
         else:
@@ -384,23 +394,25 @@ class Engine:
         _check(self._L.ohs_num_groups(self._h, C.byref(n)))
         return n.value
 
-    def process_grouped(self, x, out=None, bus_stride: int | None = None) -> np.ndarray:
-        """Host flavour returning only the group buses (ohs_process_grouped): renders what process_pcm(x, FMT_F32) renders
-        and returns the buses as float32 [n_groups, 2, n] (the input format follows the dtype, as in process_pcm).  `out`:
-        a writeable C-contiguous float32 [n_groups, 2, bus_stride] array (e.g. a PinnedBuffer's); the first n frames of
-        each of its rows are written and returned as a view."""
+    def process_grouped(self, x, out=None, bus_stride: int | None = None, bus_format: int = FMT_F32) -> np.ndarray:
+        """Host flavour returning only the group buses (ohs_process_grouped_pcm): renders what process_pcm(x, FMT_F32) renders
+        and returns the buses [n_groups, 2, n] in `bus_format`: float32 (FMT_F32), int16 (FMT_S16) or packed uint8
+        [n_groups, 2, 3n] (FMT_S24), the integer ones dithered as set_dither says (the input format follows the dtype, as in
+        process_pcm).  `out`: a writeable C-contiguous array of that dtype and shape [n_groups, 2, bus_stride] (3 * bus_stride
+        bytes per row for S24; e.g. a PinnedBuffer's); the first n frames of each of its rows are written and returned as a
+        view."""
         x, fmt, n = _pcm_input(x, self.n_streams)
+        _pcm_rows((n,), bus_format)   # an unknown format is refused before the library is asked for the group count
         bs = n if bus_stride is None else int(bus_stride)
-        want = (self.n_groups, 2, bs)
+        want = _pcm_rows((self.n_groups, 2, bs), bus_format)
         if out is None:
-            y = np.empty(want, np.float32)
+            y = np.empty(*want)
         else:
             y = out
-            if not (isinstance(y, np.ndarray) and y.dtype == np.float32 and y.shape == want and y.flags["C_CONTIGUOUS"]
-                    and y.flags["WRITEABLE"]):
-                raise ValueError("out must be a writeable C-contiguous float32 array of shape %s" % (want,))
-        _check(self._L.ohs_process_grouped(self._h, x.ctypes.data, fmt, y.ctypes.data, n, n, bs))
-        return y[:, :, :n]
+            if not (isinstance(y, np.ndarray) and (y.shape, y.dtype) == want and y.flags["C_CONTIGUOUS"] and y.flags["WRITEABLE"]):
+                raise ValueError("out must be a writeable C-contiguous %s array of shape %s" % (want[1], want[0]))
+        _check(self._L.ohs_process_grouped_pcm(self._h, x.ctypes.data, fmt, y.ctypes.data, bus_format, n, n, bs))
+        return y[:, :, :_pcm_rows((n,), bus_format)[0][0]]
 
     def process_device_pcm(self, d_in: int, in_format: int, d_out: int, out_format: int, n_frames: int, row_stride: int | None = None):
         """Device flavour of process_pcm on raw device pointers; row_stride counts frames for both buffers."""
@@ -433,11 +445,13 @@ class Engine:
             raise ValueError("hrir_schedule must be [n_streams, n_blocks], got %s" % (sched.shape,))
         _check(self._L.ohs_process_device_scheduled(self._h, d_in, d_out, n_frames, rs, sched.ctypes.data, sched.shape[1]))
 
-    def mix_device(self, d_in: int, d_bus: int, n_frames: int, row_stride: int | None = None, bus_stride: int | None = None):
+    def mix_device(self, d_in: int, d_bus: int, n_frames: int, row_stride: int | None = None, bus_stride: int | None = None,
+                   bus_format: int = FMT_F32):
         """Sum the rendered streams of each group (set_groups; by default one group of every stream, the config 4 object
-        mixdown) into its stereo bus: 2 * n_groups rows [n_groups][2][bus_stride] at d_bus."""
-        _check(self._L.ohs_mix_device(self._h, d_in, d_bus, n_frames, n_frames if row_stride is None else row_stride,
-                                      n_frames if bus_stride is None else bus_stride))
+        mixdown) into its stereo bus: 2 * n_groups rows [n_groups][2][bus_stride] at d_bus, in `bus_format`
+        (ohs_mix_device_pcm: an integer bus is dithered as set_dither says, in the same launch)."""
+        _check(self._L.ohs_mix_device_pcm(self._h, d_in, d_bus, bus_format, n_frames, n_frames if row_stride is None else row_stride,
+                                          n_frames if bus_stride is None else bus_stride))
 
     def sync(self):
         _check(self._L.ohs_sync(self._h))

@@ -152,16 +152,17 @@ def _shape_rows(v, d, h, e, lo, hi):
     return q, raw
 
 
-def pcm_encode_dithered(y, fmt: int, seed: int, position: int, shape=(), state=None):
-    """The dithered encode of include/ohs.h (ohs_set_dither): y[..., n] float32 rows, row r = the flat index over the
-    leading axes (2*stream + channel for [S, 2, n]), frame f at dither position position + f.  shape = (h_1, ..., h_M)
-    noise-shapes; `state` is the error history [rows, M] (most recent first, None = zeros after ohs_set_dither).
+def pcm_encode_dithered(y, fmt: int, seed: int, position: int, shape=(), state=None, first_row: int = 0):
+    """The dithered encode of include/ohs.h (ohs_set_dither): y[..., n] float32 rows, row r = first_row + the flat index over
+    the leading axes (2*stream + channel for [S, 2, n]; the buses of a grouped call, mix_groups(y, first), start at
+    first_row = 2 * n_streams), frame f at dither position position + f.  shape = (h_1, ..., h_M) noise-shapes; `state` is
+    the error history [rows, M] (most recent first, None = zeros after ohs_set_dither).
     Returns (q, state): int16 for S16, int32 (unpacked) for S24, and the history after the last frame."""
     b = PCM_BITS[fmt]
     y = np.asarray(y, dtype=np.float32)
     v = (y.reshape(-1, y.shape[-1]) * np.float32(2.0 ** (b - 1))).astype(np.float32)
     rows, n = v.shape
-    d = tpdf_noise(seed, np.arange(rows), position, n)
+    d = tpdf_noise(seed, first_row + np.arange(rows), position, n)
     lo, hi = -(2.0 ** (b - 1)), 2.0 ** (b - 1) - 1
     h = np.asarray(shape, np.float32).ravel()
     e = np.zeros((rows, h.size), np.float32) if state is None else np.array(state, np.float32).reshape(rows, h.size)
