@@ -326,15 +326,6 @@ int set_band_host(ohs_engine* h, int eq_set, int band, const float c[5], int ena
     return OHS_OK;
 }
 
-int check_audio_args(ohs_engine* h, const void* in, const void* out, size_t n_frames, size_t row_stride, bool device) {
-    if (!in || !out) return fail(OHS_ERR_INVALID, "null audio pointer");
-    if (h->conv_enable && n_frames % (size_t)h->B) return fail(OHS_ERR_INVALID, "n_frames %zu is not a multiple of the engine block %d (use ohs_process_fifo)", n_frames, h->B);
-    if (row_stride < n_frames) return fail(OHS_ERR_INVALID, "row_stride %zu < n_frames %zu", row_stride, n_frames);
-    if (device && (((uintptr_t)in | (uintptr_t)out) & 15u || (row_stride & 3u)))
-        return fail(OHS_ERR_ALIGNMENT, "device audio pointers must be 16-byte aligned and row_stride a multiple of 4 frames");
-    return OHS_OK;
-}
-
 size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
 // Frames per chunk of a call of n_frames: about budget_bytes of rows at bytes_per_sample, whole blocks, at least one
@@ -364,35 +355,90 @@ template <typename T> int grow_buffers(ohs_engine* h, T** bufs, int n, size_t& c
     return OHS_OK;
 }
 
-// ---- integer PCM (ohs_process_pcm, ohs_process_device_pcm) --------------------------------------------------------
-size_t pcm_sample_bytes(int fmt) { return fmt == OHS_FMT_S16 ? 2 : fmt == OHS_FMT_S24 ? 3 : 4; }
-// frames in one 16-byte-aligned unit of the format: device rows start 16-byte aligned when the pitch is a multiple
-size_t pcm_align_frames(int fmt) { return fmt == OHS_FMT_S16 ? 8 : fmt == OHS_FMT_S24 ? 16 : 4; }
+// ---- audio I/O: the sides of a call, their argument rules, and the PCM conversions ---------------------------------
+static_assert((int)kPcmF32 == OHS_FMT_F32 && (int)kPcmS16 == OHS_FMT_S16 && (int)kPcmS24 == OHS_FMT_S24, "PcmFormat is OHS_FMT_*");
+static_assert(kShapeTaps == OHS_MAX_SHAPE_TAPS, "history rows of the shaped encode");
 
-int check_pcm_args(ohs_engine* h, const void* in, int in_format, const void* out, int out_format, size_t n_frames, size_t row_stride,
-                   bool device) {
-    for (int f : {in_format, out_format})
-        if (f != OHS_FMT_F32 && f != OHS_FMT_S16 && f != OHS_FMT_S24) return fail(OHS_ERR_INVALID, "unknown sample format %d", f);
-    int rc = check_audio_args(h, in, out, n_frames, row_stride, false);
-    if (rc) return rc;
-    if (in_format != out_format) {
-        // the decode of a later chunk must not read what the encode of an earlier one has written
-        const size_t rows = (size_t)h->cfg.n_streams * 2;
-        const uintptr_t a = (uintptr_t)in, b = (uintptr_t)out;
-        const size_t na = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(in_format);
-        const size_t nb = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(out_format);
-        if (a == b || (a < b + nb && b < a + na))
-            return fail(OHS_ERR_INVALID, "input and output overlap; in place needs equal sample formats");
+// f(std::integral_constant<int, Fmt>{}) for the runtime sample format fmt; `otherwise` for an unknown format
+template <typename R, typename F> R with_pcm_format(int fmt, R otherwise, F&& f) {
+    switch (fmt) {
+        case OHS_FMT_F32: return f(std::integral_constant<int, kPcmF32>{});
+        case OHS_FMT_S16: return f(std::integral_constant<int, kPcmS16>{});
+        case OHS_FMT_S24: return f(std::integral_constant<int, kPcmS24>{});
     }
-    if (device) {
-        const size_t align = std::max(pcm_align_frames(in_format), pcm_align_frames(out_format));
-        if ((((uintptr_t)in | (uintptr_t)out) & 15u) || row_stride % align)
-            return fail(OHS_ERR_ALIGNMENT, "device PCM pointers must be 16-byte aligned and row_stride a multiple of %zu frames", align);
+    return otherwise;
+}
+
+int n_groups(const ohs_engine* h) { return (int)h->h_group_first.size() - 1; }
+
+// One side of an audio call, or of a chunk's work in HBM: rows of `fmt` samples from p on, `stride` frames apart; the
+// 2 * n_groups bus rows with `bus`, else the 2 * n_streams stream rows.  An input side is only read.
+struct Rows {
+    void* p;
+    int fmt;
+    size_t stride;
+    bool bus = false;
+    // 0 for an unknown format
+    size_t sample_bytes() const { return with_pcm_format(fmt, (size_t)0, [](auto f) { return (size_t)PcmTraits<f>::kBytes; }); }
+    // frames in whole 16-byte units of the format: rows start 16-byte aligned when the stride is a multiple
+    size_t align_frames() const { return with_pcm_format(fmt, (size_t)0, [](auto f) { return (size_t)PcmTraits<f>::kGroup; }); }
+    size_t count(const ohs_engine* h) const { return bus ? (size_t)2 * n_groups(h) : (size_t)h->cfg.n_streams * 2; }
+    Rows from(size_t f0) const { return {static_cast<unsigned char*>(p) + f0 * sample_bytes(), fmt, stride, bus}; }
+};
+
+// What an audio entry point asks of its arguments beyond known formats, non-null pointers and strides >= n_frames
+enum CallRule : unsigned {
+    kWholeBlocks = 1,          // a render: n_frames a multiple of the engine block while the convolution is on
+    kSeparate = 2,             // the output (a bus) overlaps no byte of the input, whatever the formats and layouts
+    kSeparateIfConverted = 4,  // when the formats differ, the output neither is nor overlaps the input: in place needs equal formats
+    kDeviceRows = 8,           // 16-byte aligned pointers, and each stride a multiple of its format's align_frames()
+    kWholeQuads = 16,          // with kDeviceRows: n_frames a multiple of 4 (the mixdown)
+};
+
+// The argument check of every audio entry point, before anything is enqueued, so a rejected call leaves the engine
+// untouched.  A call with several faults gets the code of the first in this order.
+int check_call(const ohs_engine* h, const Rows& in, const Rows& out, size_t n_frames, unsigned rules) {
+    for (const Rows* r : {&in, &out})
+        if (!r->sample_bytes()) return fail(OHS_ERR_INVALID, "unknown sample format %d", r->fmt);
+    if (!in.p || !out.p) return fail(OHS_ERR_INVALID, "null audio pointer");
+    if ((rules & kWholeBlocks) && h->conv_enable && n_frames % (size_t)h->B)
+        return fail(OHS_ERR_INVALID, "n_frames %zu is not a multiple of the engine block %d (use ohs_process_fifo)", n_frames, h->B);
+    for (const Rows* r : {&in, &out})
+        if (r->stride < n_frames) return fail(OHS_ERR_INVALID, "%s %zu < n_frames %zu", r->bus ? "bus_stride" : "row_stride", r->stride, n_frames);
+    // the decode or copy-in of a later chunk must not read what the encode or copy-out of an earlier one has written
+    const bool converted = (rules & kSeparateIfConverted) && in.fmt != out.fmt;
+    if ((rules & kSeparate) || converted) {
+        const uintptr_t a = (uintptr_t)in.p, b = (uintptr_t)out.p;
+        const size_t na = ((in.count(h) - 1) * in.stride + n_frames) * in.sample_bytes();
+        const size_t nb = ((out.count(h) - 1) * out.stride + n_frames) * out.sample_bytes();
+        if ((converted && a == b) || (a < b + nb && b < a + na))
+            return fail(OHS_ERR_INVALID, out.bus ? "the bus overlaps the input" : "input and output overlap; in place needs equal sample formats");
     }
+    if ((rules & kDeviceRows) && ((((uintptr_t)in.p | (uintptr_t)out.p) & 15u) || in.stride % in.align_frames() ||
+                                  out.stride % out.align_frames() || ((rules & kWholeQuads) && n_frames % 4)))
+        return fail(OHS_ERR_ALIGNMENT, "device audio needs 16-byte aligned pointers and strides that are multiples of 4 / 8 / 16 frames "
+                                       "(F32 / S16 / S24)%s", (rules & kWholeQuads) ? ", and n_frames a multiple of 4" : "");
     return OHS_OK;
 }
 
-static_assert(kShapeTaps == OHS_MAX_SHAPE_TAPS, "history rows of the shaped encode");
+// Grid of the decode and flat-encode kernels over `rows` rows of n frames: one thread per group of PcmTraits<Fmt>::kGroup
+// frames of a row, at most 2^20 CTAs of 256 (the kernels stride over the rest)
+template <int Fmt> struct GroupGrid {
+    size_t groups, total;
+    unsigned blocks;
+    GroupGrid(size_t rows, size_t n) : groups((n + PcmTraits<Fmt>::kGroup - 1) / PcmTraits<Fmt>::kGroup), total(rows * groups),
+                                       blocks((unsigned)std::min<size_t>((total + 255) / 256, (size_t)1 << 20)) {}
+};
+
+// the PCM stream rows `pcm` decoded into the f32 rows x (pitch p floats) on the engine's stream
+template <int Fmt> int launch_decode(ohs_engine* h, const Rows& pcm, float* x, size_t p, size_t n_frames) {
+    const GroupGrid<Fmt> g((size_t)h->cfg.n_streams * 2, n_frames);
+    pcm_decode_kernel<Fmt><<<g.blocks, 256, 0, h->stream>>>(static_cast<const unsigned char*>(pcm.p), pcm.stride * PcmTraits<Fmt>::kBytes,
+                                                            x, p, n_frames, g.groups, g.total);
+    OHS_CUDA(cudaGetLastError());
+    h->launches++;
+    return OHS_OK;
+}
 
 // pcm_encode_shaped_kernel<Fmt, M, Mix> for the runtime tap count m (1..OHS_MAX_SHAPE_TAPS)
 template <int Fmt, bool Mix, int M = 1>
@@ -408,56 +454,32 @@ void launch_encode_shaped(int m, cudaStream_t st, const float* f32, size_t f32_p
     }
 }
 
-int n_groups(const ohs_engine* h) { return (int)h->h_group_first.size() - 1; }
 // the bus rows' error history: behind the 2 * n_streams stream rows, room for 2 * n_streams bus rows
 float* bus_hist(const ohs_engine* h) { return h->d_dither_hist + (size_t)h->cfg.n_streams * 2 * kShapeTaps; }
 size_t bus_hist_bytes(const ohs_engine* h) { return sizeof(float) * (size_t)h->cfg.n_streams * 2 * kShapeTaps; }
 
-// The encode of f32 rows into PCM rows, dithered as ohs_set_dither says.  Mix: the rows are the 2 * n_groups bus rows, each
-// the sum of its group's stream rows of `f32` (pcm_encode_kernel / pcm_encode_shaped_kernel with Mix): dither row numbers
-// from 2 * n_streams on, i.e. the key hash with the seed seed + phi * 2S, and the error history behind the streams' rows.
+// The encode of the f32 stream rows x (pitch p floats) into the PCM rows `pcm` on the engine's stream, dithered as
+// ohs_set_dither says, its first frame at dither position pos.  Mix: `pcm` is the 2 * n_groups bus rows, each the sum of
+// its group's stream rows of x (pcm_encode_kernel / pcm_encode_shaped_kernel with Mix): dither row numbers from
+// 2 * n_streams on, i.e. the key hash with the seed seed + phi * 2S, and the error history behind the streams' rows.
 template <int Fmt, bool Mix>
-void launch_encode(ohs_engine* h, unsigned char* pcm, size_t pcm_pitch, const float* f32, size_t f32_pitch, size_t n_frames,
-                   unsigned long long pos) {
+int launch_encode(ohs_engine* h, const Rows& pcm, const float* x, size_t p, size_t n_frames, unsigned long long pos) {
     const size_t S2 = (size_t)h->cfg.n_streams * 2, rows = Mix ? (size_t)2 * n_groups(h) : S2;
-    const size_t groups = (n_frames + PcmTraits<Fmt>::kGroup - 1) / PcmTraits<Fmt>::kGroup, total = rows * groups;
-    const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
+    const GroupGrid<Fmt> g(rows, n_frames);
+    unsigned char* q = static_cast<unsigned char*>(pcm.p);
+    const size_t q_pitch = pcm.stride * PcmTraits<Fmt>::kBytes;
     const unsigned long long seed = h->dither_seed + (Mix ? kDitherPhi * S2 : 0ull);
     float* hist = h->d_dither_hist ? h->d_dither_hist + (Mix ? S2 * kShapeTaps : 0) : nullptr;
     const int* gf = Mix ? h->d_group_first : nullptr;
     if (h->dither_mode == OHS_DITHER_TPDF && h->dither_taps > 0)
-        launch_encode_shaped<Fmt, Mix>(h->dither_taps, h->stream, f32, f32_pitch, pcm, pcm_pitch, n_frames, (int)rows, seed, pos,
-                                       h->dither_h, hist, gf);
+        launch_encode_shaped<Fmt, Mix>(h->dither_taps, h->stream, x, p, q, q_pitch, n_frames, (int)rows, seed, pos, h->dither_h, hist, gf);
     else if (h->dither_mode == OHS_DITHER_TPDF)
-        pcm_encode_kernel<Fmt, true, Mix><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, seed,
-                                                                             pos, gf);
+        pcm_encode_kernel<Fmt, true, Mix><<<g.blocks, 256, 0, h->stream>>>(x, p, q, q_pitch, n_frames, g.groups, g.total, seed, pos, gf);
     else
-        pcm_encode_kernel<Fmt, false, Mix><<<blocks, threads, 0, h->stream>>>(f32, f32_pitch, pcm, pcm_pitch, n_frames, groups, total, 0,
-                                                                              0, gf);
-}
-
-// PCM rows <-> f32 rows on the engine's stream; pcm_pitch in bytes, f32_pitch in floats.  An encode is dithered as
-// ohs_set_dither says, its first frame at dither position dither_pos + pos_offset (the frame's offset in the call).  mix:
-// an encode of the group buses of the f32 stream rows into 2 * n_groups PCM bus rows (launch_encode).
-int launch_pcm(ohs_engine* h, bool decode, int fmt, unsigned char* pcm, size_t pcm_pitch, float* f32, size_t f32_pitch, size_t n_frames,
-               size_t pos_offset = 0, bool mix = false) {
-    const size_t rows = (size_t)h->cfg.n_streams * 2;
-    const size_t groups = (n_frames + pcm_align_frames(fmt) - 1) / pcm_align_frames(fmt), total = rows * groups;
-    const unsigned threads = 256, blocks = (unsigned)std::min<size_t>((total + threads - 1) / threads, (size_t)1 << 20);
-    const unsigned long long pos = h->dither_pos + pos_offset;
-    if (decode && fmt == OHS_FMT_S16)
-        pcm_decode_kernel<kPcmS16><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
-    else if (decode)
-        pcm_decode_kernel<kPcmS24><<<blocks, threads, 0, h->stream>>>(pcm, pcm_pitch, f32, f32_pitch, n_frames, groups, total);
-    else if (fmt == OHS_FMT_S16)
-        mix ? launch_encode<kPcmS16, true>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos)
-            : launch_encode<kPcmS16, false>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos);
-    else
-        mix ? launch_encode<kPcmS24, true>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos)
-            : launch_encode<kPcmS24, false>(h, pcm, pcm_pitch, f32, f32_pitch, n_frames, pos);
+        pcm_encode_kernel<Fmt, false, Mix><<<g.blocks, 256, 0, h->stream>>>(x, p, q, q_pitch, n_frames, g.groups, g.total, 0, 0, gf);
     OHS_CUDA(cudaGetLastError());
     h->launches++;
-    if (mix) h->bus_hist_live = true;
+    if (Mix) h->bus_hist_live = true;
     return OHS_OK;
 }
 
@@ -1234,42 +1256,54 @@ int process_device_impl(ohs_engine* h, const float* d_in, float* d_out, size_t n
     return OHS_OK;
 }
 
-// ohs_process_device_pcm past validation, at least one side an integer format
-int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_format, unsigned char* out, int out_format, size_t n_frames,
-                            size_t row_stride) {
+// One chunk of f32 stream rows x (pitch p floats, n frames, at frame f0 of the call) in HBM: the PCM input side decoded
+// into x (an f32 input side is x already), x rendered in place when `render`, then x encoded into the PCM output rows,
+// mixed into the f32 bus, or mixed and encoded into the PCM bus (an f32 output side that is not a bus is x itself).  An
+// encode's first frame is at dither position dither_pos + f0: the position moves once per call, at the call's exit.
+int chunk_step(ohs_engine* h, const Rows& in, float* x, size_t p, size_t n, size_t f0, bool render, const Rows& out) {
+    int rc = with_pcm_format(in.fmt, (int)OHS_ERR_INVALID, [&](auto f) {
+        if constexpr (f == kPcmF32) return (int)OHS_OK;
+        else return launch_decode<f>(h, in, x, p, n);
+    });
+    if (!rc && render) rc = process_device_impl(h, x, x, n, p, nullptr, 0);
+    if (rc) return rc;
+    const unsigned long long pos = h->dither_pos + f0;
+    return with_pcm_format(out.fmt, (int)OHS_ERR_INVALID, [&](auto f) {
+        if constexpr (f == kPcmF32) return out.bus ? launch_mix(h, x, p, static_cast<float*>(out.p), out.stride, n) : (int)OHS_OK;
+        else return out.bus ? launch_encode<f, true>(h, out, x, p, n, pos) : launch_encode<f, false>(h, out, x, p, n, pos);
+    });
+}
+
+// include/ohs.h: a call with integer output (the output format, or a bus call's bus format) moves the dither position on
+// by n_frames, bypassed or not; F32 output and F32 buses leave it
+bool moves_dither(const Rows& out) { return out.fmt != OHS_FMT_F32; }
+
+// ohs_process_device_pcm past validation with at least one side an integer format, and the mixdowns (out.bus: the f32
+// input rows mixed into the bus, never rendered)
+int process_device_io(ohs_engine* h, const Rows& in, const Rows& out, size_t n_frames) {
     if (n_frames == 0) return OHS_OK;
-    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
-    unsigned char* src = const_cast<unsigned char*>(in);   // the decode only reads it
-    if (h->bypass && in_format == out_format) {
-        if (in != out)
-            OHS_CUDA(cudaMemcpy2DAsync(out, row_stride * bo, in, row_stride * bi, n_frames * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
-        h->dither_pos += n_frames;   // an integer output format: the position moves on, although nothing was encoded
-        return OHS_OK;
-    }
-    if (out_format == OHS_FMT_F32) {   // decode straight into the output rows, render them in place
-        float* y = reinterpret_cast<float*>(out);
-        int rc = launch_pcm(h, true, in_format, src, row_stride * bi, y, row_stride, n_frames);
-        if (rc || h->bypass) return rc;
-        return process_device_impl(h, y, y, n_frames, row_stride, nullptr, 0);
-    }
-    int rc = OHS_OK;
-    if (in_format == OHS_FMT_F32 && h->bypass) {
-        rc = launch_pcm(h, false, out_format, out, row_stride * bo, reinterpret_cast<float*>(src), row_stride, n_frames);
+    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = in.sample_bytes();
+    const bool render = !h->bypass && !out.bus;
+    if (h->bypass && !out.bus && in.fmt == out.fmt) {   // nothing to convert: the rows as they are
+        if (in.p != out.p)
+            OHS_CUDA(cudaMemcpy2DAsync(out.p, out.stride * bi, in.p, in.stride * bi, n_frames * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
     } else {
-        const size_t chunk = chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float));
-        if ((rc = ensure_pcm_scratch(h, chunk))) return rc;
-        float* x = h->d_pcm_scratch;
+        // the f32 rows the call works in, chosen once: the input rows when there is nothing to decode or render, the output
+        // rows (decoded into, rendered in place) for F32 output, else the scratch rows, in time chunks
+        const Rows* whole = in.fmt == OHS_FMT_F32 && !render ? &in : out.fmt == OHS_FMT_F32 && !out.bus ? &out : nullptr;
+        const size_t chunk = whole ? n_frames : chunk_frames(h, n_frames, kPcmScratchBytes, sizeof(float));
+        int rc;
+        if (!whole && (rc = ensure_pcm_scratch(h, chunk))) return rc;
+        float* x = whole ? static_cast<float*>(whole->p) : h->d_pcm_scratch;
         for (size_t f0 = 0; f0 < n_frames; f0 += chunk) {
-            const size_t n = std::min(chunk, n_frames - f0), pitch = round_up(n, 4);
-            if (in_format == OHS_FMT_F32)
-                OHS_CUDA(cudaMemcpy2DAsync(x, pitch * sizeof(float), src + f0 * bi, row_stride * bi, n * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
-            else if ((rc = launch_pcm(h, true, in_format, src + f0 * bi, row_stride * bi, x, pitch, n))) return rc;
-            if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
-            if ((rc = launch_pcm(h, false, out_format, out + f0 * bo, row_stride * bo, x, pitch, n, f0))) return rc;
+            const size_t n = std::min(chunk, n_frames - f0), p = whole ? whole->stride : round_up(n, 4);
+            if (!whole && in.fmt == OHS_FMT_F32)
+                OHS_CUDA(cudaMemcpy2DAsync(x, p * bi, in.from(f0).p, in.stride * bi, n * bi, rows, cudaMemcpyDeviceToDevice, h->stream));
+            if ((rc = chunk_step(h, in.from(f0), x, p, n, f0, render, out.from(f0)))) return rc;
         }
     }
-    if (rc == OHS_OK) h->dither_pos += n_frames;
-    return rc;
+    if (moves_dither(out)) h->dither_pos += n_frames;
+    return OHS_OK;
 }
 
 }  // namespace
@@ -1277,17 +1311,14 @@ int process_device_pcm_impl(ohs_engine* h, const unsigned char* in, int in_forma
 extern "C" {
 
 int ohs_process_device(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride) {
-    OHS_CHECK_HANDLE(h);
-    int rc = check_audio_args(h, d_in, d_out, n_frames, row_stride, true);
-    if (rc) return rc;
-    OHS_CUDA(cudaSetDevice(h->cfg.device));
-    return process_device_impl(h, d_in, d_out, n_frames, row_stride, nullptr, 0);
+    return ohs_process_device_pcm(h, d_in, OHS_FMT_F32, d_out, OHS_FMT_F32, n_frames, row_stride);
 }
 
 int ohs_process_device_scheduled(ohs_engine* h, const float* d_in, float* d_out, size_t n_frames, size_t row_stride,
                                  const int32_t* sets, size_t sets_stride) {
     OHS_CHECK_HANDLE(h);
-    int rc = check_audio_args(h, d_in, d_out, n_frames, row_stride, true);
+    const int rc = check_call(h, {const_cast<float*>(d_in), OHS_FMT_F32, row_stride}, {d_out, OHS_FMT_F32, row_stride}, n_frames,
+                              kWholeBlocks | kDeviceRows);
     if (rc) return rc;
     if (!sets) return fail(OHS_ERR_INVALID, "null schedule");
     if (!h->conv_enable) return fail(OHS_ERR_INVALID, "a schedule needs the convolution enabled");
@@ -1304,13 +1335,13 @@ int ohs_process_device_scheduled(ohs_engine* h, const float* d_in, float* d_out,
 
 int ohs_process_device_pcm(ohs_engine* h, const void* d_in, int in_format, void* d_out, int out_format, size_t n_frames, size_t row_stride) {
     OHS_CHECK_HANDLE(h);
-    int rc = check_pcm_args(h, d_in, in_format, d_out, out_format, n_frames, row_stride, true);
+    const Rows in{const_cast<void*>(d_in), in_format, row_stride}, out{d_out, out_format, row_stride};
+    const int rc = check_call(h, in, out, n_frames, kWholeBlocks | kSeparateIfConverted | kDeviceRows);
     if (rc) return rc;
-    if (in_format == OHS_FMT_F32 && out_format == OHS_FMT_F32)
-        return ohs_process_device(h, static_cast<const float*>(d_in), static_cast<float*>(d_out), n_frames, row_stride);
     OHS_CUDA(cudaSetDevice(h->cfg.device));
-    return process_device_pcm_impl(h, static_cast<const unsigned char*>(d_in), in_format, static_cast<unsigned char*>(d_out), out_format,
-                                   n_frames, row_stride);
+    if (in_format == OHS_FMT_F32 && out_format == OHS_FMT_F32)
+        return process_device_impl(h, static_cast<const float*>(d_in), static_cast<float*>(d_out), n_frames, row_stride, nullptr, 0);
+    return process_device_io(h, in, out, n_frames);
 }
 
 int ohs_sync(ohs_engine* h) {
@@ -1346,36 +1377,17 @@ int ohs_last_kernel_ms(ohs_engine* h, float* ms) {
 }
 
 int ohs_mix_device(ohs_engine* h, const float* d_in, float* d_bus, size_t n_frames, size_t row_stride, size_t bus_stride) {
-    OHS_CHECK_HANDLE(h);
-    if (!d_in || !d_bus) return fail(OHS_ERR_INVALID, "null audio pointer");
-    if (n_frames % 4 || row_stride % 4 || bus_stride % 4 || (((uintptr_t)d_in | (uintptr_t)d_bus) & 15u))
-        return fail(OHS_ERR_ALIGNMENT, "mixdown needs 16-byte aligned pointers and frame counts / strides that are multiples of 4");
-    if (row_stride < n_frames || bus_stride < n_frames) return fail(OHS_ERR_INVALID, "stride smaller than n_frames");
-    OHS_CUDA(cudaSetDevice(h->cfg.device));
-    if (n_frames == 0) return OHS_OK;
-    return launch_mix(h, d_in, row_stride, d_bus, bus_stride, n_frames);
+    return ohs_mix_device_pcm(h, d_in, d_bus, OHS_FMT_F32, n_frames, row_stride, bus_stride);
 }
 
 int ohs_mix_device_pcm(ohs_engine* h, const float* d_in, void* d_bus, int bus_format, size_t n_frames, size_t row_stride,
                        size_t bus_stride) {
     OHS_CHECK_HANDLE(h);
-    if (bus_format != OHS_FMT_F32 && bus_format != OHS_FMT_S16 && bus_format != OHS_FMT_S24)
-        return fail(OHS_ERR_INVALID, "unknown bus format %d", bus_format);
-    if (bus_format == OHS_FMT_F32) return ohs_mix_device(h, d_in, static_cast<float*>(d_bus), n_frames, row_stride, bus_stride);
-    if (!d_in || !d_bus) return fail(OHS_ERR_INVALID, "null audio pointer");
-    const size_t align = pcm_align_frames(bus_format);
-    if (n_frames % 4 || row_stride % 4 || bus_stride % align || (((uintptr_t)d_in | (uintptr_t)d_bus) & 15u))
-        return fail(OHS_ERR_ALIGNMENT, "mixdown needs 16-byte aligned pointers, n_frames and row_stride multiples of 4 and bus_stride a "
-                                       "multiple of %zu frames", align);
-    if (row_stride < n_frames || bus_stride < n_frames) return fail(OHS_ERR_INVALID, "stride smaller than n_frames");
+    const Rows in{const_cast<float*>(d_in), OHS_FMT_F32, row_stride}, bus{d_bus, bus_format, bus_stride, true};
+    const int rc = check_call(h, in, bus, n_frames, kDeviceRows | kWholeQuads);
+    if (rc) return rc;
     OHS_CUDA(cudaSetDevice(h->cfg.device));
-    if (n_frames) {
-        const int rc = launch_pcm(h, false, bus_format, static_cast<unsigned char*>(d_bus), bus_stride * pcm_sample_bytes(bus_format),
-                                  const_cast<float*>(d_in), row_stride, n_frames, 0, true);
-        if (rc) return rc;
-    }
-    h->dither_pos += n_frames;
-    return OHS_OK;
+    return process_device_io(h, in, bus, n_frames);
 }
 
 int ohs_set_groups(ohs_engine* h, const int32_t* first, int n_groups) {
@@ -1563,35 +1575,20 @@ namespace {
 
 // Host-pointer flavour: time chunks are staged through three slots in HBM; copy-in, kernels and copy-out of consecutive
 // chunks overlap on three CUDA streams.  Integer PCM crosses the link as PCM and is converted in HBM.  Per chunk: copy-in
-// (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), decode into the f32 buffer, render
-// there in place, encode back into the PCM buffer, copy-out.  ohs_process is the F32 -> F32 case.  With `bus`
-// (ohs_process_grouped_pcm: F32 output, `out` unused) the rendered rows are mixed into the slot's group buses instead,
-// encoded to bus_format in the same launch for an integer bus, and only those 2 * n_groups rows are copied out.  Arguments
-// are validated by the caller.
-int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride,
-                      void* bus = nullptr, int bus_format = OHS_FMT_F32, size_t bus_stride = 0) {
-    OHS_CUDA(cudaSetDevice(h->cfg.device));
-    if (n_frames == 0) return OHS_OK;
+// (PCM rows into the slot's PCM buffer, or f32 rows straight into its f32 buffer), chunk_step on the f32 buffer, and
+// copy-out of the step's output side: the PCM buffer, the f32 buffer, or for a bus (ohs_process_grouped_pcm) the slot's
+// bus rows, so that only those 2 * n_groups rows cross back.  ohs_process is the F32 -> F32 case.
+int process_host_chunks(ohs_engine* h, const Rows& in, const Rows& out, size_t n_frames) {
     int rc = OHS_OK;
-    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = pcm_sample_bytes(in_format), bo = pcm_sample_bytes(out_format);
-    const size_t bus_rows = (size_t)2 * n_groups(h), bb = pcm_sample_bytes(bus_format);
-    const unsigned char* src = static_cast<const unsigned char*>(in);
-    unsigned char* dst = static_cast<unsigned char*>(out);
-    unsigned char* bus_dst = static_cast<unsigned char*>(bus);
-    // the output words this call delivers: an integer format moves the dither position on
-    const bool int_out = bus ? bus_format != OHS_FMT_F32 : out_format != OHS_FMT_F32;
-    if (h->bypass && in_format == out_format && !bus) {
-        if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(dst + r * row_stride * bo, src + r * row_stride * bi, n_frames * bi);
-        if (int_out) h->dither_pos += n_frames;
-        return OHS_OK;
-    }
-    const bool pcm_in = in_format != OHS_FMT_F32, pcm_out = out_format != OHS_FMT_F32, pcm_bus = bus && bus_format != OHS_FMT_F32;
+    const size_t rows = (size_t)h->cfg.n_streams * 2, bi = in.sample_bytes();
+    const bool pcm_in = in.fmt != OHS_FMT_F32, int_out = out.fmt != OHS_FMT_F32, pcm_out = int_out && !out.bus;
+    const size_t bo = out.bus ? sizeof(float) : out.sample_bytes();   // a bus call's stream rows stay f32
     // about stage_bytes per copy of the wider side's rows: 24 MiB by default, measured best on PCIe Gen5 x16 with both
     // directions busy (tools/e2e_probe.py)
     const size_t chunk = chunk_frames(h, n_frames, h->stage_bytes, std::max(bi, bo));
     if ((rc = grow_buffers(h, h->d_stage, kPipe, h->stage_cap, rows * chunk * sizeof(float))) ||
         (rc = grow_buffers(h, h->d_pcm_stage, kPipe, h->pcm_stage_cap, rows * chunk * std::max(pcm_in ? bi : 0, pcm_out ? bo : 0))) ||
-        (bus && (rc = grow_buffers(h, h->d_bus_stage, kPipe, h->bus_stage_cap, bus_rows * chunk * sizeof(float)))))
+        (out.bus && (rc = grow_buffers(h, h->d_bus_stage, kPipe, h->bus_stage_cap, out.count(h) * chunk * sizeof(float)))))
         return rc;
     if (!h->bypass) {
         rc = commit_filters(h);
@@ -1606,32 +1603,20 @@ int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, i
         const size_t pitch = round_up(n, 4), pcm_pitch = round_up(n, 16);   // 16-byte aligned rows in every format
         const int b = idx % kPipe;
         float* x = h->d_stage[b];
-        unsigned char* q = h->d_pcm_stage[b];
-        float* g = h->d_bus_stage[b];
-        unsigned char* gq = reinterpret_cast<unsigned char*>(g);   // an integer bus: packed rows, pcm_pitch frames each
+        void* q = h->d_pcm_stage[b];
+        // the step's sides in the slot; an integer bus is packed rows of pcm_pitch frames in the bus buffer
+        const Rows si{pcm_in ? q : x, in.fmt, pcm_in ? pcm_pitch : pitch};
+        const Rows so{out.bus ? h->d_bus_stage[b] : pcm_out ? q : x, out.fmt, int_out ? pcm_pitch : pitch, out.bus};
+        const size_t ob = so.sample_bytes();
         if (used[b]) OHS_CUDA(cudaStreamWaitEvent(h->h2d, h->ev_out[b], 0));  // buffers free once their copy-out finished
-        if (pcm_in)
-            OHS_CUDA(cudaMemcpy2DAsync(q, pcm_pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
-        else
-            OHS_CUDA(cudaMemcpy2DAsync(x, pitch * bi, src + done * bi, row_stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
+        OHS_CUDA(cudaMemcpy2DAsync(si.p, si.stride * bi, in.from(done).p, in.stride * bi, n * bi, rows, cudaMemcpyHostToDevice, h->h2d));
         OHS_CUDA(cudaEventRecord(h->ev_in[b], h->h2d));
         OHS_CUDA(cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-        if (pcm_in && (rc = launch_pcm(h, true, in_format, q, pcm_pitch * bi, x, pitch, n))) return rc;
-        if (!h->bypass && (rc = process_device_impl(h, x, x, n, pitch, nullptr, 0))) return rc;
-        if (pcm_out && (rc = launch_pcm(h, false, out_format, q, pcm_pitch * bo, x, pitch, n, done))) return rc;
-        if (pcm_bus && (rc = launch_pcm(h, false, bus_format, gq, pcm_pitch * bb, x, pitch, n, done, true))) return rc;
-        if (bus && !pcm_bus && (rc = launch_mix(h, x, pitch, g, pitch, n))) return rc;
+        if ((rc = chunk_step(h, si, x, pitch, n, done, !h->bypass, so))) return rc;
         OHS_CUDA(cudaEventRecord(h->ev_comp[b], h->stream));
         OHS_CUDA(cudaStreamWaitEvent(h->d2h, h->ev_comp[b], 0));
-        if (pcm_bus)
-            OHS_CUDA(cudaMemcpy2DAsync(bus_dst + done * bb, bus_stride * bb, gq, pcm_pitch * bb, n * bb, bus_rows, cudaMemcpyDeviceToHost,
-                                       h->d2h));
-        else if (bus)
-            OHS_CUDA(cudaMemcpy2DAsync(bus_dst + done * bb, bus_stride * bb, g, pitch * bb, n * bb, bus_rows, cudaMemcpyDeviceToHost, h->d2h));
-        else if (pcm_out)
-            OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, q, pcm_pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
-        else
-            OHS_CUDA(cudaMemcpy2DAsync(dst + done * bo, row_stride * bo, x, pitch * bo, n * bo, rows, cudaMemcpyDeviceToHost, h->d2h));
+        OHS_CUDA(cudaMemcpy2DAsync(out.from(done).p, out.stride * ob, so.p, so.stride * ob, n * ob, so.count(h), cudaMemcpyDeviceToHost,
+                                   h->d2h));
         OHS_CUDA(cudaEventRecord(h->ev_out[b], h->d2h));
         used[b] = true;
         done += n;
@@ -1639,7 +1624,23 @@ int process_host_impl(ohs_engine* h, const void* in, int in_format, void* out, i
     }
     OHS_CUDA(cudaStreamSynchronize(h->d2h));
     OHS_CUDA(cudaStreamSynchronize(h->stream));
-    if (int_out) h->dither_pos += n_frames;
+    return OHS_OK;
+}
+
+// ohs_process_pcm and ohs_process_grouped_pcm past validation
+int process_host_impl(ohs_engine* h, const Rows& in, const Rows& out, size_t n_frames) {
+    OHS_CUDA(cudaSetDevice(h->cfg.device));
+    if (n_frames == 0) return OHS_OK;
+    if (h->bypass && !out.bus && in.fmt == out.fmt) {   // nothing to convert: the rows as they are
+        const size_t rows = (size_t)h->cfg.n_streams * 2, bytes = in.sample_bytes();
+        if (in.p != out.p)
+            for (size_t r = 0; r < rows; ++r)
+                memcpy(static_cast<unsigned char*>(out.p) + r * out.stride * bytes, static_cast<const unsigned char*>(in.p) + r * in.stride * bytes,
+                       n_frames * bytes);
+    } else if (const int rc = process_host_chunks(h, in, out, n_frames)) {
+        return rc;
+    }
+    if (moves_dither(out)) h->dither_pos += n_frames;
     return OHS_OK;
 }
 
@@ -1649,26 +1650,19 @@ extern "C" {
 
 int ohs_process_pcm(ohs_engine* h, const void* in, int in_format, void* out, int out_format, size_t n_frames, size_t row_stride) {
     OHS_CHECK_HANDLE(h);
-    const int rc = check_pcm_args(h, in, in_format, out, out_format, n_frames, row_stride, false);
+    const Rows src{const_cast<void*>(in), in_format, row_stride}, dst{out, out_format, row_stride};
+    const int rc = check_call(h, src, dst, n_frames, kWholeBlocks | kSeparateIfConverted);
     if (rc) return rc;
-    return process_host_impl(h, in, in_format, out, out_format, n_frames, row_stride);
+    return process_host_impl(h, src, dst, n_frames);
 }
 
 int ohs_process_grouped_pcm(ohs_engine* h, const void* in, int in_format, void* bus, int bus_format, size_t n_frames, size_t row_stride,
                             size_t bus_stride) {
     OHS_CHECK_HANDLE(h);
-    for (int f : {in_format, bus_format})
-        if (f != OHS_FMT_F32 && f != OHS_FMT_S16 && f != OHS_FMT_S24) return fail(OHS_ERR_INVALID, "unknown sample format %d", f);
-    int rc = check_audio_args(h, in, bus, n_frames, row_stride, false);
+    const Rows src{const_cast<void*>(in), in_format, row_stride}, dst{bus, bus_format, bus_stride, true};
+    const int rc = check_call(h, src, dst, n_frames, kWholeBlocks | kSeparate);
     if (rc) return rc;
-    if (bus_stride < n_frames) return fail(OHS_ERR_INVALID, "bus_stride %zu < n_frames %zu", bus_stride, n_frames);
-    // the decode or copy-in of a later chunk must not read what the copy-out of an earlier one has written
-    const size_t rows = (size_t)h->cfg.n_streams * 2, bus_rows = (size_t)2 * n_groups(h);
-    const uintptr_t a = (uintptr_t)in, b = (uintptr_t)bus;
-    const size_t na = ((rows - 1) * row_stride + n_frames) * pcm_sample_bytes(in_format);
-    const size_t nb = ((bus_rows - 1) * bus_stride + n_frames) * pcm_sample_bytes(bus_format);
-    if (a < b + nb && b < a + na) return fail(OHS_ERR_INVALID, "the bus overlaps the input");
-    return process_host_impl(h, in, in_format, nullptr, OHS_FMT_F32, n_frames, row_stride, bus, bus_format, bus_stride);
+    return process_host_impl(h, src, dst, n_frames);
 }
 
 int ohs_process_grouped(ohs_engine* h, const void* in, int in_format, float* bus, size_t n_frames, size_t row_stride,
@@ -1684,8 +1678,8 @@ int ohs_process(ohs_engine* h, const float* in, float* out, size_t n_frames, siz
 // run every complete engine block, hand back n frames if that many are ready, else silence (and keep what is queued).
 int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames, size_t row_stride) {
     OHS_CHECK_HANDLE(h);
-    if (!in || !out) return fail(OHS_ERR_INVALID, "null audio pointer");
-    if (row_stride < n_frames) return fail(OHS_ERR_INVALID, "row_stride %zu < n_frames %zu", row_stride, n_frames);
+    int rc = check_call(h, {const_cast<float*>(in), OHS_FMT_F32, row_stride}, {out, OHS_FMT_F32, row_stride}, n_frames, 0);
+    if (rc) return rc;
     const size_t rows = (size_t)h->cfg.n_streams * 2;
     if (h->bypass) {
         if (in != out) for (size_t r = 0; r < rows; ++r) memcpy(out + r * row_stride, in + r * row_stride, n_frames * sizeof(float));
@@ -1710,7 +1704,7 @@ int ohs_process_fifo(ohs_engine* h, const float* in, float* out, size_t n_frames
         // FIFO (src/lib.rs:1194-1199) — per-sample filtering, so the result is identical.
         std::vector<float> tmp(rows * whole);
         for (size_t r = 0; r < rows; ++r) memcpy(&tmp[r * whole], &h->fifo_in[r * cap], whole * sizeof(float));
-        int rc = ohs_process(h, tmp.data(), tmp.data(), whole, whole);
+        rc = ohs_process(h, tmp.data(), tmp.data(), whole, whole);
         if (rc) return rc;
         for (size_t r = 0; r < rows; ++r) {
             memcpy(&h->fifo_out[r * cap + h->fifo_out_len], &tmp[r * whole], whole * sizeof(float));

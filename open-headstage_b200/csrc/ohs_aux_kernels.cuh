@@ -377,6 +377,9 @@ __global__ void mix_streams_kernel(const float* __restrict__ in, float* __restri
 enum PcmFormat { kPcmF32 = 0, kPcmS16 = 1, kPcmS24 = 2 };   // OHS_FMT_*
 
 template <int Fmt> struct PcmTraits;
+template <> struct PcmTraits<kPcmF32> {   // f32 rows (sizes on the host only: no kernel converts F32)
+    static constexpr int kBytes = 4, kGroup = 4;
+};
 template <> struct PcmTraits<kPcmS16> {
     static constexpr int kBytes = 2, kGroup = 8;
     static constexpr float kDecode = 0x1p-15f, kEncode = 0x1p15f, kLo = -32768.0f, kHi = 32767.0f;

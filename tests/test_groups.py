@@ -411,6 +411,14 @@ def test_rejected_calls_leave_the_engine_untouched():
     assert lib.ohs_process_grouped(b._h, qp + 64, S16, qp, n, n, n) == ERR_INVALID
     assert b.state_export() == blob
     assert not bus.any()
+    # one stream per group: the 2G bus rows have exactly the input's layout, and still the bus may not be the input
+    c = make_engine(4)
+    c.set_groups([0, 1, 2, 3, 4])
+    blob_c = c.state_export()
+    x4 = inputs(4, n)
+    keep = x4.tobytes()
+    assert lib.ohs_process_grouped(c._h, x4.ctypes.data, F32, x4.ctypes.data, n, n, n) == ERR_INVALID
+    assert c.state_export() == blob_c and x4.tobytes() == keep
     # the groups set before the rejected calls are still in force
     twin_call(a, b, q, first)
     same_state(a, b, inputs(n_streams, 512, seed=2))
